@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...        # the CPU port of the reference path on the host cores
+    python bench.py ... --dump-outputs DIR      # also write the headline's last timed frame to DIR/frame.npy
 
 Headline (every N): BASELINE configs[4] AT SPEC -- a procedural 10^8-triangle scene with an environment light, 3840x2160,
 stratified sampler with 1024 samples per pixel, path_mis maxDepth 5 (SURVEY 8d-5).  The scene is generated on the device from a
@@ -24,8 +25,10 @@ import argparse
 import json
 import math
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -39,6 +42,24 @@ for p in (os.path.join(ROOT, "nano-kazen_b200"), os.path.join(ROOT, "tests")):
 SPP_TOTAL = 1024          # configs[4]
 SPP_PER_STEP = 64
 WARM_XML = os.path.join(ROOT, "tests", "data", "kazen_scenes", "2022_q1", "WarmStudio", "WarmStudio.xml")
+DUMP_MAX_PIXELS = 1 << 21     # 32 MiB of RGBW float32
+DUMP_SEED = 0
+
+
+def dump_frame(frame, out_dir):
+    """Writes a (H+2b, W+2b, 4) float32 device frame to out_dir/frame.npy: the whole frame when it has at most DUMP_MAX_PIXELS
+    pixels, else a (DUMP_MAX_PIXELS, 4) sample of its pixels, chosen with DUMP_SEED and kept in row-major order, so that two
+    builds run with the same arguments write the same pixels.  The path contributions are summed into the frame by atomic adds in
+    no fixed order, so two runs of one build agree to float rounding, not bit for bit: compare with a relative tolerance."""
+    import torch
+    fh, fw, _ = frame.shape
+    if fh * fw <= DUMP_MAX_PIXELS:
+        out = frame.cpu().numpy()
+    else:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(fh * fw, DUMP_MAX_PIXELS, replace=False))
+        out = frame.reshape(-1, 4).index_select(0, torch.from_numpy(idx).to(frame.device)).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "frame.npy"), np.ascontiguousarray(out, np.float32))
 
 
 def b_ray(n_tris, shadow=False):
@@ -216,8 +237,13 @@ def main():
     ap.add_argument("--height", type=int, default=2160)
     ap.add_argument("--legs", default="auto", help="comma list of headline,soup1m,soup10m,c0,c2,c3 (auto: all at N=1, headline+c0 at N>1)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline legs")
-    ap.add_argument("--cfg-dir", default=os.path.join(ROOT, "tests", "data", "_generated", "bench"))
+    ap.add_argument("--cfg-dir", default=None, help="directory for the generated configs[2] / configs[3] scenes (default: a temporary one, removed at exit)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frame of the headline's last timed step to DIR/frame.npy (float32, see dump_frame)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's frame; it does not apply to --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -257,9 +283,11 @@ def main():
     def rsum(v): return reduce_scalar(v, dist.ReduceOp.SUM) if world > 1 else v
 
     # ------------------------------------------------------------------------------------------ a path-tracing leg
-    def path_leg(G, n_tris, W, H, spp_step, spp_total, steps, warmup, label, upload_ms, build_ms, oracle_desc=None, cpu_rect=None, clocks_on=False):
+    def path_leg(G, n_tris, W, H, spp_step, spp_total, steps, warmup, label, upload_ms, build_ms, oracle_desc=None, cpu_rect=None, clocks_on=False,
+                 dump_dir=None):
         """Times `steps` steps of spp_step sample indices each (strong scaling: this rank's shard + the NCCL reduce), then the same
-        through the host-frame C ABI call, then (rank 0, N = 1) a bounded sample on the CPU port."""
+        through the host-frame C ABI call, then (rank 0, N = 1) a bounded sample on the CPU port.  dump_dir: rank 0 writes the frame
+        of the last timed step there (dump_frame)."""
         fh, fw, _ = G.frame_shape()
         frame = torch.zeros((fh, fw, 4), dtype=torch.float32, device=dev)
         host_frame = torch.zeros((fh, fw, 4), dtype=torch.float32).pin_memory() if rank == 0 else None
@@ -289,6 +317,8 @@ def main():
             torch.cuda.profiler.stop()
         ms = rmax(e0.elapsed_time(e1)) / steps
         clk = clocks.stop() if clocks else None
+        if dump_dir and rank == 0:
+            dump_frame(frame, dump_dir)
         st = G.stats(reset=True)
         npaths = W * H * spp_step
         n_ext = rsum(st["rays_extension"]) / steps / npaths
@@ -474,7 +504,8 @@ def main():
     torch.cuda.empty_cache()
     W, H = args.width, args.height
     head = path_leg(G, args.tris, W, H, SPP_PER_STEP, SPP_TOTAL, args.steps, args.warmup, headline_config(args, world)["workload"], st0["ms_upload"], st0["ms_build"],
-                    oracle_desc=oracle_desc, cpu_rect=(W // 4, H // 4, W // 4 + W // 2, H // 4 + H // 2) if args.tris > 100000 else None, clocks_on=True)
+                    oracle_desc=oracle_desc, cpu_rect=(W // 4, H // 4, W // 4 + W // 2, H // 4 + H // 2) if args.tris > 100000 else None, clocks_on=True,
+                    dump_dir=args.dump_outputs)
     head["roofline"]["traffic"] = committed_traffic(tris=args.tris, kernel="k_extend")
     G.close()
     oracle_desc = None
@@ -488,15 +519,20 @@ def main():
         import importlib.util
         spec = importlib.util.spec_from_file_location("make_configs", os.path.join(ROOT, "tests", "data", "make_configs.py"))
         mc = importlib.util.module_from_spec(spec); spec.loader.exec_module(mc)
-        cfg = mc.generate(args.cfg_dir, tex_res=4096)
-        if "c2" in legs:
-            extra["lookdev_4k"] = xml_leg(os.path.join(cfg, "c3_lookdev_4k.xml"), {}, pk.BUILD_HOST_SAH,
-                                          "BASELINE configs[2] stand-in: normalmap + kiss + 4096^2 image textures through blend, thin lens", 64,
-                                          cpu_rect=(1440, 810, 2400, 1350))
-        if "c3" in legs:
-            extra["pmj02bn_1080p"] = xml_leg(os.path.join(cfg, "c4_pmj02bn_1080p.xml"), {}, pk.BUILD_HOST_SAH,
-                                             "BASELINE configs[3] stand-in: pmj02bn sampler, traceBias 1e-3, regularization, low-poly smooth sphere", 64,
-                                             cpu_rect=(480, 270, 1440, 810))
+        cfg = args.cfg_dir or tempfile.mkdtemp(prefix="kz_bench_cfg_")       # the tree may be read-only
+        try:
+            mc.generate(cfg, tex_res=4096)
+            if "c2" in legs:
+                extra["lookdev_4k"] = xml_leg(os.path.join(cfg, "c3_lookdev_4k.xml"), {}, pk.BUILD_HOST_SAH,
+                                              "BASELINE configs[2] stand-in: normalmap + kiss + 4096^2 image textures through blend, thin lens", 64,
+                                              cpu_rect=(1440, 810, 2400, 1350))
+            if "c3" in legs:
+                extra["pmj02bn_1080p"] = xml_leg(os.path.join(cfg, "c4_pmj02bn_1080p.xml"), {}, pk.BUILD_HOST_SAH,
+                                                 "BASELINE configs[3] stand-in: pmj02bn sampler, traceBias 1e-3, regularization, low-poly smooth sphere", 64,
+                                                 cpu_rect=(480, 270, 1440, 810))
+        finally:
+            if not args.cfg_dir:
+                shutil.rmtree(cfg, ignore_errors=True)
     if "soup1m" in legs:
         extra["soup_1m"] = soup_leg(1 << 20, pk.BUILD_HOST_SAH, 6, True)
     if "soup10m" in legs:

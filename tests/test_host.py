@@ -16,7 +16,6 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 BOX = os.path.join(HERE, "data", "box", "box.xml")
 KAZEN = os.path.join(ROOT, "nano-kazen_b200", "host", "kazen")
-REF_SCENES = "/root/reference/scene/2022_q1"
 SHIPPED_SCENES = os.path.join(HERE, "data", "kazen_scenes", "2022_q1")      # byte copies of two reference scenes (inputs, see the README there)
 WARM = os.path.join(SHIPPED_SCENES, "WarmStudio", "WarmStudio.xml")
 PARAM = os.path.join(SHIPPED_SCENES, "parameters", "default_m0_r0.5.xml")
@@ -181,23 +180,16 @@ def test_extra_bsdf_plugins_from_xml(host, tmp_path):
         host.HostScene(str(tmp_path / "bad.xml"))
 
 
-def test_cli_fails_loudly_without_gpu(host):
-    try:
-        import torch
-        if torch.cuda.is_available():
-            pytest.skip("GPU present")
-    except ImportError:
-        pass
-    r = subprocess.run([KAZEN, BOX, "-o", "/tmp/kazen_cli_test"], capture_output=True, text=True)
+def test_cli_fails_loudly_without_gpu(host, tmp_path):
+    """run where no device is visible, so that the check holds on GPU machines as well"""
+    r = subprocess.run([KAZEN, BOX, "-o", str(tmp_path / "box")], capture_output=True, text=True, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
     assert r.returncode != 0 and "no CUDA device" in r.stderr and "no CPU fallback" in r.stderr
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SCENES), reason="reference scenes are only mounted in the build container")
 def test_reference_scenes_parse_unchanged(host, kzo):
-    """kazen's own scene files load unchanged through the plugin system (22 parameter sweeps + WarmStudio)"""
-    xmls = [os.path.join(REF_SCENES, "WarmStudio", "WarmStudio.xml")] + \
-           sorted(os.path.join(REF_SCENES, "parameters", f) for f in os.listdir(os.path.join(REF_SCENES, "parameters")) if f.endswith(".xml"))
-    assert len(xmls) == 23
+    """kazen's own scene files as tests/data/kazen_scenes ships them (WarmStudio + the default parameter-sweep scene) load unchanged
+    through the plugin system"""
+    xmls = [WARM, PARAM]
     tris = {}
     for x in xmls:
         hs = host.HostScene(x, {"camera.width": "i:64", "camera.height": "i:36"})
@@ -213,19 +205,29 @@ def test_reference_scenes_parse_unchanged(host, kzo):
     m = srgb.reshape(-1, 3).mean(0)
     assert 20 < m[0] < 45 and 14 < m[1] < 34 and 5 < m[2] < 18 and m[0] > m[1] > m[2]       # shipped PNG: (36.5, 27.5, 13.1)
     O.close(); hs.close()
+    # the default parameter-sweep scene against the mean of the reference's golden PNG of it (8-bit and older than the Q2
+    # changes, so the frame mean sits up to ~0.045 lower here)
+    hs = host.HostScene(xmls[1], {"camera.width": "i:192", "camera.height": "i:108", "sampler.sampleCount": "i:36", "sampler.type": "s:stratified"})
+    O = kzo.Oracle(hs.desc)
+    rgb, _ = O.resolve(O.render())
+    d = np.minimum(rgb, 1.0).mean(axis=(0, 1)) - np.array(_golden_means()["default_m0_r0.5"])
+    assert (-0.045 < d).all() and (d < 0.005).all(), d
+    O.close(); hs.close()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SCENES), reason="reference scenes are only mounted in the build container")
 def test_shipped_scene_fixtures_are_the_reference_files():
-    """tests/data/kazen_scenes holds byte copies of the reference's scene files (so that 'an existing scene file renders unchanged')"""
-    n = 0
+    """tests/data/kazen_scenes holds byte copies of the reference's scene files (so that 'an existing scene file renders unchanged');
+    tests/golden/kazen_scenes_sha256.json holds the SHA-256 of each reference file, taken when the copies were compared byte for byte
+    with the reference tree"""
+    import hashlib
+    gold = json.load(open(os.path.join(HERE, "golden", "kazen_scenes_sha256.json")))
+    got = {}
     for root, _, files in os.walk(SHIPPED_SCENES):
         for f in files:
             p = os.path.join(root, f)
-            ref = os.path.join(REF_SCENES, os.path.relpath(p, SHIPPED_SCENES))
-            assert open(p, "rb").read() == open(ref, "rb").read(), p
-            n += 1
-    assert n == 11
+            got[os.path.relpath(p, SHIPPED_SCENES)] = hashlib.sha256(open(p, "rb").read()).hexdigest()
+    assert got == gold
+    assert len(got) == 11
 
 
 def test_shipped_scenes_parse(host, kzo):
@@ -445,36 +447,6 @@ def test_kazen_cli_resumes_a_render(host, tmp_path):
     assert np.allclose(a, c, rtol=1e-4, atol=1e-5)
     r = subprocess.run([KAZEN, BOX, "-o", rest, "--size", "33x17", "--resume", part + ".rgbw"], capture_output=True, text=True)
     assert r.returncode != 0 and "does not match" in r.stderr
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_SCENES), reason="reference scenes are only mounted in the build container")
-def test_kiss_parameter_sweeps_follow_the_golden_images(host, kzo):
-    """The reference ships one golden PNG per parameter-sweep scene (kiss metallic / roughness / specular / specularTint / clearcoat /
-    clearcoatRoughness / sheen / sheenTint).  The goldens predate the Q2 changes and are 8-bit, so absolute means sit ~0.02-0.03
-    lower here, but the EFFECT of every parameter (difference of frame means between two scenes of a sweep) must match the
-    reference's own images: that pins the kiss parameter semantics of the oracle (and so of the GPU path) to reference output."""
-    import json
-    gold = json.load(open(os.path.join(HERE, "golden", "param_means.json")))
-    ours = {}
-    for name in gold:
-        if name == "WarmStudio":
-            continue
-        hs = host.HostScene(os.path.join(REF_SCENES, "parameters", name + ".xml"),
-                            {"camera.width": "i:192", "camera.height": "i:108", "sampler.sampleCount": "i:36", "sampler.type": "s:stratified"})
-        O = kzo.Oracle(hs.desc)
-        rgb, _ = O.resolve(O.render())
-        ours[name] = np.minimum(rgb, 1.0).mean(axis=(0, 1))
-        O.close(); hs.close()
-        d = ours[name] - np.array(gold[name])
-        assert (-0.045 < d).all() and (d < 0.005).all(), (name, d)
-    sweeps = [("m0_r0_spec0", "m0_r0_spec0.5"), ("m0_r0_spec0.5", "m0_r0_spec1"), ("m0_r0_spec1", "m0_r0_spec1_st0.5"), ("m0_r0_spec1_st0.5", "m0_r0_spec1_st1"),
-              ("r0.5_c0", "r0.5_c0.5"), ("r0.5_c0.5", "r0.5_c1"), ("r0.5_c1", "r0.5_c1_cr0.5"), ("r0.5_c1_cr0.5", "r0.5_c1_cr1"),
-              ("r0_s0", "r0_s0.5"), ("r0_s0.5", "r0_s1"), ("r0_s1", "r0_s1_st0.5"), ("r0_s1_st0.5", "r0_s1_st1"),
-              ("m0.0_r0", "m0.0_r0.5"), ("m0.0_r0.5", "m0.0_r1"), ("m1_r0.5", "m1_r1")]
-    for a, b in sweeps:
-        eff_ours = ours[b] - ours[a]
-        eff_gold = np.array(gold[b]) - np.array(gold[a])
-        assert np.abs(eff_ours - eff_gold).max() < 2.5e-3, (a, b, eff_ours, eff_gold)
 
 
 def test_image_readers(host, tmp_path):

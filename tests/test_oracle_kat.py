@@ -203,15 +203,3 @@ def test_math_helpers_match_the_reference_bodies(kzo):
         seen.add(case["fn"])
     assert len(seen) == 46 and {"kissEval", "kissPdf", "kissSample", "sampleVNDF", "dpdfSample", "samplerStratified", "samplerCorrelated",
                                 "extraEval", "extraPdf", "extraSample", "texColorRamp", "texBlend", "texBackgroundUV", "texBackgroundDir", "sceneBackground", "pmj02bnTileSize"} <= seen
-
-
-@pytest.mark.skipif(not os.path.isdir("/root/reference/include/kazen"), reason="the reference is only mounted in the build container")
-def test_reference_math_bodies_run_here_agree(kzo):
-    """Where the reference is mounted: build oracle/_ref/ref_math_kat from the reference's sources in place and require 0 mismatches
-    over all 251 000 cases (incl. Scene::getBackgroundColor, the seven other BSDF plugins, the texture expression nodes, the PMJ02BN sampler body over synthetic tables, post-intersection, Mesh::sample and AreaLight on random meshes, and 36 000 whole paths through the reference's own PathMisIntegrator::Li body on random scenes) (the golden file keeps about 1 200 of them)."""
-    import subprocess
-    root = os.path.dirname(HERE)
-    subprocess.check_call(["make", "-s", "-C", os.path.join(root, "oracle"), "_ref/ref_math_kat"])
-    r = subprocess.run([os.path.join(root, "oracle", "_ref", "ref_math_kat")], capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr[-2000:]
-    assert "0 mismatches" in r.stderr and "pathMisLi: 36000 paths" in r.stderr
