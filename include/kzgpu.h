@@ -241,6 +241,7 @@ typedef struct kz_stats {
     double   ms_build;         /* wall time of the last kzgpu_accel_build (host + device) */
     double   ms_upload;        /* wall time of the last kzgpu_scene_upload           */
     double   ms_merge;         /* device time in the multi-device frame merge since reset */
+    uint64_t rays_seeded;      /* primary rays whose traversal started from their pixel's previous hit (the "primary_hint" option) */
 } kz_stats;
 
 #define KZ_BUILD_HOST_SAH 0    /* binned SAH on the host, collapsed to 8-wide, uploaded */
@@ -319,7 +320,9 @@ int  kzgpu_light_sample_dump(kzgpu_ctx *ctx, const float *ref3, const float *u5,
  * indices per pixel tile in path order; also read from KZGPU_LANES / KZGPU_POOL_LOG2 / KZGPU_SPP_GROUP at
  * kzgpu_create).  "lanes" = concurrent chunks per device (1 = strictly serial kernels, which is what per-kernel timings in
  * kz_stats need to be meaningful), "pool_log2" = log2 of the path slots per chunk, "spp_group" = consecutive sample indices of a pixel
- * tile that are neighbours in path order (1 = sample-major).  None of them changes which paths are traced. */
+ * tile that are neighbours in path order (1 = sample-major), "primary_hint" (KZGPU_PRIMARY_HINT) = whether a primary ray's traversal
+ * starts from the triangle its pixel's previous primary ray hit: 0 = never, 1 (default) = in scenes of at least 2^20 triangles (where
+ * it pays), 2 = always.  None of them changes which paths are traced or what they hit. */
 int  kzgpu_configure(kzgpu_ctx *ctx, const char *key, int value);
 
 int  kzgpu_stats(kzgpu_ctx *ctx, kz_stats *out);

@@ -51,6 +51,11 @@ struct Device {
     uint32_t *cursor = nullptr;      /* batch-trace fetch cursor */
     KzF4 *frame = nullptr;
     size_t frame_texels = 0;
+    /* primary-hit hints (KzExtendJob<true>::seed): (geomID, primID) per film pixel, allocated by the first render that uses them and
+     * invalidated (all 0xFF) whenever the accel or the film may have changed -- a hint is only worth something for the same triangles */
+    uint2 *hint = nullptr;
+    size_t hint_px = 0;
+    bool hint_stale = true;
     cudaEvent_t splat_done = nullptr, merge_done = nullptr;   /* multi-device frame merge (k_frame_reduce) */
     /* scratch for host-pointer entry points */
     void *scratch[3] = {nullptr, nullptr, nullptr};
@@ -73,6 +78,10 @@ struct kzgpu_ctx {
     bool uploaded = false, built = false;
     uint32_t pool_cap = 1u << 24;     /* path slots per chunk and lane (160 B each = 2.5 GiB): every launch costs ~18 us of ramp + tail, so few big chunks win */
     int lanes = 3;                    /* concurrent chunks per device at most, 1..4 (KZGPU_LANES=1: strictly serial chunks); frames below 2^25 paths use two */
+    int primary_hint = 1;             /* seed primary rays with the triangle their pixel hit last (KzExtendJob<true>::seed; KZGPU_PRIMARY_HINT / "primary_hint"):
+                                       * 0 = never, 1 = for scenes of at least KZ_HINT_MIN_TRIS triangles, 2 = always.  Measured on B200, Mpaths/s off -> on:
+                                       * 10^8-triangle 4K headline 909 -> 975 (primary pass ~25 % shorter); WarmStudio.xml 1292 -> 1269, configs[2] 873 -> 866,
+                                       * configs[3] 849 -> 838 (few triangles: the primaries are cheap, the extra loads and spills of the seed are not) */
     int spp_group = 64;               /* sample indices of one tile that are neighbours in path order (KZGPU_SPP_GROUP, 1 = sample-major).  Measured on the
                                        * 10^8-triangle 4K headline / WarmStudio.xml / configs[2], Mpaths/s, with k_accumulate splatting one 32-path unit per warp at a time
                                        * (the splats of neighbouring warps then pile onto the same texels): 1 -> 827 / 1213 / 821, 8 -> 842 / 1213 / 823, 64 -> 807 / 1110 / 780;
@@ -340,12 +349,20 @@ int replicate_accel(kzgpu_ctx *ctx, Device &dst, const Device &src) {
 /* One chunk of path slots through the whole wavefront on stream `s` with the pool of lane `L`; never synchronises (except the
  * unbounded whitted / path_mats loops, which poll a queue count). */
 /* `ectx` receives error messages (nullptr inside the per-device worker threads of kzgpu_render, which report through g_error). */
+#ifndef KZ_HINT_MIN_TRIS
+#define KZ_HINT_MIN_TRIS (1u << 20)
+#endif
+bool hints_on(const kzgpu_ctx *ctx) {
+    return ctx->primary_hint == 2 || (ctx->primary_hint == 1 && ctx->hs->total_triangles >= KZ_HINT_MIN_TRIS);
+}
+
 int enqueue_chunk(const kzgpu_ctx *ctx, kzgpu_ctx *ectx, Device &d, Lane &L, const KzChunk &ch, unsigned long long new_paths, cudaStream_t s) {
     const KzScene &sc = d.sc;
     const int max_depth = sc.integrator.max_depth;
     /* the pass after the last vertex only resolves "miss -> background" (integrator.cpp:315-318) */
     const int last_pass = sc.background >= 0 ? max_depth : max_depth - 1;
     const bool alt = sc.integrator.type != KZ_INTEGRATOR_PATH_MIS;
+    uint2 *const hint = hints_on(ctx) ? d.hint : nullptr;
     if (d.pending.size() > 8192) fold_events(d);       /* very long renders: bound the number of live timing events */
     {
         Timed t(d, s, CAT_SHADE);
@@ -362,8 +379,8 @@ int enqueue_chunk(const kzgpu_ctx *ctx, kzgpu_ctx *ectx, Device &d, Lane &L, con
             {
                 Timed t(d, s, CAT_TRACE);
                 k_bounce_reset<<<1, 32, 0, s>>>(L.ctl, nxt);
-                if (b == 0) k_extend<true><<<d.grid_extend0, KZ_TRACE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, cur);
-                else k_extend<false><<<d.grid_extend, KZ_TRACE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, cur);
+                if (b == 0) k_extend<true><<<d.grid_extend0, KZ_TRACE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, cur, hint);
+                else k_extend<false><<<d.grid_extend, KZ_TRACE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, cur, nullptr);
                 d.launches += 2;
             }
             {
@@ -389,8 +406,8 @@ int enqueue_chunk(const kzgpu_ctx *ctx, kzgpu_ctx *ectx, Device &d, Lane &L, con
         {
             Timed t(d, s, CAT_TRACE);
             k_bounce_reset<<<1, 32, 0, s>>>(L.ctl, nxt);
-            if (b == 0) k_extend<true><<<d.grid_extend0, KZ_TRACE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, cur);
-            else k_extend<false><<<d.grid_extend, KZ_TRACE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, cur);
+            if (b == 0) k_extend<true><<<d.grid_extend0, KZ_TRACE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, cur, hint);
+            else k_extend<false><<<d.grid_extend, KZ_TRACE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, cur, nullptr);
             d.launches += 2;
         }
         {
@@ -446,6 +463,19 @@ int enqueue_render(const kzgpu_ctx *ctx, kzgpu_ctx *ectx, Device &d, const kz_re
     const uint32_t cap = (uint32_t)((((total + n_chunks - 1) / n_chunks) + 31ull) & ~31ull);
     int rc;
     for (int l = 0; l < lanes; ++l) if ((rc = ensure_pool(ectx, d.lane[l], cap))) return rc;
+    if (hints_on(ctx)) {
+        /* every pixel k_raygen can produce lies on the film (check_req), whatever the rectangle or the device's share of samples */
+        const size_t npx = (size_t)sc.camera.width * (size_t)sc.camera.height;
+        if (d.hint_px < npx) {
+            if (d.hint) { cudaFree(d.hint); d.hint = nullptr; d.hint_px = 0; }
+            KZ_CUDA(ectx, cudaMalloc(&d.hint, npx * sizeof(uint2)));
+            d.hint_px = npx; d.hint_stale = true;
+        }
+        if (d.hint_stale) {     /* before anything of this request, on s: the other lanes start after it (below) */
+            KZ_CUDA(ectx, cudaMemsetAsync(d.hint, 0xFF, d.hint_px * sizeof(uint2), s));
+            d.hint_stale = false;
+        }
+    }
     Timed total_t(d, s, CAT_TOTAL);
     if (lanes > 1) {       /* the other lanes start after what is already queued on s (frame clear, earlier requests) */
         KZ_CUDA(ectx, cudaEventRecord(d.lane[0].done, s));
@@ -495,6 +525,7 @@ int kzgpu_create(const int *device_ids, int n_devices, kzgpu_ctx **out) {
     if (const char *p = getenv("KZGPU_POOL_LOG2")) { int l = atoi(p); if (l >= 10 && l <= 26) ctx->pool_cap = 1u << l; }
     if (const char *p = getenv("KZGPU_LANES")) { int l = atoi(p); if (l >= 1 && l <= KZ_MAX_LANES) ctx->lanes = l; }
     if (const char *p = getenv("KZGPU_SPP_GROUP")) { int g = atoi(p); if (g >= 1) ctx->spp_group = g; }
+    if (const char *p = getenv("KZGPU_PRIMARY_HINT")) { int h = atoi(p); if (h >= 0 && h <= 2) ctx->primary_hint = h; }
     for (int id : ids) {
         if (id < 0 || id >= count) return fail(nullptr, KZ_ERR_NO_DEVICE, "device id " + std::to_string(id) + " out of range");
         cudaDeviceProp prop;
@@ -555,6 +586,7 @@ void kzgpu_destroy(kzgpu_ctx *ctx) {
         fold_events(d);
         for (cudaEvent_t e : d.free_events) cudaEventDestroy(e);
         free_all(d.scene_allocs); free_all(d.accel_allocs);
+        if (d.hint) cudaFree(d.hint);
         for (Lane &L : d.lane) { free_all(L.allocs); cudaFree(L.ctl); if (L.done) cudaEventDestroy(L.done); if (L.stream) cudaStreamDestroy(L.stream); }
         for (int k = 0; k < 3; ++k) if (d.scratch[k]) cudaFree(d.scratch[k]);
         cudaFree(d.cursor);
@@ -606,6 +638,7 @@ int kzgpu_scene_upload(kzgpu_ctx *ctx, const kz_scene_desc *scene) {
     for (Device &d : ctx->devs) {
         KZ_CUDA(ctx, cudaSetDevice(d.id));
         d.has_accel = false;
+        d.hint_stale = true;
         free_all(d.accel_allocs);
         int rc = upload_tables(ctx, d);
         if (rc) return rc;
@@ -674,6 +707,7 @@ int kzgpu_accel_build(kzgpu_ctx *ctx, int builder) {
         }
         KZ_CUDA(ctx, cudaSetDevice(d0.id));
     }
+    for (Device &d : ctx->devs) d.hint_stale = true;
     ctx->ms_build = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     ctx->built = true;
     return KZ_OK;
@@ -1076,6 +1110,7 @@ int kzgpu_configure(kzgpu_ctx *ctx, const char *key, int value) {
     if (k == "lanes") { if (value < 1 || value > KZ_MAX_LANES) return fail(ctx, KZ_ERR_INVALID, "lanes must be 1.." + std::to_string(KZ_MAX_LANES)); ctx->lanes = value; return KZ_OK; }
     if (k == "pool_log2") { if (value < 10 || value > 26) return fail(ctx, KZ_ERR_INVALID, "pool_log2 must be 10..26"); ctx->pool_cap = 1u << value; return KZ_OK; }
     if (k == "spp_group") { if (value < 1) return fail(ctx, KZ_ERR_INVALID, "spp_group must be >= 1"); ctx->spp_group = value; return KZ_OK; }
+    if (k == "primary_hint") { if (value < 0 || value > 2) return fail(ctx, KZ_ERR_INVALID, "primary_hint must be 0, 1 or 2"); ctx->primary_hint = value; return KZ_OK; }
     return fail(ctx, KZ_ERR_INVALID, "unknown option \"" + k + "\"");
 }
 
@@ -1090,6 +1125,7 @@ int kzgpu_stats(kzgpu_ctx *ctx, kz_stats *out) {
             KzControl c;
             KZ_CUDA(ctx, cudaMemcpy(&c, L.ctl, sizeof(c), cudaMemcpyDeviceToHost));
             out->paths += c.paths; out->rays_extension += c.rays_ext; out->rays_shadow += c.rays_shadow; out->vertices += c.vertices;
+            out->rays_seeded += c.rays_seeded;
         }
         out->kernel_launches += d.launches;
         out->ms_trace = std::max(out->ms_trace, d.ms[CAT_TRACE]);
@@ -1109,7 +1145,7 @@ int kzgpu_stats_reset(kzgpu_ctx *ctx) {
         fold_events(d);
         for (double &m : d.ms) m = 0; d.launches = 0;
         /* keep queue state, zero the counters */
-        for (Lane &L : d.lane) KZ_CUDA(ctx, cudaMemset(reinterpret_cast<char *>(L.ctl) + offsetof(KzControl, paths), 0, 4 * sizeof(unsigned long long)));
+        for (Lane &L : d.lane) KZ_CUDA(ctx, cudaMemset(reinterpret_cast<char *>(L.ctl) + offsetof(KzControl, paths), 0, 5 * sizeof(unsigned long long)));
     }
     return KZ_OK;
 }

@@ -39,7 +39,7 @@ struct KzControl {
     uint32_t n_class[KZ_NUM_CLASSES];     /* material-class queue counts                    */
     uint32_t head_ext, head_shadow, head_trace;   /* persistent-fetch cursors               */
     uint32_t pad[1];
-    unsigned long long paths, rays_ext, rays_shadow, vertices;
+    unsigned long long paths, rays_ext, rays_shadow, vertices, rays_seeded;
 };
 
 struct KzQueues {
@@ -99,17 +99,19 @@ __device__ __forceinline__ uint32_t kz_fetch32(uint32_t *cursor) {
 }
 
 __device__ __forceinline__ void kz_flush_counters(KzControl *ctl, const KzCounters &c) {
-    unsigned long long e = c.rays_ext, s = c.rays_shadow, v = c.vertices;
+    unsigned long long e = c.rays_ext, s = c.rays_shadow, v = c.vertices, h = c.rays_seeded;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         e += __shfl_down_sync(KZ_FULL, e, o);
         s += __shfl_down_sync(KZ_FULL, s, o);
         v += __shfl_down_sync(KZ_FULL, v, o);
+        h += __shfl_down_sync(KZ_FULL, h, o);
     }
     if (kz_lane() == 0u) {
         if (e) atomicAdd(&ctl->rays_ext, e);
         if (s) atomicAdd(&ctl->rays_shadow, s);
         if (v) atomicAdd(&ctl->vertices, v);
+        if (h) atomicAdd(&ctl->rays_seeded, h);
     }
 }
 
@@ -123,6 +125,8 @@ __device__ __forceinline__ void kz_flush_counters(KzControl *ctl, const KzCounte
  *
  * Job: per-lane policy object.
  *   void begin(uint32_t item, KzRayIn &r)                   load the ray of work item `item`
+ *   void seed(const KzScene &sc, KzTrav &t)                 called right after the traversal of that ray was initialised: may preset
+ *                                                           its best hit (kz_trav_seed); not called for follow-up rays
  *   bool end(uint32_t item, const KzHit &h, KzRayIn &r)     consume the closest hit; return true and fill `r`
  *                                                           to continue the same item with a follow-up ray
  *   static constexpr bool kStopsEarly                       the job only asks WHETHER something opaque is hit (shadow rays)
@@ -177,6 +181,7 @@ __device__ __forceinline__ void kz_warp_trace(const KzScene &sc, const KzStackRe
                         KzRayIn r;
                         job.begin(item, r);
                         kz_trav_init(sc, t, r.ox, r.oy, r.oz, r.dx, r.dy, r.dz, r.tmin, r.tmax);
+                        job.seed(sc, t);
                         active = true;
                     }
                 }
@@ -316,12 +321,29 @@ struct KzExtendJob {
     static constexpr bool kStopsEarly = false;
     __device__ __forceinline__ bool stop(const KzScene &, const KzTrav &) { return false; }
     const KzScene &sc; const KzPathState &st; KzControl *ctl; const KzQueues &q; const uint32_t *queue;
+    uint2 *hint;                     /* primary rays: per film pixel the (geomID, primID) its last primary ray hit, or nullptr (no hints) */
     KzCounters cnt;
-    uint32_t slot;
+    uint32_t slot, n_seeded;
     KzHit first_hit; bool retraced;
     kz3 d;
-    __device__ KzExtendJob(const KzScene &s, const KzPathState &p, KzControl *c, const KzQueues &qq, const uint32_t *qu)
-        : sc(s), st(p), ctl(c), q(qq), queue(qu) { cnt.paths = cnt.rays_ext = cnt.rays_shadow = cnt.vertices = 0ull; }
+    __device__ KzExtendJob(const KzScene &s, const KzPathState &p, KzControl *c, const KzQueues &qq, const uint32_t *qu, uint2 *h)
+        : sc(s), st(p), ctl(c), q(qq), queue(qu), hint(h), n_seeded(0u) { cnt.paths = cnt.rays_ext = cnt.rays_shadow = cnt.vertices = cnt.rays_seeded = 0ull; }
+    /* hint slot of the path's pixel; ~0 for the padding lanes of k_raygen (pix = 0xFFFFFFFF lies outside every film) */
+    __device__ __forceinline__ size_t hint_index() const {
+        const uint32_t pix = st.b[slot].smp.pix, px = pix & 0xFFFFu, py = pix >> 16;
+        if (px >= (uint32_t)sc.camera.width || py >= (uint32_t)sc.camera.height) return ~(size_t)0;
+        return (size_t)py * (uint32_t)sc.camera.width + px;
+    }
+    /* One triangle covers several pixels and every pixel is sampled many times, so the triangle the pixel's last primary ray hit is
+     * usually hit again: as the preset best hit it lets the node step cull with its t from the root on, instead of walking every
+     * box along the ray up to the hit.  The hit found is the same either way (kz_trav_seed). */
+    __device__ __forceinline__ void seed(const KzScene &s, KzTrav &t) {
+        if (!FIRST || hint == nullptr) return;
+        const size_t i = hint_index();
+        if (i == ~(size_t)0) return;
+        const uint2 h = hint[i];
+        n_seeded += kz_trav_seed(s, t, h.x, h.y) ? 1u : 0u;
+    }
     __device__ __forceinline__ void begin(uint32_t item, KzRayIn &r) {
         slot = queue[item];
         const KzRayRec ray = st.a[slot].ray;
@@ -335,6 +357,9 @@ struct KzExtendJob {
         cnt.rays_ext += 1;
         KzHit h = hit;
         if (FIRST) {
+            /* the hint for the pixel's next sample: what this first trace hit (a miss clears it).  Samples of one pixel in flight
+             * together race on the slot; whichever store lands, it is a triangle (or none) and only ever a hint. */
+            if (hint != nullptr && !retraced) { const size_t i = hint_index(); if (i != ~(size_t)0) hint[i] = make_uint2(h.geom, h.prim); }
             if (retraced) { if (h.geom == KZ_INVALID_ID) h = first_hit; }     /* a miss keeps the light hit */
             else if (h.geom != KZ_INVALID_ID && sc.integrator.type == KZ_INTEGRATOR_PATH_MIS) {
                 const uint32_t fl = sc.meshes[h.geom].flags;
@@ -355,11 +380,13 @@ struct KzExtendJob {
     }
 };
 
+/* hint: k_extend<true> only (primary rays), nullptr = no hints */
 template <bool FIRST>
-__global__ void __launch_bounds__(KZ_TRACE_THREADS, KZ_TRACE_MIN_BLOCKS) k_extend(KzScene sc, KzPathState st, KzControl *ctl, KzQueues q, int cur) {
+__global__ void __launch_bounds__(KZ_TRACE_THREADS, KZ_TRACE_MIN_BLOCKS) k_extend(KzScene sc, KzPathState st, KzControl *ctl, KzQueues q, int cur, uint2 *hint) {
     const KzStackRef stk = kz_trav_shared_init();
-    KzExtendJob<FIRST> job(sc, st, ctl, q, q.ext[cur]);
+    KzExtendJob<FIRST> job(sc, st, ctl, q, q.ext[cur], FIRST ? hint : nullptr);
     kz_warp_trace(sc, stk, &ctl->head_ext, kz_ext_count(ctl, cur), job);
+    job.cnt.rays_seeded = job.n_seeded;
     kz_flush_counters(ctl, job.cnt);
 }
 
@@ -381,7 +408,7 @@ __global__ void __launch_bounds__(KZ_SHADE_THREADS, (CLS == KZ_CLASS_DIFFUSE ? K
     const uint32_t n = ctl->n_class[CLS];
     const uint32_t *queue = q.cls[CLS];
     const uint32_t stride = gridDim.x * blockDim.x;
-    KzCounters cnt; cnt.paths = cnt.rays_ext = cnt.rays_shadow = cnt.vertices = 0ull;
+    KzCounters cnt; cnt.paths = cnt.rays_ext = cnt.rays_shadow = cnt.vertices = cnt.rays_seeded = 0ull;
 #if KZ_SHADE_BLOCK_PUSH
     /* queue space for the whole CTA with ONE packed atomic per iteration (the counter is a single address: 1.8 M warp-level
      * atomics per frame serialise in the L2) */
@@ -465,9 +492,10 @@ struct KzWalk {
 struct KzShadowJob {
     static constexpr bool kStopsEarly = true;
     __device__ __forceinline__ bool stop(const KzScene &s, const KzTrav &t) { return KzWalk::settles(s, t); }
+    __device__ __forceinline__ void seed(const KzScene &, KzTrav &) {}
     const KzScene &sc; const KzPathState &st; const uint32_t *queue;
     KzCounters cnt; uint32_t slot; KzWalk walk;
-    __device__ KzShadowJob(const KzScene &s, const KzPathState &p, const uint32_t *qu) : sc(s), st(p), queue(qu) { cnt.paths = cnt.rays_ext = cnt.rays_shadow = cnt.vertices = 0ull; }
+    __device__ KzShadowJob(const KzScene &s, const KzPathState &p, const uint32_t *qu) : sc(s), st(p), queue(qu) { cnt.paths = cnt.rays_ext = cnt.rays_shadow = cnt.vertices = cnt.rays_seeded = 0ull; }
     __device__ __forceinline__ void begin(uint32_t item, KzRayIn &r) {
         slot = queue[item];
         const KzF4 so = st.a[slot].ray.o;
@@ -574,6 +602,7 @@ __global__ void __launch_bounds__(KZ_SHADE_THREADS) k_accumulate(KzScene sc, KzP
 struct KzTraceJob {
     static constexpr bool kStopsEarly = false;
     __device__ __forceinline__ bool stop(const KzScene &, const KzTrav &) { return false; }
+    __device__ __forceinline__ void seed(const KzScene &, KzTrav &) {}
     const KzF4 *rays; float *hits;
     __device__ __forceinline__ void begin(uint32_t item, KzRayIn &r) {
         const KzU4 a = kz_load_u4(rays + 2 * (size_t)item), b = kz_load_u4(rays + 2 * (size_t)item + 1);
@@ -596,10 +625,11 @@ __global__ void __launch_bounds__(KZ_TRACE_THREADS, KZ_BATCH_MIN_BLOCKS) k_trace
 struct KzOccludedJob {
     static constexpr bool kStopsEarly = true;
     __device__ __forceinline__ bool stop(const KzScene &s, const KzTrav &t) { return KzWalk::settles(s, t); }
+    __device__ __forceinline__ void seed(const KzScene &, KzTrav &) {}
     const KzScene &sc; const KzF4 *rays; float eps; uint8_t *occ, *segments;
     KzCounters cnt; KzWalk walk;
     __device__ KzOccludedJob(const KzScene &s, const KzF4 *r, float e, uint8_t *o, uint8_t *sg) : sc(s), rays(r), eps(e), occ(o), segments(sg) {
-        cnt.paths = cnt.rays_ext = cnt.rays_shadow = cnt.vertices = 0ull;
+        cnt.paths = cnt.rays_ext = cnt.rays_shadow = cnt.vertices = cnt.rays_seeded = 0ull;
     }
     __device__ __forceinline__ void begin(uint32_t item, KzRayIn &r) {
         const KzU4 a = kz_load_u4(rays + 2 * (size_t)item), b = kz_load_u4(rays + 2 * (size_t)item + 1);

@@ -45,7 +45,7 @@ struct KzPathState {
 KZ_HD KzHitRec mk_hit_rec(const KzHit &h) { KzHitRec r; r.t = h.t; r.u = h.u; r.v = h.v; r.prim = h.prim; r.geom = h.geom; r.pad0 = r.pad1 = r.pad2 = 0u; return r; }
 
 struct KzCounters {
-    unsigned long long paths, rays_ext, rays_shadow, vertices;
+    unsigned long long paths, rays_ext, rays_shadow, vertices, rays_seeded;     /* rays_seeded: primary rays that started from a hit hint */
 };
 
 #define KZ_SHADE_CONTINUE 1u   /* extension ray written, path goes to the next extend pass */

@@ -344,14 +344,42 @@ KZ_HD bool kz_trav_tri(const KzScene &sc, KzTrav &t) {
     return false;
 }
 
+/* Presets the best hit of a freshly initialised traversal with triangle `prim` of mesh `geom` (a hint, e.g. what this ray's pixel
+ * hit last time) if the ray hits it; returns true if it did.  An index out of range, or KZ_INVALID_ID, leaves the traversal as it was.
+ *
+ * The closest hit the traversal returns does not change, so a wrong or stale hint costs time, never correctness:
+ *   - kz_trav_tri keeps the minimum of (t, geomID, primID) over the triangles it accepts, and kz_pluecker accepts t <= tfar
+ *     inclusively, so the true closest triangle -- whose t is <= the seed's -- still becomes the best hit when it is tested, and a
+ *     tie at equal t still goes to the smaller (geomID, primID);
+ *   - the node step culls with cmax - cmin >= 0 = "may hit" on conservative boxes, so with tfar = the seed's t it still visits every
+ *     node that holds a triangle hit at t <= tfar, the true closest one included;
+ *   - if the seed is the closest triangle itself, its t, u, v must be the bits the traversal computes for it.  They are: the vertices
+ *     are read from the shading records (KzVertex px|py|pz through the index record), which are the very floats, in the very order,
+ *     that the accel's 48-byte triangle record was gathered from (k_gather_tris, KzHostScene::flatten; both builders copy them
+ *     unchanged), and the test is the same kz_pluecker with the same tnear (t.tmin) and tfar (the ray's tmax). */
+KZ_HD bool kz_trav_seed(const KzScene &sc, KzTrav &t, uint32_t geom, uint32_t prim) {
+    if (geom >= sc.n_meshes || t.ng_y == 0u) return false;          /* kz_trav_init made it an immediate miss (NaN ray, empty accel) */
+    const KzMeshRec &m = sc.meshes[geom];
+    if (prim >= m.n_triangles) return false;
+    const KzU4 ix = kz_load_u4(sc.indices + (m.index_offset + prim));
+    const KzVertex *vb = sc.vertices + m.vertex_offset;
+    const KzU4 a = kz_load_u4(vb + ix.x), b = kz_load_u4(vb + ix.y), c = kz_load_u4(vb + ix.z);      /* px, py, pz, (u: unused) */
+    float tt, u, v;
+    if (!kz_pluecker(t.ox, t.oy, t.oz, t.dx, t.dy, t.dz, t.tmin, t.best.t, a, b, c, tt, u, v)) return false;
+    t.best.t = tt; t.best.u = u; t.best.v = v; t.best.geom = geom; t.best.prim = prim;
+    return true;
+}
+
 /* The plain per-ray loop.  `stk` gives the shared-memory short stack on the device; on the host
- * everything lives in the local array.  any_hit: return at the first accepted hit. */
+ * everything lives in the local array.  any_hit: return at the first accepted hit.  (seed_geom, seed_prim): optional hint for the
+ * closest hit (kz_trav_seed). */
 KZ_HD KzHit kz_trace(const KzScene &sc, const KzStackRef &stk, float ox, float oy, float oz, float dx, float dy, float dz,
-                     float tmin, float tmax, bool any_hit) {
+                     float tmin, float tmax, bool any_hit, uint32_t seed_geom = KZ_INVALID_ID, uint32_t seed_prim = KZ_INVALID_ID) {
     KzTrav t;
     KzLocalStack ls;
     kz_trav_init(sc, t, ox, oy, oz, dx, dy, dz, tmin, tmax);
     if (sc.n_nodes == 0) return t.best;
+    if (!any_hit) kz_trav_seed(sc, t, seed_geom, seed_prim);     /* an any-hit query would stop at the seed */
     for (;;) {
         if (t.ng_y > 0x00FFFFFFu) kz_trav_node(sc, t, stk, ls);
         while (t.tg_y != 0u) {

@@ -98,7 +98,7 @@ class Stats(C.Structure):
     _fields_ = [("paths", C.c_uint64), ("rays_extension", C.c_uint64), ("rays_shadow", C.c_uint64), ("vertices", C.c_uint64),
                 ("kernel_launches", C.c_uint64), ("ms_trace", C.c_double), ("ms_shade", C.c_double), ("ms_total", C.c_double),
                 ("bvh_nodes", C.c_uint64), ("bvh_bytes", C.c_uint64), ("ms_build", C.c_double),
-                ("ms_upload", C.c_double), ("ms_merge", C.c_double)]
+                ("ms_upload", C.c_double), ("ms_merge", C.c_double), ("rays_seeded", C.c_uint64)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
