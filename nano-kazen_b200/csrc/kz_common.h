@@ -142,7 +142,12 @@ KZ_HD kz3 to_world(const KzFrame &f, kz3 v) { return f.s * v.x + f.t * v.y + f.n
 KZ_HD kz3 reflect3(kz3 wi, kz3 n) { return 2 * dot(n, wi) * n - wi; }   /* common.cpp:536-538 */
 KZ_HD float luminance(kz3 c) { return c.x * 0.212671f + c.y * 0.715160f + c.z * 0.072169f; }
 KZ_HD float srgb_to_linear1(float v) { return v <= 0.04045f ? v * (1.0f / 12.92f) : powf((v + 0.055f) * (1.0f / 1.055f), 2.4f); }
-KZ_HD float linear_to_srgb1(float v) { return v <= 0.0031308f ? 12.92f * v : (1.0f + 0.055f) * powf(v, 1.0f / 2.4f) - 0.055f; }
+/* toSRGB (color.h) as the reference rounds it, for the resolve's 8-bit codes: the product is rounded before the subtraction (a
+ * contracted FFMA changes the code of some linear values), and the power is the double one rounded once, which gives glibc
+ * powf's code on all of (0.0031308, 1].  Runs once per pixel of a resolved frame, never in a render. */
+KZ_HD float linear_to_srgb1(float v) {
+    return v <= 0.0031308f ? kz_mul(12.92f, v) : kz_sub(kz_mul(1.0f + 0.055f, (float)pow((double)v, (double)(1.0f / 2.4f))), 0.055f);
+}
 KZ_HD bool color_valid(kz3 c) {   /* common.cpp:384-391 */
     return !(c.x < 0 || !isfinite(c.x) || c.y < 0 || !isfinite(c.y) || c.z < 0 || !isfinite(c.z));
 }
