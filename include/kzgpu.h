@@ -256,6 +256,32 @@ const char *kzgpu_last_error(const kzgpu_ctx *ctx);   /* ctx may be NULL: global
 int  kzgpu_scene_upload(kzgpu_ctx *ctx, const kz_scene_desc *scene);
 int  kzgpu_accel_build(kzgpu_ctx *ctx, int builder);
 
+/* Animation: change an uploaded scene in place, then refit its accel instead of uploading and building again.
+ * Like kzgpu_scene_upload and kzgpu_accel_build, these calls require that everything enqueued with kzgpu_render_device
+ * or kzgpu_trace_device has finished (synchronise the stream first); they do not wait for it themselves. */
+
+/* Replaces the vertex positions of mesh `mesh` of the uploaded scene, and its normals if `normals` != NULL.
+ * Each array holds 3 * n_vertices floats, laid out as in kz_mesh_desc, and may be a host or a device pointer.
+ * Topology, uvs, materials and lights are unchanged; an emitter's area CDF and the bounds of the invisible emitters
+ * are recomputed.  Passing normals for a mesh uploaded without normals is KZ_ERR_INVALID; an invalid call changes nothing.
+ * Entry points that need the accel return KZ_ERR_STATE until kzgpu_accel_refit or kzgpu_accel_build has run.
+ * The primary-hit hints are kept: any hint yields the same hits, and those of the last frame are the best guess. */
+int  kzgpu_mesh_update(kzgpu_ctx *ctx, int mesh, const float *positions, const float *normals);
+
+/* Refits the built accel to the current vertex positions on every device of the context.
+ * The tree is the same; the boxes, triangle records and traversal slack are recomputed, so trace and render return
+ * exactly what a fresh build over the new positions returns (the tree only decides how fast).  A tree built for very
+ * different positions traces slower: rebuild when the motion is large (DESIGN.md section 7 has measurements).
+ * Returns when done, like kzgpu_accel_build.  KZ_ERR_STATE if no accel was built since the last upload. */
+int  kzgpu_accel_refit(kzgpu_ctx *ctx);
+
+/* Replaces the camera.  width/height must equal the uploaded ones (the frame and the hints are sized by them). */
+int  kzgpu_camera_update(kzgpu_ctx *ctx, const kz_camera_desc *camera);
+
+/* Parity probe: copies device `device`'s accel (n_nodes 80-byte nodes, 3 * n_tris float4) to host buffers sized from
+ * kz_stats: n_nodes = bvh_nodes, n_tris = (bvh_bytes - 80 * bvh_nodes) / 48. */
+int  kzgpu_accel_dump(kzgpu_ctx *ctx, int device, void *nodes, void *tris);
+
 /* Closest-hit queries on host buffers (H2D + trace + D2H), shadow=1 uses the
  * shadow-ray variant of accel.cpp:100-104 (same closest-hit, u/v/prim still filled). */
 int  kzgpu_trace(kzgpu_ctx *ctx, int device, const kz_ray *rays, size_t n, int shadow, kz_hit *hits);

@@ -9,6 +9,7 @@
 #include "kz_host_scene.h"
 #include "kz_lbvh.cuh"
 #include "kz_ingest.cuh"
+#include "kz_refit.cuh"
 #include <cuda_runtime.h>
 #include <chrono>
 #include <cstdio>
@@ -57,6 +58,12 @@ struct Device {
     size_t hint_px = 0;
     bool hint_stale = true;
     cudaEvent_t splat_done = nullptr, merge_done = nullptr;   /* multi-device frame merge (k_frame_reduce) */
+    /* kzgpu_accel_refit: node boxes of the level below (kept between refits), its two result words (max |coordinate| as an ordered
+     * uint, a failed level check) and whether this accel's level layout was checked on this device */
+    KzBox *refit_boxes = nullptr;
+    size_t refit_cap = 0;
+    uint32_t *refit_flags = nullptr;
+    bool levels_checked = false;
     /* scratch for host-pointer entry points */
     void *scratch[3] = {nullptr, nullptr, nullptr};
     size_t scratch_bytes[3] = {0, 0, 0};
@@ -92,6 +99,7 @@ struct kzgpu_ctx {
     uint64_t bvh_nodes = 0, bvh_bytes = 0;
     double last_total_ms = 0;
     double ms_upload = 0;             /* wall time of the last kzgpu_scene_upload */
+    std::vector<uint32_t> levels;     /* wide-tree level l of the built accel = nodes [levels[l], levels[l + 1]); empty: not laid out by level */
     std::string error;
 };
 
@@ -500,7 +508,9 @@ int enqueue_render(const kzgpu_ctx *ctx, kzgpu_ctx *ectx, Device &d, const kz_re
 int check_ready(kzgpu_ctx *ctx, bool need_accel) {
     if (!ctx) return fail(nullptr, KZ_ERR_INVALID, "null context");
     if (!ctx->uploaded) return fail(ctx, KZ_ERR_STATE, "no scene uploaded");
-    if (need_accel && !ctx->built) return fail(ctx, KZ_ERR_STATE, "accel not built: call kzgpu_accel_build first");
+    if (need_accel && !ctx->built)
+        return fail(ctx, KZ_ERR_STATE, ctx->devs[0].has_accel ? "the vertices changed since the accel was built: call kzgpu_accel_refit or kzgpu_accel_build"
+                                                              : "accel not built: call kzgpu_accel_build first");
     return KZ_OK;
 }
 
@@ -587,6 +597,8 @@ void kzgpu_destroy(kzgpu_ctx *ctx) {
         for (cudaEvent_t e : d.free_events) cudaEventDestroy(e);
         free_all(d.scene_allocs); free_all(d.accel_allocs);
         if (d.hint) cudaFree(d.hint);
+        if (d.refit_boxes) cudaFree(d.refit_boxes);
+        if (d.refit_flags) cudaFree(d.refit_flags);
         for (Lane &L : d.lane) { free_all(L.allocs); cudaFree(L.ctl); if (L.done) cudaEventDestroy(L.done); if (L.stream) cudaStreamDestroy(L.stream); }
         for (int k = 0; k < 3; ++k) if (d.scratch[k]) cudaFree(d.scratch[k]);
         cudaFree(d.cursor);
@@ -639,6 +651,7 @@ int kzgpu_scene_upload(kzgpu_ctx *ctx, const kz_scene_desc *scene) {
         KZ_CUDA(ctx, cudaSetDevice(d.id));
         d.has_accel = false;
         d.hint_stale = true;
+        d.levels_checked = false;
         free_all(d.accel_allocs);
         int rc = upload_tables(ctx, d);
         if (rc) return rc;
@@ -679,6 +692,7 @@ int kzgpu_accel_build(kzgpu_ctx *ctx, int builder) {
         kzbvh::Built built;
         kzbvh::buildHostSah(tris, 0, built);
         if (built.depth > KZ_MAX_ACCEL_DEPTH) return fail(ctx, KZ_ERR_UNSUPPORTED, "accel deeper than the traversal stack allows");
+        if (!kz_refit_levels(built.nodes.data(), (uint32_t)built.nodes.size(), ctx->levels)) ctx->levels.clear();
         for (Device &d : ctx->devs) {
             KZ_CUDA(ctx, cudaSetDevice(d.id));
             if ((rc = upload_accel(ctx, d, built))) return rc;
@@ -696,6 +710,8 @@ int kzgpu_accel_build(kzgpu_ctx *ctx, int builder) {
         if (rc) return fail(ctx, rc, err);
         if (r.depth > KZ_MAX_ACCEL_DEPTH) return fail(ctx, KZ_ERR_UNSUPPORTED, "accel deeper than the traversal stack allows");
         d0.sc.nodes = r.nodes; d0.sc.tris = r.tris; d0.sc.n_nodes = r.n_nodes; d0.sc.n_tris = r.n_tris; d0.sc.scene_max_abs = r.max_abs;
+        ctx->levels = r.n_nodes ? r.level_first : std::vector<uint32_t>(1, 0u);
+        if (ctx->levels.back() != r.n_nodes) ctx->levels.clear();
         d0.has_accel = true;
         d0.launches += r.launches;
         ctx->bvh_nodes = r.n_nodes;
@@ -707,9 +723,174 @@ int kzgpu_accel_build(kzgpu_ctx *ctx, int builder) {
         }
         KZ_CUDA(ctx, cudaSetDevice(d0.id));
     }
-    for (Device &d : ctx->devs) d.hint_stale = true;
+    for (Device &d : ctx->devs) { d.hint_stale = true; d.levels_checked = false; }
     ctx->ms_build = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     ctx->built = true;
+    return KZ_OK;
+}
+
+int kzgpu_mesh_update(kzgpu_ctx *ctx, int mesh, const float *positions, const float *normals) {
+    if (!ctx) return fail(nullptr, KZ_ERR_INVALID, "null context");
+    if (!ctx->uploaded) return fail(ctx, KZ_ERR_STATE, "no scene uploaded");
+    KzHostScene &h = *ctx->hs;
+    if (mesh < 0 || mesh >= (int)h.meshes.size()) return fail(ctx, KZ_ERR_INVALID, "mesh index out of range");
+    if (!positions) return fail(ctx, KZ_ERR_INVALID, "null positions");
+    KzMeshRec &r = h.meshes[(size_t)mesh];
+    if (normals && !(r.flags & KZ_MESH_HAS_NORMALS)) return fail(ctx, KZ_ERR_INVALID, "normals given for a mesh uploaded without normals");
+    const uint32_t nv = (uint32_t)(((size_t)mesh + 1 < h.meshes.size() ? (uint64_t)h.meshes[(size_t)mesh + 1].vertex_offset : h.total_vertices) - r.vertex_offset);
+    Device &d0 = ctx->devs[0];
+    KZ_CUDA(ctx, cudaSetDevice(d0.id));
+    /* an emitter's area CDF, normalisation and bounds are recomputed on the host from its new positions (read back if they are a
+     * device array, as kzgpu_scene_upload does) and its index records (read back from HBM); nothing is written before this succeeded */
+    std::vector<float> cdf, bounds(6);
+    float inv_area = 0.f;
+    size_t light_k = 0;
+    if (r.flags & KZ_MESH_IS_LIGHT) {
+        std::vector<float> pos;
+        const float *hp = positions;
+        if (is_device_ptr(positions)) {
+            pos.resize((size_t)nv * 3);
+            KZ_CUDA(ctx, cudaMemcpy(pos.data(), positions, (size_t)nv * 12, cudaMemcpyDeviceToHost));
+            hp = pos.data();
+        }
+        std::vector<KzU4> rec(r.n_triangles);
+        KZ_CUDA(ctx, cudaMemcpyAsync(rec.data(), d0.sc.indices + r.index_offset, (size_t)r.n_triangles * sizeof(KzU4), cudaMemcpyDeviceToHost, d0.stream));
+        KZ_CUDA(ctx, cudaStreamSynchronize(d0.stream));
+        std::vector<uint32_t> idx((size_t)r.n_triangles * 3);
+        for (size_t f = 0; f < rec.size(); ++f) { idx[3 * f] = rec[f].x; idx[3 * f + 1] = rec[f].y; idx[3 * f + 2] = rec[f].z; }
+        cdf.resize((size_t)r.n_triangles + 1);
+        KzHostScene::emitter_tables(hp, idx.data(), r.n_triangles, cdf.data(), inv_area, bounds.data());
+        while (h.light_meshes[light_k] != mesh) ++light_k;
+    }
+    /* from here on the scene changes: the accel no longer matches it until a refit or a build */
+    ctx->built = false;
+    /* vertex records of device 0: host arrays are staged with one copy each, device arrays read in place */
+    {
+        std::vector<void *> temp;
+        const float *src[2] = {positions, normals};
+        cudaError_t e = cudaSuccess;
+        for (int k = 0; k < 2 && e == cudaSuccess; ++k) {
+            if (!src[k] || is_device_ptr(src[k])) continue;
+            float *stage = nullptr;
+            int rc = temp_alloc(ctx, temp, (size_t)nv * 3, d0.stream, &stage);
+            if (rc) { temp_free_all(temp, d0.stream); return rc; }
+            e = cudaMemcpyAsync(stage, src[k], (size_t)nv * 12, cudaMemcpyHostToDevice, d0.stream);
+            src[k] = stage;
+        }
+        if (e == cudaSuccess && nv) {
+            k_update_vertices<<<grid_for(nv, 256, d0.sm_count), 256, 0, d0.stream>>>(src[0], src[1], nv, const_cast<KzVertex *>(d0.sc.vertices) + r.vertex_offset);
+            ++d0.launches;
+            e = cudaGetLastError();
+        }
+        if (e == cudaSuccess) e = cudaStreamSynchronize(d0.stream);
+        temp_free_all(temp, d0.stream);
+        if (e != cudaSuccess) return fail(ctx, KZ_ERR_CUDA, std::string("mesh update: ") + cudaGetErrorString(e));
+    }
+    if (r.flags & KZ_MESH_IS_LIGHT) {
+        std::copy(cdf.begin(), cdf.end(), h.light_cdf.begin() + r.cdf_offset);
+        r.inv_area = inv_area;
+        std::copy(bounds.begin(), bounds.end(), h.light_bounds.begin() + 6 * light_k);
+        h.invisible_light_bounds();
+    }
+    for (Device &d : ctx->devs) {
+        KZ_CUDA(ctx, cudaSetDevice(d.id));
+        if (&d != &d0 && nv)
+            KZ_CUDA(ctx, cudaMemcpyPeerAsync(const_cast<KzVertex *>(d.sc.vertices) + r.vertex_offset, d.id, d0.sc.vertices + r.vertex_offset, d0.id, (size_t)nv * sizeof(KzVertex), d.stream));
+        if (r.flags & KZ_MESH_IS_LIGHT) {
+            KZ_CUDA(ctx, cudaMemcpyAsync(const_cast<KzMeshRec *>(d.sc.meshes), h.meshes.data(), h.meshes.size() * sizeof(KzMeshRec), cudaMemcpyHostToDevice, d.stream));
+            KZ_CUDA(ctx, cudaMemcpyAsync(const_cast<float *>(d.sc.light_cdf), h.light_cdf.data(), h.light_cdf.size() * sizeof(float), cudaMemcpyHostToDevice, d.stream));
+            for (int a = 0; a < 3; ++a) { d.sc.inv_light_lo[a] = h.sc.inv_light_lo[a]; d.sc.inv_light_hi[a] = h.sc.inv_light_hi[a]; }
+        }
+        KZ_CUDA(ctx, cudaStreamSynchronize(d.stream));
+    }
+    KZ_CUDA(ctx, cudaSetDevice(d0.id));
+    return KZ_OK;
+}
+
+int kzgpu_accel_refit(kzgpu_ctx *ctx) {
+    if (!ctx) return fail(nullptr, KZ_ERR_INVALID, "null context");
+    if (!ctx->uploaded) return fail(ctx, KZ_ERR_STATE, "no scene uploaded");
+    for (const Device &d : ctx->devs)
+        if (!d.has_accel) return fail(ctx, KZ_ERR_STATE, "no accel built since the last upload: call kzgpu_accel_build first");
+    if (ctx->levels.empty()) return fail(ctx, KZ_ERR_STATE, "the accel is not laid out level by level: call kzgpu_accel_build");
+    const std::vector<uint32_t> &L = ctx->levels;
+    const int nl = (int)L.size() - 1;
+    /* once per built accel and device: every internal child one level down, every triangle in the record array */
+    for (Device &d : ctx->devs) {
+        KZ_CUDA(ctx, cudaSetDevice(d.id));
+        if (!d.refit_flags) KZ_CUDA(ctx, cudaMalloc(&d.refit_flags, 2 * sizeof(uint32_t)));
+        KZ_CUDA(ctx, cudaMemsetAsync(d.refit_flags, 0, 2 * sizeof(uint32_t), d.stream));
+        if (d.levels_checked || d.sc.n_nodes == 0) continue;
+        for (int l = 0; l < nl; ++l) {
+            const uint32_t next_hi = l + 1 < nl ? L[(size_t)l + 2] : L[(size_t)l + 1];
+            k_refit_check<<<grid_for(L[(size_t)l + 1] - L[(size_t)l], 256, d.sm_count), 256, 0, d.stream>>>(d.sc.nodes, L[(size_t)l], L[(size_t)l + 1], L[(size_t)l + 1], next_hi,
+                                                                                                          d.sc.n_tris, d.refit_flags + 1);
+            ++d.launches;
+        }
+        KZ_CUDA(ctx, cudaGetLastError());
+    }
+    for (Device &d : ctx->devs) {
+        if (d.levels_checked || d.sc.n_nodes == 0) continue;
+        uint32_t bad = 0;
+        KZ_CUDA(ctx, cudaSetDevice(d.id));
+        KZ_CUDA(ctx, cudaMemcpyAsync(&bad, d.refit_flags + 1, 4, cudaMemcpyDeviceToHost, d.stream));
+        KZ_CUDA(ctx, cudaStreamSynchronize(d.stream));
+        if (bad || L.back() != d.sc.n_nodes) return fail(ctx, KZ_ERR_STATE, "the accel is not laid out level by level: call kzgpu_accel_build");
+        d.levels_checked = true;
+    }
+    /* every device refits its own copy (the same records and vertices everywhere, exact arithmetic: the same bytes) */
+    for (Device &d : ctx->devs) {
+        if (d.sc.n_nodes == 0) continue;
+        KZ_CUDA(ctx, cudaSetDevice(d.id));
+        if (d.refit_cap < d.sc.n_nodes) {
+            if (d.refit_boxes) { cudaFree(d.refit_boxes); d.refit_boxes = nullptr; d.refit_cap = 0; }
+            KZ_CUDA(ctx, cudaMalloc(&d.refit_boxes, (size_t)d.sc.n_nodes * sizeof(KzBox)));
+            d.refit_cap = d.sc.n_nodes;
+        }
+        KzF4 *tris = const_cast<KzF4 *>(d.sc.tris);
+        KzNode8 *nodes = const_cast<KzNode8 *>(d.sc.nodes);
+        k_refit_tris<<<grid_for(d.sc.n_tris, 256, d.sm_count), 256, 0, d.stream>>>(d.sc.meshes, d.sc.vertices, d.sc.indices, tris, d.sc.n_tris, d.refit_flags);
+        for (int l = nl - 1; l >= 0; --l)
+            k_refit_level<<<grid_for(L[(size_t)l + 1] - L[(size_t)l], 128, d.sm_count), 128, 0, d.stream>>>(nodes, tris, d.refit_boxes, L[(size_t)l], L[(size_t)l + 1]);
+        d.launches += 1 + (uint64_t)nl;
+        KZ_CUDA(ctx, cudaGetLastError());
+    }
+    for (Device &d : ctx->devs) {
+        if (d.sc.n_nodes == 0) continue;
+        uint32_t mabs = 0;
+        KZ_CUDA(ctx, cudaSetDevice(d.id));
+        KZ_CUDA(ctx, cudaMemcpyAsync(&mabs, d.refit_flags, 4, cudaMemcpyDeviceToHost, d.stream));
+        KZ_CUDA(ctx, cudaStreamSynchronize(d.stream));
+        d.sc.scene_max_abs = kzlbvh::ord2f(mabs);
+    }
+    KZ_CUDA(ctx, cudaSetDevice(ctx->devs[0].id));
+    ctx->built = true;
+    return KZ_OK;
+}
+
+int kzgpu_camera_update(kzgpu_ctx *ctx, const kz_camera_desc *camera) {
+    if (!ctx) return fail(nullptr, KZ_ERR_INVALID, "null context");
+    if (!ctx->uploaded) return fail(ctx, KZ_ERR_STATE, "no scene uploaded");
+    if (!camera) return fail(ctx, KZ_ERR_INVALID, "null camera");
+    if (camera->width <= 0 || camera->height <= 0 || camera->width > 65535 || camera->height > 65535) return fail(ctx, KZ_ERR_INVALID, "camera size out of range");
+    if (camera->width != ctx->hs->sc.camera.width || camera->height != ctx->hs->sc.camera.height)
+        return fail(ctx, KZ_ERR_INVALID, "camera size differs from the uploaded one (the frame and the primary-hit hints are sized by it)");
+    ctx->hs->sc.camera = *camera;
+    for (Device &d : ctx->devs) d.sc.camera = *camera;
+    return KZ_OK;
+}
+
+int kzgpu_accel_dump(kzgpu_ctx *ctx, int device, void *nodes, void *tris) {
+    if (!ctx) return fail(nullptr, KZ_ERR_INVALID, "null context");
+    if (!ctx->uploaded) return fail(ctx, KZ_ERR_STATE, "no scene uploaded");
+    Device *d;
+    int rc;
+    if ((rc = select(ctx, device, &d))) return rc;
+    if (!d->has_accel) return fail(ctx, KZ_ERR_STATE, "no accel built since the last upload");
+    if ((d->sc.n_nodes && !nodes) || (d->sc.n_tris && !tris)) return fail(ctx, KZ_ERR_INVALID, "null buffer");
+    if (d->sc.n_nodes) KZ_CUDA(ctx, cudaMemcpyAsync(nodes, d->sc.nodes, (size_t)d->sc.n_nodes * sizeof(KzNode8), cudaMemcpyDeviceToHost, d->stream));
+    if (d->sc.n_tris) KZ_CUDA(ctx, cudaMemcpyAsync(tris, d->sc.tris, (size_t)d->sc.n_tris * 3 * sizeof(KzF4), cudaMemcpyDeviceToHost, d->stream));
+    KZ_CUDA(ctx, cudaStreamSynchronize(d->stream));
     return KZ_OK;
 }
 

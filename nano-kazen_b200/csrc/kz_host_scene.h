@@ -16,6 +16,7 @@ struct KzHostScene {
     std::vector<float> light_cdf;
     std::vector<KzU4> indices;
     std::vector<int32_t> light_meshes;
+    std::vector<float> light_bounds;    /* per emitter (light_meshes order): lo[3], hi[3] of its vertices */
     std::vector<kz_bsdf_desc> bsdfs;
     std::vector<kz_texture_desc> textures;
     std::vector<KzImageRec> images;
@@ -85,7 +86,6 @@ struct KzHostScene {
         }
         uint64_t voff = 0, foff = 0;
         sc.n_invisible_lights = 0;
-        for (int a = 0; a < 3; ++a) { sc.inv_light_lo[a] = kz_u2f(0x7f800000u); sc.inv_light_hi[a] = kz_u2f(0xff800000u); }
         for (uint32_t g = 0; g < d->n_meshes; ++g) {
             const kz_mesh_desc &m = d->meshes[g];
             if (!m.positions || !m.indices) { error = "mesh buffers missing"; return false; }
@@ -118,29 +118,10 @@ struct KzHostScene {
                 r.flags |= KZ_MESH_IS_LIGHT;
                 if (d->lights[m.light].primary_visibility) r.flags |= KZ_MESH_LIGHT_VISIBLE;
                 else ++sc.n_invisible_lights;
-                /* Mesh::activate + DiscretePDF::normalize */
                 r.cdf_offset = (uint32_t)light_cdf.size();
-                light_cdf.push_back(0.0f);
-                for (uint32_t f = 0; f < m.n_triangles; ++f) {
-                    const float *p0 = m.positions + 3 * (size_t)m.indices[3 * f], *p1 = m.positions + 3 * (size_t)m.indices[3 * f + 1],
-                                *p2 = m.positions + 3 * (size_t)m.indices[3 * f + 2];
-                    if (!d->lights[m.light].primary_visibility)        /* bounds of the invisible emitters: shadow rays stop early outside them */
-                        for (const float *q : {p0, p1, p2})
-                            for (int a = 0; a < 3; ++a) { sc.inv_light_lo[a] = fminf(sc.inv_light_lo[a], q[a]); sc.inv_light_hi[a] = fmaxf(sc.inv_light_hi[a], q[a]); }
-                    kz3 e1 = mk3(kz_sub(p1[0], p0[0]), kz_sub(p1[1], p0[1]), kz_sub(p1[2], p0[2]));
-                    kz3 e2 = mk3(kz_sub(p2[0], p0[0]), kz_sub(p2[1], p0[1]), kz_sub(p2[2], p0[2]));
-                    kz3 c = mk3(kz_sub(kz_mul(e1.y, e2.z), kz_mul(e1.z, e2.y)), kz_sub(kz_mul(e1.z, e2.x), kz_mul(e1.x, e2.z)),
-                                kz_sub(kz_mul(e1.x, e2.y), kz_mul(e1.y, e2.x)));
-                    float n2 = kz_add(kz_add(kz_mul(c.x, c.x), kz_mul(c.y, c.y)), kz_mul(c.z, c.z));
-                    float area = kz_mul(0.5f, kz_sqrt(n2));
-                    light_cdf.push_back(kz_add(light_cdf.back(), area));
-                }
-                float sum = light_cdf.back();
-                if (sum > 0) {
-                    r.inv_area = kz_div(1.0f, sum);
-                    for (size_t k = r.cdf_offset + 1; k < light_cdf.size(); ++k) light_cdf[k] = kz_mul(light_cdf[k], r.inv_area);
-                    light_cdf.back() = 1.0f;
-                } else r.inv_area = 0.f;
+                light_cdf.resize(light_cdf.size() + m.n_triangles + 1);
+                light_bounds.resize(light_bounds.size() + 6);
+                emitter_tables(m.positions, m.indices, m.n_triangles, light_cdf.data() + r.cdf_offset, r.inv_area, light_bounds.data() + light_bounds.size() - 6);
                 light_meshes.push_back((int32_t)g);
             }
             for (uint32_t f = 0; geometry && f < m.n_triangles; ++f) {
@@ -156,6 +137,7 @@ struct KzHostScene {
             voff += m.n_vertices; foff += m.n_triangles;
         }
         total_vertices = voff; total_triangles = foff;
+        invisible_light_bounds();
         sc.n_meshes = d->n_meshes;
         sc.n_light_meshes = (int32_t)light_meshes.size();
         sc.background = d->background;
@@ -181,6 +163,45 @@ struct KzHostScene {
         }
         finalize();
         return true;
+    }
+
+    /* Mesh::activate + DiscretePDF::normalize (mesh.cpp:24-45, dpdf.h:35-81) for an emitter of n_triangles > 0 triangles: its area CDF
+     * (n_triangles + 1 floats from 0 to 1), the normalisation 1 / sum(area) and the bounds of the vertices its triangles use.
+     * kzgpu_scene_upload (through flatten) and kzgpu_mesh_update both come here, so an updated emitter samples as a freshly uploaded one. */
+    static void emitter_tables(const float *positions, const uint32_t *idx, uint32_t n_triangles, float *cdf, float &inv_area, float *bounds) {
+        for (int a = 0; a < 3; ++a) { bounds[a] = kz_u2f(0x7f800000u); bounds[3 + a] = kz_u2f(0xff800000u); }
+        cdf[0] = 0.0f;
+        for (uint32_t f = 0; f < n_triangles; ++f) {
+            const float *p0 = positions + 3 * (size_t)idx[3 * (size_t)f], *p1 = positions + 3 * (size_t)idx[3 * (size_t)f + 1],
+                        *p2 = positions + 3 * (size_t)idx[3 * (size_t)f + 2];
+            for (const float *q : {p0, p1, p2})
+                for (int a = 0; a < 3; ++a) { bounds[a] = fminf(bounds[a], q[a]); bounds[3 + a] = fmaxf(bounds[3 + a], q[a]); }
+            kz3 e1 = mk3(kz_sub(p1[0], p0[0]), kz_sub(p1[1], p0[1]), kz_sub(p1[2], p0[2]));
+            kz3 e2 = mk3(kz_sub(p2[0], p0[0]), kz_sub(p2[1], p0[1]), kz_sub(p2[2], p0[2]));
+            kz3 c = mk3(kz_sub(kz_mul(e1.y, e2.z), kz_mul(e1.z, e2.y)), kz_sub(kz_mul(e1.z, e2.x), kz_mul(e1.x, e2.z)),
+                        kz_sub(kz_mul(e1.x, e2.y), kz_mul(e1.y, e2.x)));
+            float n2 = kz_add(kz_add(kz_mul(c.x, c.x), kz_mul(c.y, c.y)), kz_mul(c.z, c.z));
+            float area = kz_mul(0.5f, kz_sqrt(n2));
+            cdf[f + 1] = kz_add(cdf[f], area);
+        }
+        const float sum = cdf[n_triangles];
+        if (sum > 0) {
+            inv_area = kz_div(1.0f, sum);
+            for (uint32_t k = 1; k <= n_triangles; ++k) cdf[k] = kz_mul(cdf[k], inv_area);
+            cdf[n_triangles] = 1.0f;
+        } else inv_area = 0.f;
+    }
+
+    /* sc.inv_light_lo / hi: the bounds of the invisible emitters' vertices (shadow rays stop early outside them, KzWalk::settles) */
+    void invisible_light_bounds() {
+        for (int a = 0; a < 3; ++a) { sc.inv_light_lo[a] = kz_u2f(0x7f800000u); sc.inv_light_hi[a] = kz_u2f(0xff800000u); }
+        for (size_t k = 0; k < light_meshes.size(); ++k) {
+            if (meshes[(size_t)light_meshes[k]].flags & KZ_MESH_LIGHT_VISIBLE) continue;
+            for (int a = 0; a < 3; ++a) {
+                sc.inv_light_lo[a] = fminf(sc.inv_light_lo[a], light_bounds[6 * k + a]);
+                sc.inv_light_hi[a] = fmaxf(sc.inv_light_hi[a], light_bounds[6 * k + 3 + a]);
+            }
+        }
     }
 
     size_t total_texels = 0;

@@ -1,6 +1,7 @@
 /* kz_ingest.cuh -- scene ingest and frame merge kernels (device side of kzgpu_scene_upload / kzgpu_render).
  *
  *   k_ingest_vertices   Mesh::m_V / m_N / m_UV (mesh.h:175-178: packed xyz / uv arrays) -> 32-byte KzVertex records
+ *   k_update_vertices   kzgpu_mesh_update: new positions (and normals) into existing KzVertex records, the other fields kept
  *   k_ingest_indices    Mesh::m_F -> 16-byte index records, validated against the vertex count
  *   k_ingest_texels     decoded rgb image -> float4 texels (level 0)
  *   k_gather_tris       (mesh table, vertex records, index records) -> the accel builders' triangle list in scene
@@ -25,6 +26,15 @@ __global__ void k_ingest_vertices(const float *pos, const float *nrm, const floa
         float4 *o = reinterpret_cast<float4 *>(out + i);
         o[0] = make_float4(v.px, v.py, v.pz, v.u);
         o[1] = make_float4(v.nx, v.ny, v.nz, v.v);
+    }
+}
+
+__global__ void k_update_vertices(const float *pos, const float *nrm, uint32_t n, KzVertex *out) {
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        float4 *o = reinterpret_cast<float4 *>(out + i);
+        const float4 a = o[0];
+        o[0] = make_float4(pos[3 * (size_t)i], pos[3 * (size_t)i + 1], pos[3 * (size_t)i + 2], a.w);
+        if (nrm) { const float4 b = o[1]; o[1] = make_float4(nrm[3 * (size_t)i], nrm[3 * (size_t)i + 1], nrm[3 * (size_t)i + 2], b.w); }
     }
 }
 

@@ -31,6 +31,7 @@ struct Result {
     float max_abs = 0.f;
     uint64_t launches = 0;
     int depth = 0;               /* wide-tree levels */
+    std::vector<uint32_t> level_first;   /* level l = nodes [level_first[l], level_first[l + 1]) (kzgpu_accel_refit) */
 };
 
 struct Box6 { float lo[3], hi[3]; };
@@ -515,6 +516,9 @@ inline int build(const kzbvh::Tri *d_tris, uint32_t n_tris_in, cudaStream_t s, s
     r.nodes = d_nodes; r.tris = d_out_tris; r.n_nodes = fin[0]; r.n_tris = fin[1];
     r.max_abs = ord2f(hb[6]);
     for (int l = 0; l < KZ_LBVH_MAX_LEVELS && fin[2 + l] != 0u; ++l) r.depth = l + 1;
+    /* level l + 1 is allocated (node_counter) while level l runs, so the levels are consecutive ranges in launch order */
+    r.level_first.assign(1, 0u);
+    for (int l = 0; l < r.depth; ++l) r.level_first.push_back(r.level_first.back() + fin[2 + l]);
     for (void *p : temp) cudaFreeAsync(p, s);
     cudaStreamSynchronize(s);
     if (fin[2 + KZ_LBVH_MAX_LEVELS] != 0u) { err = "lbvh: accel deeper than the traversal stack allows"; return KZ_ERR_UNSUPPORTED; }

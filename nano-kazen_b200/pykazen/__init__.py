@@ -163,6 +163,16 @@ def lookat(origin, target, up):
     return M.astype(np.float32)
 
 
+def fill_camera(c, width, height, fov, to_world, near=1e-4, far=1e4, thinlens=None):
+    """CameraDesc `c` of a perspective (thinlens = (aperture_radius, focus_distance): thin-lens) camera after Camera::activate"""
+    c.type = CAM_THINLENS if thinlens else CAM_PERSPECTIVE
+    c.width, c.height, c.near_clip, c.far_clip = width, height, near, far
+    c.sample_to_camera[:] = perspective_sample_to_camera(width, height, fov, near, far).reshape(-1).tolist()
+    c.camera_to_world[:] = np.asarray(to_world, np.float32).reshape(-1).tolist()
+    c.aperture_radius, c.focus_distance = thinlens if thinlens else (1.0, 0.0)
+    return c
+
+
 class SceneBuilder:
     """Assembles a kz_scene_desc; keeps every numpy buffer alive for the lifetime of the object."""
 
@@ -288,12 +298,7 @@ class SceneBuilder:
 
     # setup --------------------------------------------------------------------------------------
     def set_camera(self, width, height, fov, to_world, near=1e-4, far=1e4, thinlens=None):
-        c = self.camera
-        c.type = CAM_THINLENS if thinlens else CAM_PERSPECTIVE
-        c.width, c.height, c.near_clip, c.far_clip = width, height, near, far
-        c.sample_to_camera[:] = perspective_sample_to_camera(width, height, fov, near, far).reshape(-1).tolist()
-        c.camera_to_world[:] = np.asarray(to_world, np.float32).reshape(-1).tolist()
-        c.aperture_radius, c.focus_distance = thinlens if thinlens else (1.0, 0.0)
+        fill_camera(self.camera, width, height, fov, to_world, near, far, thinlens)
 
     def set_sampler(self, kind, sample_count, seed=1, resolution=4, tables=None):
         """Applies the constructors' rounding rules (sampler.cpp:83-93,178-189,275-289)."""
@@ -557,6 +562,39 @@ class Gpu(_Backend):
 
     def configure(self, key, value):
         self._call("configure", self.h, key.encode(), C.c_int(int(value)))
+
+    # animation: update -> refit -> render ---------------------------------------------------------
+    def mesh_update(self, mesh, positions, normals=None):
+        """new vertex positions (and normals) of mesh `mesh`: numpy arrays of 3 * n_vertices floats, or device pointers (ints, e.g. a
+        torch CUDA tensor's data_ptr()).  Trace and render need refit() (or a rebuild) afterwards."""
+        def ptr(a):
+            if a is None:
+                return None
+            if isinstance(a, (int, np.integer)):
+                return C.c_void_p(int(a))
+            a = np.ascontiguousarray(a, np.float32)
+            keep.append(a)
+            return a.ctypes.data_as(C.c_void_p)
+        keep = []
+        self._call("mesh_update", self.h, C.c_int(mesh), ptr(positions), ptr(normals))
+
+    def refit(self):
+        """refits the accel to the current vertex positions on every device (same tree, new boxes)"""
+        self._call("accel_refit", self.h)
+
+    def camera_update(self, width, height, fov, to_world, near=1e-4, far=1e4, thinlens=None):
+        """replaces the camera (arguments as SceneBuilder.set_camera; width / height must be the uploaded ones)"""
+        c = fill_camera(CameraDesc(), width, height, fov, to_world, near, far, thinlens)
+        self._call("camera_update", self.h, C.byref(c))
+
+    def accel_dump(self, device=0):
+        """device `device`'s accel: (nodes as raw (n_nodes, 80) uint8, triangle records as (n_tris, 3, 4) float32)"""
+        s = Stats()
+        self._call("stats", self.h, C.byref(s))
+        n_tris = (s.bvh_bytes - 80 * s.bvh_nodes) // 48
+        nodes = np.zeros((s.bvh_nodes, 80), np.uint8); tris = np.zeros((n_tris, 3, 4), np.float32)
+        self._call("accel_dump", self.h, C.c_int(device), nodes.ctypes.data_as(C.c_void_p), tris.ctypes.data_as(C.c_void_p))
+        return nodes, tris
 
     def render_host_ptr(self, spp_begin, spp_end, frame_ptr, clear=True, rect=None):
         """kzgpu_render into a caller-owned (pinned) host frame given by address"""
