@@ -10,6 +10,7 @@
 #include "kz_lbvh.cuh"
 #include "kz_ingest.cuh"
 #include "kz_refit.cuh"
+#include "kz_owner.h"
 #include <cuda_runtime.h>
 #include <chrono>
 #include <cstdio>
@@ -29,44 +30,50 @@ struct EvPair { cudaEvent_t a, b; int cat; };
 
 #define KZ_MAX_LANES 4
 struct Lane {
-    cudaStream_t stream = nullptr;   /* lane 1 only; lane 0 runs on the caller's stream */
-    cudaEvent_t done = nullptr;
+    Stream stream;                   /* lane 1.. only; lane 0 runs on the caller's stream */
+    Event done;
+    DevMem ctl_mem;
+    KzControl *ctl = nullptr;
     uint32_t pool_cap = 0;
+    DevMem pool[6 + KZ_NUM_CLASSES]; /* pool_cap slots each: the path state and the queues below */
     KzPathState st{};
     KzQueues q{};
-    KzControl *ctl = nullptr;
-    std::vector<void *> allocs;
+};
+
+/* A device's accel: the node and triangle arrays (KzNode8[n_nodes], KzF4[3 * n_tris]) and the max |coordinate| they were built for */
+struct Accel {
+    DevMem nodes, tris;
+    uint32_t n_nodes = 0, n_tris = 0;
+    float max_abs = 0.f;
 };
 
 struct Device {
     int id = -1;
     int sm_count = 0;
-    cudaStream_t stream = nullptr, copy_in = nullptr, copy_out = nullptr;
-    std::vector<void *> scene_allocs, accel_allocs;
-    KzScene sc;                      /* device pointers */
+    Stream stream, copy_in, copy_out;
+    std::vector<DevMem> tables;      /* scene tables and the vertex / index / texel records that sc points into */
+    Accel accel;
+    KzScene sc{};                    /* device pointers */
     bool has_accel = false;
     /* wavefront pools: the chunks of a render alternate between two lanes (own stream, path state, queues and control block), so
      * the ramp-up and the tail of one chunk's persistent kernels are filled by the other chunk's work */
     Lane lane[KZ_MAX_LANES];
     KzControl *ctl = nullptr;        /* = lane[0].ctl: counters of the batch entry points */
-    uint32_t *cursor = nullptr;      /* batch-trace fetch cursor */
+    DevMem cursor;                   /* batch-trace fetch cursor */
+    DevMem frame_mem;                /* the context's own frame; frame may point at a caller's instead (kzgpu_render_device) */
     KzF4 *frame = nullptr;
     size_t frame_texels = 0;
     /* primary-hit hints (KzExtendJob<true>::seed): (geomID, primID) per film pixel, allocated by the first render that uses them and
      * invalidated (all 0xFF) whenever the accel or the film may have changed -- a hint is only worth something for the same triangles */
-    uint2 *hint = nullptr;
-    size_t hint_px = 0;
+    DevMem hint;
     bool hint_stale = true;
-    cudaEvent_t splat_done = nullptr, merge_done = nullptr;   /* multi-device frame merge (k_frame_reduce) */
+    Event splat_done, merge_done;    /* multi-device frame merge (k_frame_reduce) */
     /* kzgpu_accel_refit: node boxes of the level below (kept between refits), its two result words (max |coordinate| as an ordered
      * uint, a failed level check) and whether this accel's level layout was checked on this device */
-    KzBox *refit_boxes = nullptr;
-    size_t refit_cap = 0;
-    uint32_t *refit_flags = nullptr;
+    DevMem refit_boxes, refit_flags;
     bool levels_checked = false;
     /* scratch for host-pointer entry points */
-    void *scratch[3] = {nullptr, nullptr, nullptr};
-    size_t scratch_bytes[3] = {0, 0, 0};
+    DevMem scratch[3];
     /* launch geometry */
     int grid_extend0 = 0, grid_extend = 0, grid_shadow = 0, grid_trace = 0, grid_occ = 0, grid_shade[KZ_NUM_CLASSES] = {0, 0, 0, 0, 0};
     /* timing */
@@ -74,6 +81,14 @@ struct Device {
     std::vector<cudaEvent_t> free_events;
     double ms[CAT_COUNT] = {0, 0, 0, 0};
     uint64_t launches = 0;
+
+    /* releases everything with this device current, after its work finished (the members go after this body) */
+    ~Device() {
+        if (id < 0) return;
+        cudaSetDevice(id);
+        cudaDeviceSynchronize();
+        for (cudaEvent_t e : free_events) cudaEventDestroy(e);
+    }
 };
 
 }  // namespace
@@ -119,47 +134,27 @@ int fail(kzgpu_ctx *ctx, int code, const std::string &msg) {
                         std::string(#call) + ": " + cudaGetErrorString(e__) + " (" + __FILE__ + ":" + std::to_string(__LINE__) + ")"); \
     } while (0)
 
-template <typename T> int dev_alloc(kzgpu_ctx *ctx, std::vector<void *> &owner, size_t count, T **out) {
-    void *p = nullptr;
-    KZ_CUDA(ctx, cudaMalloc(&p, std::max<size_t>(16, count * sizeof(T))));
-    owner.push_back(p);
-    *out = reinterpret_cast<T *>(p);
+template <typename T> int dev_alloc(kzgpu_ctx *ctx, DevMem &m, size_t count, T **out) {
+    KZ_CUDA(ctx, m.alloc(count * sizeof(T)));
+    *out = m.as<T>();
     return KZ_OK;
 }
-template <typename T> int dev_upload(kzgpu_ctx *ctx, Device &d, std::vector<void *> &owner, const T *src, size_t count, const T **out) {
+template <typename T> int dev_upload(kzgpu_ctx *ctx, Device &d, DevMem &m, const T *src, size_t count, const T **out) {
     T *p = nullptr;
-    int rc = dev_alloc(ctx, owner, count, &p);
+    int rc = dev_alloc(ctx, m, count, &p);
     if (rc) return rc;
     if (count) KZ_CUDA(ctx, cudaMemcpyAsync(p, src, count * sizeof(T), cudaMemcpyHostToDevice, d.stream));
     *out = p;
     return KZ_OK;
 }
-void free_all(std::vector<void *> &v) {
-    for (void *p : v) cudaFree(p);
-    v.clear();
-}
 /* Short-lived buffers (ingest staging, the builders' triangle list) come from the device's stream-ordered memory pool: a plain
  * cudaMalloc maps every new block into all peers once peer access is enabled (multi-device contexts, NCCL in the same process). */
-template <typename T> int temp_alloc(kzgpu_ctx *ctx, std::vector<void *> &owner, size_t count, cudaStream_t s, T **out) {
-    void *p = nullptr;
-    KZ_CUDA(ctx, cudaMallocAsync(&p, std::max<size_t>(16, count * sizeof(T)), s));
-    owner.push_back(p);
-    *out = reinterpret_cast<T *>(p);
+template <typename T> int temp_alloc(kzgpu_ctx *ctx, AsyncMem &m, size_t count, cudaStream_t s, T **out) {
+    KZ_CUDA(ctx, m.alloc(count * sizeof(T), s));
+    *out = m.as<T>();
     return KZ_OK;
 }
-void temp_free_all(std::vector<void *> &v, cudaStream_t s) {
-    for (void *p : v) cudaFreeAsync(p, s);
-    v.clear();
-}
-
-int ensure_scratch(kzgpu_ctx *ctx, Device &d, int k, size_t bytes) {
-    if (d.scratch_bytes[k] >= bytes) return KZ_OK;
-    if (d.scratch[k]) { cudaFree(d.scratch[k]); d.scratch[k] = nullptr; d.scratch_bytes[k] = 0; }
-    size_t want = std::max<size_t>(bytes, 1u << 20);
-    KZ_CUDA(ctx, cudaMalloc(&d.scratch[k], want));
-    d.scratch_bytes[k] = want;
-    return KZ_OK;
-}
+const size_t SCRATCH_MIN = 1u << 20;     /* the scratch buffers of the host-pointer entry points never shrink, nor start below this */
 
 cudaEvent_t get_event(Device &d) {
     if (!d.free_events.empty()) { cudaEvent_t e = d.free_events.back(); d.free_events.pop_back(); return e; }
@@ -221,24 +216,25 @@ int grid_for(size_t n, int threads, int sm_count) {
  * first device and copied to the others over NVLink (replicate_geometry). */
 int upload_tables(kzgpu_ctx *ctx, Device &d) {
     const KzHostScene &h = *ctx->hs;
-    free_all(d.scene_allocs);
-    d.sc = h.sc;
-    d.sc.nodes = nullptr; d.sc.tris = nullptr; d.sc.n_nodes = 0; d.sc.n_tris = 0;
+    d.tables.clear();
+    d.frame_mem.reset();
+    d.sc = h.sc;     /* flatten() without geometry leaves the accel fields of h.sc empty, as drop_all() left those of d.sc */
+    auto next = [&d]() -> DevMem & { d.tables.emplace_back(); return d.tables.back(); };
     int rc;
-#define UP(field, vec) if ((rc = dev_upload(ctx, d, d.scene_allocs, (vec).data(), (vec).size(), &d.sc.field))) return rc
+#define UP(field, vec) if ((rc = dev_upload(ctx, d, next(), (vec).data(), (vec).size(), &d.sc.field))) return rc
     UP(meshes, h.meshes);
     UP(light_cdf, h.light_cdf); UP(light_meshes, h.light_meshes); UP(bsdfs, h.bsdfs); UP(textures, h.textures);
     UP(images, h.images); UP(lights, h.lights); UP(blue_noise, h.blue_noise); UP(pmj02bn, h.pmj);
     UP(pmj_pixel_samples, h.pmj_pixel_samples);
 #undef UP
     KzVertex *v = nullptr; KzU4 *ix = nullptr; KzF4 *tx = nullptr;
-    if ((rc = dev_alloc(ctx, d.scene_allocs, (size_t)h.total_vertices, &v))) return rc;
-    if ((rc = dev_alloc(ctx, d.scene_allocs, (size_t)h.total_triangles, &ix))) return rc;
-    if ((rc = dev_alloc(ctx, d.scene_allocs, h.total_texels, &tx))) return rc;
+    if ((rc = dev_alloc(ctx, next(), (size_t)h.total_vertices, &v))) return rc;
+    if ((rc = dev_alloc(ctx, next(), (size_t)h.total_triangles, &ix))) return rc;
+    if ((rc = dev_alloc(ctx, next(), h.total_texels, &tx))) return rc;
     d.sc.vertices = v; d.sc.indices = ix; d.sc.texels = tx;
     /* frame */
     const size_t texels = (size_t)(h.sc.camera.width + 2 * h.sc.border) * (size_t)(h.sc.camera.height + 2 * h.sc.border);
-    if ((rc = dev_alloc(ctx, d.scene_allocs, texels, &d.frame))) return rc;
+    if ((rc = dev_alloc(ctx, d.frame_mem, texels, &d.frame))) return rc;
     d.frame_texels = texels;
     KZ_CUDA(ctx, cudaMemsetAsync(d.frame, 0, texels * sizeof(KzF4), d.stream));
     return KZ_OK;
@@ -254,11 +250,11 @@ int ingest_geometry(kzgpu_ctx *ctx, Device &d, const kz_scene_desc *scene) {
         stage_bytes = std::max(stage_bytes, (size_t)m.n_vertices * 32 + (size_t)m.n_triangles * 12 + 64);
     }
     for (uint32_t i = 0; i < scene->n_images; ++i) stage_bytes = std::max(stage_bytes, (size_t)scene->images[i].width * scene->images[i].height * 12);
-    std::vector<void *> temp;
+    AsyncMem stage_mem, bad_mem;
     char *stage = nullptr; uint32_t *bad = nullptr;
     int rc;
-    if ((rc = temp_alloc(ctx, temp, stage_bytes, d.stream, &stage))) { temp_free_all(temp, d.stream); return rc; }
-    if ((rc = temp_alloc(ctx, temp, 4, d.stream, &bad))) { temp_free_all(temp, d.stream); return rc; }
+    if ((rc = temp_alloc(ctx, stage_mem, stage_bytes, d.stream, &stage))) return rc;
+    if ((rc = temp_alloc(ctx, bad_mem, 4, d.stream, &bad))) return rc;
     cudaError_t e = cudaMemsetAsync(bad, 0, 4, d.stream);
     auto fetch = [&](const void *src, size_t bytes, size_t &cursor) -> const void * {      /* device-visible view of a caller array */
         if (!src || e != cudaSuccess) return nullptr;
@@ -296,7 +292,6 @@ int ingest_geometry(kzgpu_ctx *ctx, Device &d, const kz_scene_desc *scene) {
     if (e == cudaSuccess) e = cudaMemcpyAsync(&h_bad, bad, 4, cudaMemcpyDeviceToHost, d.stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(d.stream);
     if (e == cudaSuccess) e = cudaGetLastError();
-    temp_free_all(temp, d.stream);
     if (e != cudaSuccess) return fail(ctx, KZ_ERR_CUDA, std::string("scene ingest: ") + cudaGetErrorString(e));
     if (h_bad) return fail(ctx, KZ_ERR_INVALID, "vertex index out of range");
     return KZ_OK;
@@ -314,10 +309,11 @@ int replicate_geometry(kzgpu_ctx *ctx, Device &dst, const Device &src) {
 
 int ensure_pool(kzgpu_ctx *ctx, Lane &L, uint32_t cap) {
     if (L.pool_cap >= cap) return KZ_OK;
-    free_all(L.allocs);
+    for (DevMem &m : L.pool) m.reset();     /* the old pool goes before the new one is allocated */
     L.pool_cap = 0;
+    DevMem *m = L.pool;
     int rc;
-#define AL(ptr) if ((rc = dev_alloc(ctx, L.allocs, (size_t)cap, &(ptr)))) return rc
+#define AL(ptr) if ((rc = dev_alloc(ctx, *m++, (size_t)cap, &(ptr)))) return rc
     AL(L.st.a); AL(L.st.b); AL(L.st.c);
     AL(L.q.ext[0]); AL(L.q.ext[1]); AL(L.q.shadow);
     for (int c = 0; c < KZ_NUM_CLASSES; ++c) AL(L.q.cls[c]);
@@ -326,31 +322,50 @@ int ensure_pool(kzgpu_ctx *ctx, Lane &L, uint32_t cap) {
     return KZ_OK;
 }
 
-int upload_accel(kzgpu_ctx *ctx, Device &d, const kzbvh::Built &b) {
-    free_all(d.accel_allocs);
-    int rc;
-    if ((rc = dev_upload(ctx, d, d.accel_allocs, b.nodes.data(), b.nodes.size(), &d.sc.nodes))) return rc;
-    if ((rc = dev_upload(ctx, d, d.accel_allocs, b.tris.data(), b.tris.size(), &d.sc.tris))) return rc;
-    d.sc.n_nodes = (uint32_t)b.nodes.size();
-    d.sc.n_tris = (uint32_t)(b.tris.size() / 3);
-    d.sc.scene_max_abs = b.max_abs;
-    KZ_CUDA(ctx, cudaStreamSynchronize(d.stream));
+/* install() and drop_all() are the only places where the accel of a device changes.  drop_all() releases the accel of every
+ * device and clears ctx->built, which only a completed build or refit sets again: from the moment an old accel is released until a
+ * new one is installed on every device, trace and render return KZ_ERR_STATE instead of reading released memory. */
+void install(Device &d, Accel &&a) {
+    d.accel = std::move(a);
+    d.sc.nodes = d.accel.nodes.as<const KzNode8>(); d.sc.tris = d.accel.tris.as<const KzF4>();
+    d.sc.n_nodes = d.accel.n_nodes; d.sc.n_tris = d.accel.n_tris; d.sc.scene_max_abs = d.accel.max_abs;
     d.has_accel = true;
+    d.hint_stale = true;
+    d.levels_checked = false;
+}
+void drop_all(kzgpu_ctx *ctx) {
+    ctx->built = false;
+    ctx->levels.clear();
+    for (Device &d : ctx->devs) {
+        cudaSetDevice(d.id);
+        d.accel = Accel();
+        d.sc.nodes = nullptr; d.sc.tris = nullptr; d.sc.n_nodes = 0; d.sc.n_tris = 0; d.sc.scene_max_abs = 0.f;
+        d.has_accel = false;
+    }
+}
+
+int upload_accel(kzgpu_ctx *ctx, Device &d, const kzbvh::Built &b) {
+    Accel a{{}, {}, (uint32_t)b.nodes.size(), (uint32_t)(b.tris.size() / 3), b.max_abs};
+    const KzNode8 *nodes; const KzF4 *tris;
+    int rc;
+    if ((rc = dev_upload(ctx, d, a.nodes, b.nodes.data(), b.nodes.size(), &nodes))) return rc;
+    if ((rc = dev_upload(ctx, d, a.tris, b.tris.data(), b.tris.size(), &tris))) return rc;
+    KZ_CUDA(ctx, cudaStreamSynchronize(d.stream));
+    install(d, std::move(a));
     return KZ_OK;
 }
 
-/* Copies the accel that device `src` built into fresh arrays of `dst` (peer copies over NVLink). */
+/* Copies the accel of device `src` into fresh arrays of `dst` (current; peer copies over NVLink). */
 int replicate_accel(kzgpu_ctx *ctx, Device &dst, const Device &src) {
-    free_all(dst.accel_allocs);
+    Accel a{{}, {}, src.accel.n_nodes, src.accel.n_tris, src.accel.max_abs};
     KzNode8 *nodes = nullptr; KzF4 *tris = nullptr;
     int rc;
-    if ((rc = dev_alloc(ctx, dst.accel_allocs, (size_t)src.sc.n_nodes, &nodes))) return rc;
-    if ((rc = dev_alloc(ctx, dst.accel_allocs, (size_t)src.sc.n_tris * 3, &tris))) return rc;
-    KZ_CUDA(ctx, cudaMemcpyPeerAsync(nodes, dst.id, src.sc.nodes, src.id, (size_t)src.sc.n_nodes * sizeof(KzNode8), dst.stream));
-    KZ_CUDA(ctx, cudaMemcpyPeerAsync(tris, dst.id, src.sc.tris, src.id, (size_t)src.sc.n_tris * 3 * sizeof(KzF4), dst.stream));
+    if ((rc = dev_alloc(ctx, a.nodes, (size_t)a.n_nodes, &nodes))) return rc;
+    if ((rc = dev_alloc(ctx, a.tris, (size_t)a.n_tris * 3, &tris))) return rc;
+    KZ_CUDA(ctx, cudaMemcpyPeerAsync(nodes, dst.id, src.sc.nodes, src.id, (size_t)a.n_nodes * sizeof(KzNode8), dst.stream));
+    KZ_CUDA(ctx, cudaMemcpyPeerAsync(tris, dst.id, src.sc.tris, src.id, (size_t)a.n_tris * 3 * sizeof(KzF4), dst.stream));
     KZ_CUDA(ctx, cudaStreamSynchronize(dst.stream));
-    dst.sc.nodes = nodes; dst.sc.tris = tris; dst.sc.n_nodes = src.sc.n_nodes; dst.sc.n_tris = src.sc.n_tris; dst.sc.scene_max_abs = src.sc.scene_max_abs;
-    dst.has_accel = true;
+    install(dst, std::move(a));
     return KZ_OK;
 }
 
@@ -370,7 +385,7 @@ int enqueue_chunk(const kzgpu_ctx *ctx, kzgpu_ctx *ectx, Device &d, Lane &L, con
     /* the pass after the last vertex only resolves "miss -> background" (integrator.cpp:315-318) */
     const int last_pass = sc.background >= 0 ? max_depth : max_depth - 1;
     const bool alt = sc.integrator.type != KZ_INTEGRATOR_PATH_MIS;
-    uint2 *const hint = hints_on(ctx) ? d.hint : nullptr;
+    uint2 *const hint = hints_on(ctx) ? d.hint.as<uint2>() : nullptr;
     if (d.pending.size() > 8192) fold_events(d);       /* very long renders: bound the number of live timing events */
     {
         Timed t(d, s, CAT_SHADE);
@@ -473,14 +488,13 @@ int enqueue_render(const kzgpu_ctx *ctx, kzgpu_ctx *ectx, Device &d, const kz_re
     for (int l = 0; l < lanes; ++l) if ((rc = ensure_pool(ectx, d.lane[l], cap))) return rc;
     if (hints_on(ctx)) {
         /* every pixel k_raygen can produce lies on the film (check_req), whatever the rectangle or the device's share of samples */
-        const size_t npx = (size_t)sc.camera.width * (size_t)sc.camera.height;
-        if (d.hint_px < npx) {
-            if (d.hint) { cudaFree(d.hint); d.hint = nullptr; d.hint_px = 0; }
-            KZ_CUDA(ectx, cudaMalloc(&d.hint, npx * sizeof(uint2)));
-            d.hint_px = npx; d.hint_stale = true;
+        const size_t bytes = (size_t)sc.camera.width * (size_t)sc.camera.height * sizeof(uint2);
+        if (d.hint.bytes < bytes) {
+            KZ_CUDA(ectx, d.hint.alloc(bytes));
+            d.hint_stale = true;
         }
         if (d.hint_stale) {     /* before anything of this request, on s: the other lanes start after it (below) */
-            KZ_CUDA(ectx, cudaMemsetAsync(d.hint, 0xFF, d.hint_px * sizeof(uint2), s));
+            KZ_CUDA(ectx, cudaMemsetAsync(d.hint.p, 0xFF, d.hint.bytes, s));
             d.hint_stale = false;
         }
     }
@@ -536,27 +550,30 @@ int kzgpu_create(const int *device_ids, int n_devices, kzgpu_ctx **out) {
     if (const char *p = getenv("KZGPU_LANES")) { int l = atoi(p); if (l >= 1 && l <= KZ_MAX_LANES) ctx->lanes = l; }
     if (const char *p = getenv("KZGPU_SPP_GROUP")) { int g = atoi(p); if (g >= 1) ctx->spp_group = g; }
     if (const char *p = getenv("KZGPU_PRIMARY_HINT")) { int h = atoi(p); if (h >= 0 && h <= 2) ctx->primary_hint = h; }
-    for (int id : ids) {
+    /* the devices are set up in place and never move (code compares &d with &ctx->devs[0]); a failure below releases all of them */
+    ctx->devs = std::vector<Device>(ids.size());
+    for (size_t i = 0; i < ids.size(); ++i) {
+        const int id = ids[i];
         if (id < 0 || id >= count) return fail(nullptr, KZ_ERR_NO_DEVICE, "device id " + std::to_string(id) + " out of range");
         cudaDeviceProp prop;
         KZ_CUDA(nullptr, cudaGetDeviceProperties(&prop, id));
         if (prop.major != 10) return fail(nullptr, KZ_ERR_NO_DEVICE, std::string("device ") + prop.name + " is sm_" + std::to_string(prop.major) + std::to_string(prop.minor) +
                                                                        "; this library is built for sm_100a only");
-        Device d;
-        d.id = id; d.sm_count = prop.multiProcessorCount;
-        memset(&d.sc, 0, sizeof(d.sc));
         KZ_CUDA(nullptr, cudaSetDevice(id));
-        KZ_CUDA(nullptr, cudaStreamCreateWithFlags(&d.stream, cudaStreamNonBlocking));
+        Device &d = ctx->devs[i];
+        d.id = id; d.sm_count = prop.multiProcessorCount;
+        KZ_CUDA(nullptr, cudaStreamCreateWithFlags(&d.stream.h, cudaStreamNonBlocking));
         for (Lane &L : d.lane) {
-            KZ_CUDA(nullptr, cudaMalloc(&L.ctl, sizeof(KzControl)));
+            KZ_CUDA(nullptr, L.ctl_mem.alloc(sizeof(KzControl)));
+            L.ctl = L.ctl_mem.as<KzControl>();
             KZ_CUDA(nullptr, cudaMemset(L.ctl, 0, sizeof(KzControl)));
-            KZ_CUDA(nullptr, cudaEventCreateWithFlags(&L.done, cudaEventDisableTiming));
+            KZ_CUDA(nullptr, cudaEventCreateWithFlags(&L.done.h, cudaEventDisableTiming));
         }
-        for (int l = 1; l < KZ_MAX_LANES; ++l) KZ_CUDA(nullptr, cudaStreamCreateWithFlags(&d.lane[l].stream, cudaStreamNonBlocking));
+        for (int l = 1; l < KZ_MAX_LANES; ++l) KZ_CUDA(nullptr, cudaStreamCreateWithFlags(&d.lane[l].stream.h, cudaStreamNonBlocking));
         d.ctl = d.lane[0].ctl;
-        KZ_CUDA(nullptr, cudaEventCreateWithFlags(&d.splat_done, cudaEventDisableTiming));
-        KZ_CUDA(nullptr, cudaEventCreateWithFlags(&d.merge_done, cudaEventDisableTiming));
-        KZ_CUDA(nullptr, cudaMalloc(&d.cursor, 64));
+        KZ_CUDA(nullptr, cudaEventCreateWithFlags(&d.splat_done.h, cudaEventDisableTiming));
+        KZ_CUDA(nullptr, cudaEventCreateWithFlags(&d.merge_done.h, cudaEventDisableTiming));
+        KZ_CUDA(nullptr, d.cursor.alloc(64));
         d.grid_extend0 = persistent_grid(d, k_extend<true>, KZ_TRACE_THREADS);
         d.grid_extend = persistent_grid(d, k_extend<false>, KZ_TRACE_THREADS);
         d.grid_shadow = persistent_grid(d, k_shadow, KZ_TRACE_THREADS);
@@ -568,7 +585,6 @@ int kzgpu_create(const int *device_ids, int n_devices, kzgpu_ctx **out) {
         d.grid_shade[2] = persistent_grid(d, k_shade<KZ_CLASS_KISS>, KZ_SHADE_THREADS);
         d.grid_shade[3] = persistent_grid(d, k_shade<KZ_CLASS_NORMALMAP>, KZ_SHADE_THREADS);
         d.grid_shade[4] = persistent_grid(d, k_shade<KZ_CLASS_GENERIC>, KZ_SHADE_THREADS);
-        ctx->devs.push_back(d);
     }
     /* a multi-device context replicates the scene and merges the frames through peer memory (NVLink / NVSwitch): every pair of its
      * devices must be able to map each other's HBM */
@@ -592,23 +608,9 @@ void kzgpu_destroy(kzgpu_ctx *ctx) {
     if (!ctx) return;
     for (Device &d : ctx->devs) {
         cudaSetDevice(d.id);
-        cudaDeviceSynchronize();
         fold_events(d);
-        for (cudaEvent_t e : d.free_events) cudaEventDestroy(e);
-        free_all(d.scene_allocs); free_all(d.accel_allocs);
-        if (d.hint) cudaFree(d.hint);
-        if (d.refit_boxes) cudaFree(d.refit_boxes);
-        if (d.refit_flags) cudaFree(d.refit_flags);
-        for (Lane &L : d.lane) { free_all(L.allocs); cudaFree(L.ctl); if (L.done) cudaEventDestroy(L.done); if (L.stream) cudaStreamDestroy(L.stream); }
-        for (int k = 0; k < 3; ++k) if (d.scratch[k]) cudaFree(d.scratch[k]);
-        cudaFree(d.cursor);
-        if (d.splat_done) cudaEventDestroy(d.splat_done);
-        if (d.merge_done) cudaEventDestroy(d.merge_done);
-        cudaStreamDestroy(d.stream);
-        if (d.copy_in) cudaStreamDestroy(d.copy_in);
-        if (d.copy_out) cudaStreamDestroy(d.copy_out);
     }
-    delete ctx;
+    delete ctx;     /* ~Device synchronises each device and releases its resources */
 }
 
 int kzgpu_scene_upload(kzgpu_ctx *ctx, const kz_scene_desc *scene) {
@@ -640,7 +642,8 @@ int kzgpu_scene_upload(kzgpu_ctx *ctx, const kz_scene_desc *scene) {
         return fail(ctx, unsupported ? KZ_ERR_UNSUPPORTED : KZ_ERR_INVALID, hs->error);
     }
     ctx->hs = std::move(hs);
-    ctx->uploaded = false; ctx->built = false;
+    ctx->uploaded = false;
+    drop_all(ctx);
     for (int c = 1; c < KZ_NUM_CLASSES; ++c) ctx->class_present[c] = false;
     for (const KzMeshRec &m : ctx->hs->meshes) {
         if (m.flags & KZ_MESH_IS_LIGHT) continue;
@@ -649,10 +652,6 @@ int kzgpu_scene_upload(kzgpu_ctx *ctx, const kz_scene_desc *scene) {
     }
     for (Device &d : ctx->devs) {
         KZ_CUDA(ctx, cudaSetDevice(d.id));
-        d.has_accel = false;
-        d.hint_stale = true;
-        d.levels_checked = false;
-        free_all(d.accel_allocs);
         int rc = upload_tables(ctx, d);
         if (rc) return rc;
         /* the first device ingests the caller's arrays, the others get its records over NVLink */
@@ -675,9 +674,10 @@ int kzgpu_accel_build(kzgpu_ctx *ctx, int builder) {
     KZ_CUDA(ctx, cudaSetDevice(d0.id));
     /* the builders' input: the triangle list in scene order, gathered on the device from the ingested records */
     const uint32_t n_tris = (uint32_t)ctx->hs->total_triangles;
-    std::vector<void *> temp;
+    std::vector<uint32_t> levels;     /* -> ctx->levels once the new accel is installed everywhere */
+    AsyncMem tris_mem;
     kzbvh::Tri *d_tris = nullptr;
-    if ((rc = temp_alloc(ctx, temp, (size_t)n_tris, d0.stream, &d_tris))) { temp_free_all(temp, d0.stream); return rc; }
+    if ((rc = temp_alloc(ctx, tris_mem, (size_t)n_tris, d0.stream, &d_tris))) return rc;
     if (n_tris) {
         k_gather_tris<<<grid_for(n_tris, 256, d0.sm_count), 256, 0, d0.stream>>>(d0.sc.meshes, d0.sc.n_meshes, d0.sc.vertices, d0.sc.indices, n_tris, d_tris);
         ++d0.launches;
@@ -687,12 +687,14 @@ int kzgpu_accel_build(kzgpu_ctx *ctx, int builder) {
         cudaError_t e = cudaSuccess;
         if (n_tris) e = cudaMemcpyAsync(tris.data(), d_tris, (size_t)n_tris * sizeof(kzbvh::Tri), cudaMemcpyDeviceToHost, d0.stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(d0.stream);
-        temp_free_all(temp, d0.stream);
+        tris_mem.reset();
         KZ_CUDA(ctx, e);
         kzbvh::Built built;
         kzbvh::buildHostSah(tris, 0, built);
+        /* a failure up to here keeps the old accel in use */
         if (built.depth > KZ_MAX_ACCEL_DEPTH) return fail(ctx, KZ_ERR_UNSUPPORTED, "accel deeper than the traversal stack allows");
-        if (!kz_refit_levels(built.nodes.data(), (uint32_t)built.nodes.size(), ctx->levels)) ctx->levels.clear();
+        if (!kz_refit_levels(built.nodes.data(), (uint32_t)built.nodes.size(), levels)) levels.clear();
+        drop_all(ctx);      /* the old accel goes before the new one is allocated: at 10^8 triangles one is about 13 GB */
         for (Device &d : ctx->devs) {
             KZ_CUDA(ctx, cudaSetDevice(d.id));
             if ((rc = upload_accel(ctx, d, built))) return rc;
@@ -700,19 +702,19 @@ int kzgpu_accel_build(kzgpu_ctx *ctx, int builder) {
         ctx->bvh_nodes = built.nodes.size();
         ctx->bvh_bytes = built.nodes.size() * sizeof(KzNode8) + built.tris.size() * sizeof(KzF4);
     } else {
-        free_all(d0.accel_allocs);
+        drop_all(ctx);
+        KZ_CUDA(ctx, cudaSetDevice(d0.id));
         kzlbvh::Result r;
         std::string err;
-        rc = kzlbvh::build(d_tris, n_tris, d0.stream, d0.accel_allocs, r, err);
-        temp_free_all(temp, d0.stream);
+        rc = kzlbvh::build(d_tris, n_tris, d0.stream, r, err);
+        tris_mem.reset();
         /* hand the pool's memory back: the path pools and the caller's own allocations need it, the next build allocates afresh */
         { cudaMemPool_t pool; if (cudaDeviceGetDefaultMemPool(&pool, d0.id) == cudaSuccess) { cudaStreamSynchronize(d0.stream); cudaMemPoolTrimTo(pool, 0); } }
         if (rc) return fail(ctx, rc, err);
         if (r.depth > KZ_MAX_ACCEL_DEPTH) return fail(ctx, KZ_ERR_UNSUPPORTED, "accel deeper than the traversal stack allows");
-        d0.sc.nodes = r.nodes; d0.sc.tris = r.tris; d0.sc.n_nodes = r.n_nodes; d0.sc.n_tris = r.n_tris; d0.sc.scene_max_abs = r.max_abs;
-        ctx->levels = r.n_nodes ? r.level_first : std::vector<uint32_t>(1, 0u);
-        if (ctx->levels.back() != r.n_nodes) ctx->levels.clear();
-        d0.has_accel = true;
+        install(d0, Accel{std::move(r.nodes), std::move(r.tris), r.n_nodes, r.n_tris, r.max_abs});
+        levels = r.n_nodes ? r.level_first : std::vector<uint32_t>(1, 0u);
+        if (levels.back() != r.n_nodes) levels.clear();
         d0.launches += r.launches;
         ctx->bvh_nodes = r.n_nodes;
         ctx->bvh_bytes = (uint64_t)r.n_nodes * sizeof(KzNode8) + (uint64_t)r.n_tris * 3 * sizeof(KzF4);
@@ -723,8 +725,8 @@ int kzgpu_accel_build(kzgpu_ctx *ctx, int builder) {
         }
         KZ_CUDA(ctx, cudaSetDevice(d0.id));
     }
-    for (Device &d : ctx->devs) { d.hint_stale = true; d.levels_checked = false; }
     ctx->ms_build = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    ctx->levels = std::move(levels);
     ctx->built = true;
     return KZ_OK;
 }
@@ -766,14 +768,14 @@ int kzgpu_mesh_update(kzgpu_ctx *ctx, int mesh, const float *positions, const fl
     ctx->built = false;
     /* vertex records of device 0: host arrays are staged with one copy each, device arrays read in place */
     {
-        std::vector<void *> temp;
+        AsyncMem stage_mem[2];
         const float *src[2] = {positions, normals};
         cudaError_t e = cudaSuccess;
         for (int k = 0; k < 2 && e == cudaSuccess; ++k) {
             if (!src[k] || is_device_ptr(src[k])) continue;
             float *stage = nullptr;
-            int rc = temp_alloc(ctx, temp, (size_t)nv * 3, d0.stream, &stage);
-            if (rc) { temp_free_all(temp, d0.stream); return rc; }
+            int rc = temp_alloc(ctx, stage_mem[k], (size_t)nv * 3, d0.stream, &stage);
+            if (rc) return rc;
             e = cudaMemcpyAsync(stage, src[k], (size_t)nv * 12, cudaMemcpyHostToDevice, d0.stream);
             src[k] = stage;
         }
@@ -783,7 +785,6 @@ int kzgpu_mesh_update(kzgpu_ctx *ctx, int mesh, const float *positions, const fl
             e = cudaGetLastError();
         }
         if (e == cudaSuccess) e = cudaStreamSynchronize(d0.stream);
-        temp_free_all(temp, d0.stream);
         if (e != cudaSuccess) return fail(ctx, KZ_ERR_CUDA, std::string("mesh update: ") + cudaGetErrorString(e));
     }
     if (r.flags & KZ_MESH_IS_LIGHT) {
@@ -818,13 +819,13 @@ int kzgpu_accel_refit(kzgpu_ctx *ctx) {
     /* once per built accel and device: every internal child one level down, every triangle in the record array */
     for (Device &d : ctx->devs) {
         KZ_CUDA(ctx, cudaSetDevice(d.id));
-        if (!d.refit_flags) KZ_CUDA(ctx, cudaMalloc(&d.refit_flags, 2 * sizeof(uint32_t)));
-        KZ_CUDA(ctx, cudaMemsetAsync(d.refit_flags, 0, 2 * sizeof(uint32_t), d.stream));
+        KZ_CUDA(ctx, d.refit_flags.ensure(2 * sizeof(uint32_t)));
+        KZ_CUDA(ctx, cudaMemsetAsync(d.refit_flags.p, 0, 2 * sizeof(uint32_t), d.stream));
         if (d.levels_checked || d.sc.n_nodes == 0) continue;
         for (int l = 0; l < nl; ++l) {
             const uint32_t next_hi = l + 1 < nl ? L[(size_t)l + 2] : L[(size_t)l + 1];
             k_refit_check<<<grid_for(L[(size_t)l + 1] - L[(size_t)l], 256, d.sm_count), 256, 0, d.stream>>>(d.sc.nodes, L[(size_t)l], L[(size_t)l + 1], L[(size_t)l + 1], next_hi,
-                                                                                                          d.sc.n_tris, d.refit_flags + 1);
+                                                                                                          d.sc.n_tris, d.refit_flags.as<uint32_t>() + 1);
             ++d.launches;
         }
         KZ_CUDA(ctx, cudaGetLastError());
@@ -833,7 +834,7 @@ int kzgpu_accel_refit(kzgpu_ctx *ctx) {
         if (d.levels_checked || d.sc.n_nodes == 0) continue;
         uint32_t bad = 0;
         KZ_CUDA(ctx, cudaSetDevice(d.id));
-        KZ_CUDA(ctx, cudaMemcpyAsync(&bad, d.refit_flags + 1, 4, cudaMemcpyDeviceToHost, d.stream));
+        KZ_CUDA(ctx, cudaMemcpyAsync(&bad, d.refit_flags.as<uint32_t>() + 1, 4, cudaMemcpyDeviceToHost, d.stream));
         KZ_CUDA(ctx, cudaStreamSynchronize(d.stream));
         if (bad || L.back() != d.sc.n_nodes) return fail(ctx, KZ_ERR_STATE, "the accel is not laid out level by level: call kzgpu_accel_build");
         d.levels_checked = true;
@@ -842,16 +843,12 @@ int kzgpu_accel_refit(kzgpu_ctx *ctx) {
     for (Device &d : ctx->devs) {
         if (d.sc.n_nodes == 0) continue;
         KZ_CUDA(ctx, cudaSetDevice(d.id));
-        if (d.refit_cap < d.sc.n_nodes) {
-            if (d.refit_boxes) { cudaFree(d.refit_boxes); d.refit_boxes = nullptr; d.refit_cap = 0; }
-            KZ_CUDA(ctx, cudaMalloc(&d.refit_boxes, (size_t)d.sc.n_nodes * sizeof(KzBox)));
-            d.refit_cap = d.sc.n_nodes;
-        }
-        KzF4 *tris = const_cast<KzF4 *>(d.sc.tris);
-        KzNode8 *nodes = const_cast<KzNode8 *>(d.sc.nodes);
-        k_refit_tris<<<grid_for(d.sc.n_tris, 256, d.sm_count), 256, 0, d.stream>>>(d.sc.meshes, d.sc.vertices, d.sc.indices, tris, d.sc.n_tris, d.refit_flags);
+        KZ_CUDA(ctx, d.refit_boxes.ensure((size_t)d.sc.n_nodes * sizeof(KzBox)));
+        KzF4 *tris = d.accel.tris.as<KzF4>();
+        KzNode8 *nodes = d.accel.nodes.as<KzNode8>();
+        k_refit_tris<<<grid_for(d.sc.n_tris, 256, d.sm_count), 256, 0, d.stream>>>(d.sc.meshes, d.sc.vertices, d.sc.indices, tris, d.sc.n_tris, d.refit_flags.as<uint32_t>());
         for (int l = nl - 1; l >= 0; --l)
-            k_refit_level<<<grid_for(L[(size_t)l + 1] - L[(size_t)l], 128, d.sm_count), 128, 0, d.stream>>>(nodes, tris, d.refit_boxes, L[(size_t)l], L[(size_t)l + 1]);
+            k_refit_level<<<grid_for(L[(size_t)l + 1] - L[(size_t)l], 128, d.sm_count), 128, 0, d.stream>>>(nodes, tris, d.refit_boxes.as<KzBox>(), L[(size_t)l], L[(size_t)l + 1]);
         d.launches += 1 + (uint64_t)nl;
         KZ_CUDA(ctx, cudaGetLastError());
     }
@@ -859,9 +856,9 @@ int kzgpu_accel_refit(kzgpu_ctx *ctx) {
         if (d.sc.n_nodes == 0) continue;
         uint32_t mabs = 0;
         KZ_CUDA(ctx, cudaSetDevice(d.id));
-        KZ_CUDA(ctx, cudaMemcpyAsync(&mabs, d.refit_flags, 4, cudaMemcpyDeviceToHost, d.stream));
+        KZ_CUDA(ctx, cudaMemcpyAsync(&mabs, d.refit_flags.p, 4, cudaMemcpyDeviceToHost, d.stream));
         KZ_CUDA(ctx, cudaStreamSynchronize(d.stream));
-        d.sc.scene_max_abs = kzlbvh::ord2f(mabs);
+        d.sc.scene_max_abs = d.accel.max_abs = kzlbvh::ord2f(mabs);
     }
     KZ_CUDA(ctx, cudaSetDevice(ctx->devs[0].id));
     ctx->built = true;
@@ -905,10 +902,10 @@ int kzgpu_trace_device(kzgpu_ctx *ctx, int device, const void *d_rays, size_t n,
     if (!d_rays || !d_hits) return fail(ctx, KZ_ERR_INVALID, "null ray/hit buffer");
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     if (d->pending.size() > 8192) fold_events(*d);      /* callers that never poll kzgpu_stats: bound the live timing events */
-    KZ_CUDA(ctx, cudaMemsetAsync(d->cursor, 0, 4, s));
+    KZ_CUDA(ctx, cudaMemsetAsync(d->cursor.p, 0, 4, s));
     {
         Timed t(*d, s, CAT_TRACE);
-        k_trace<<<d->grid_trace, KZ_TRACE_THREADS, 0, s>>>(d->sc, reinterpret_cast<const KzF4 *>(d_rays), (uint32_t)n, reinterpret_cast<float *>(d_hits), d->cursor, d->ctl);
+        k_trace<<<d->grid_trace, KZ_TRACE_THREADS, 0, s>>>(d->sc, reinterpret_cast<const KzF4 *>(d_rays), (uint32_t)n, reinterpret_cast<float *>(d_hits), d->cursor.as<uint32_t>(), d->ctl);
         ++d->launches;
     }
     KZ_CUDA(ctx, cudaGetLastError());
@@ -923,12 +920,12 @@ int kzgpu_trace(kzgpu_ctx *ctx, int device, const kz_ray *rays, size_t n, int sh
     if (n == 0) return KZ_OK;
     if (!rays || !hits) return fail(ctx, KZ_ERR_INVALID, "null ray/hit buffer");
     if (n > 0x7FFFFFFFull) return fail(ctx, KZ_ERR_INVALID, "batch larger than 2^31-1 rays");
-    if ((rc = ensure_scratch(ctx, *d, 0, n * sizeof(kz_ray)))) return rc;
-    if ((rc = ensure_scratch(ctx, *d, 1, n * sizeof(kz_hit)))) return rc;
+    KZ_CUDA(ctx, d->scratch[0].ensure(n * sizeof(kz_ray), SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[1].ensure(n * sizeof(kz_hit), SCRATCH_MIN));
     /* Three-stage pipeline over ray chunks: H2D of chunk c+1, traversal of chunk c and D2H of chunk c-1 run
      * concurrently (PCIe is full duplex; with pinned host buffers the call costs max(copy, trace), not the sum). */
-    if (!d->copy_in) KZ_CUDA(ctx, cudaStreamCreateWithFlags(&d->copy_in, cudaStreamNonBlocking));
-    if (!d->copy_out) KZ_CUDA(ctx, cudaStreamCreateWithFlags(&d->copy_out, cudaStreamNonBlocking));
+    if (!d->copy_in) KZ_CUDA(ctx, cudaStreamCreateWithFlags(&d->copy_in.h, cudaStreamNonBlocking));
+    if (!d->copy_out) KZ_CUDA(ctx, cudaStreamCreateWithFlags(&d->copy_out.h, cudaStreamNonBlocking));
     static const size_t n_chunks = [] { const char *e = getenv("KZGPU_TRACE_CHUNKS"); const int k = e ? atoi(e) : 16; return (size_t)(k < 1 ? 1 : (k > 256 ? 256 : k)); }();
     const size_t chunk = std::min<size_t>(n, std::max<size_t>(1u << 20, (n + n_chunks - 1) / n_chunks));
     /* The call ends with the traversal and the D2H copy of the LAST chunk, which nothing overlaps (and starts with the H2D copy of the
@@ -951,7 +948,7 @@ int kzgpu_trace(kzgpu_ctx *ctx, int device, const kz_ray *rays, size_t n, int sh
         }
     }
     std::vector<cudaEvent_t> evs;
-    char *d_rays = reinterpret_cast<char *>(d->scratch[0]), *d_hits = reinterpret_cast<char *>(d->scratch[1]);
+    char *d_rays = reinterpret_cast<char *>(d->scratch[0].p), *d_hits = reinterpret_cast<char *>(d->scratch[1].p);
     size_t first = 0;
     for (size_t ci = 0; ci < sizes.size() && rc == KZ_OK; first += sizes[ci], ++ci) {
         const size_t cnt = sizes[ci];
@@ -980,16 +977,16 @@ int kzgpu_occluded(kzgpu_ctx *ctx, int device, const kz_ray *rays, size_t n, flo
     if (n == 0) return KZ_OK;
     if (n > 0x7FFFFFFFull) return fail(ctx, KZ_ERR_INVALID, "batch larger than 2^31-1 rays");
     if (!rays || !occluded) return fail(ctx, KZ_ERR_INVALID, "null buffer");
-    if ((rc = ensure_scratch(ctx, *d, 0, n * sizeof(kz_ray)))) return rc;
-    if ((rc = ensure_scratch(ctx, *d, 1, 2 * n))) return rc;
-    uint8_t *d_occ = reinterpret_cast<uint8_t *>(d->scratch[1]);
-    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0], rays, n * sizeof(kz_ray), cudaMemcpyHostToDevice, d->stream));
+    KZ_CUDA(ctx, d->scratch[0].ensure(n * sizeof(kz_ray), SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[1].ensure(2 * n, SCRATCH_MIN));
+    uint8_t *d_occ = reinterpret_cast<uint8_t *>(d->scratch[1].p);
+    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0].p, rays, n * sizeof(kz_ray), cudaMemcpyHostToDevice, d->stream));
     if (d->pending.size() > 8192) fold_events(*d);
-    KZ_CUDA(ctx, cudaMemsetAsync(d->cursor, 0, 4, d->stream));
+    KZ_CUDA(ctx, cudaMemsetAsync(d->cursor.p, 0, 4, d->stream));
     {
         Timed t(*d, d->stream, CAT_TRACE);
-        k_occluded<<<d->grid_occ, KZ_TRACE_THREADS, 0, d->stream>>>(d->sc, reinterpret_cast<const KzF4 *>(d->scratch[0]), (uint32_t)n, trace_bias, d_occ, d_occ + n,
-                                                                    d->cursor, d->ctl);
+        k_occluded<<<d->grid_occ, KZ_TRACE_THREADS, 0, d->stream>>>(d->sc, reinterpret_cast<const KzF4 *>(d->scratch[0].p), (uint32_t)n, trace_bias, d_occ, d_occ + n,
+                                                                    d->cursor.as<uint32_t>(), d->ctl);
         ++d->launches;
     }
     KZ_CUDA(ctx, cudaMemcpyAsync(occluded, d_occ, n, cudaMemcpyDeviceToHost, d->stream));
@@ -1010,15 +1007,15 @@ int kzgpu_sample_dump(kzgpu_ctx *ctx, const int32_t *triples, size_t n, const ch
         per += (*p == '1') ? 1 : 2;
     }
     if (n == 0 || per == 0) return KZ_OK;
-    if ((rc = ensure_scratch(ctx, *d, 0, n * 12))) return rc;
-    if ((rc = ensure_scratch(ctx, *d, 1, n * per * 4))) return rc;
-    if ((rc = ensure_scratch(ctx, *d, 2, plen + 1))) return rc;
-    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0], triples, n * 12, cudaMemcpyHostToDevice, d->stream));
-    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[2], pattern, plen + 1, cudaMemcpyHostToDevice, d->stream));
-    k_sample_dump<<<(unsigned)((n + 127) / 128), 128, 0, d->stream>>>(d->sc, reinterpret_cast<const int32_t *>(d->scratch[0]), (uint32_t)n,
-                                                                      reinterpret_cast<const char *>(d->scratch[2]), (uint32_t)per, reinterpret_cast<float *>(d->scratch[1]));
+    KZ_CUDA(ctx, d->scratch[0].ensure(n * 12, SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[1].ensure(n * per * 4, SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[2].ensure(plen + 1, SCRATCH_MIN));
+    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0].p, triples, n * 12, cudaMemcpyHostToDevice, d->stream));
+    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[2].p, pattern, plen + 1, cudaMemcpyHostToDevice, d->stream));
+    k_sample_dump<<<(unsigned)((n + 127) / 128), 128, 0, d->stream>>>(d->sc, reinterpret_cast<const int32_t *>(d->scratch[0].p), (uint32_t)n,
+                                                                      reinterpret_cast<const char *>(d->scratch[2].p), (uint32_t)per, reinterpret_cast<float *>(d->scratch[1].p));
     ++d->launches;
-    KZ_CUDA(ctx, cudaMemcpyAsync(out, d->scratch[1], n * per * 4, cudaMemcpyDeviceToHost, d->stream));
+    KZ_CUDA(ctx, cudaMemcpyAsync(out, d->scratch[1].p, n * per * 4, cudaMemcpyDeviceToHost, d->stream));
     KZ_CUDA(ctx, cudaStreamSynchronize(d->stream));
     return KZ_OK;
 }
@@ -1030,12 +1027,12 @@ int kzgpu_camera_rays(kzgpu_ctx *ctx, const float *samples4, size_t n, kz_ray *o
     if ((rc = select(ctx, 0, &d))) return rc;
     if (n == 0) return KZ_OK;
     if (!samples4 || !out) return fail(ctx, KZ_ERR_INVALID, "null argument");
-    if ((rc = ensure_scratch(ctx, *d, 0, n * 16))) return rc;
-    if ((rc = ensure_scratch(ctx, *d, 1, n * 32))) return rc;
-    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0], samples4, n * 16, cudaMemcpyHostToDevice, d->stream));
-    k_camera_rays<<<(unsigned)((n + 127) / 128), 128, 0, d->stream>>>(d->sc, reinterpret_cast<const KzF4 *>(d->scratch[0]), (uint32_t)n, reinterpret_cast<KzF4 *>(d->scratch[1]));
+    KZ_CUDA(ctx, d->scratch[0].ensure(n * 16, SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[1].ensure(n * 32, SCRATCH_MIN));
+    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0].p, samples4, n * 16, cudaMemcpyHostToDevice, d->stream));
+    k_camera_rays<<<(unsigned)((n + 127) / 128), 128, 0, d->stream>>>(d->sc, reinterpret_cast<const KzF4 *>(d->scratch[0].p), (uint32_t)n, reinterpret_cast<KzF4 *>(d->scratch[1].p));
     ++d->launches;
-    KZ_CUDA(ctx, cudaMemcpyAsync(out, d->scratch[1], n * 32, cudaMemcpyDeviceToHost, d->stream));
+    KZ_CUDA(ctx, cudaMemcpyAsync(out, d->scratch[1].p, n * 32, cudaMemcpyDeviceToHost, d->stream));
     KZ_CUDA(ctx, cudaStreamSynchronize(d->stream));
     return KZ_OK;
 }
@@ -1054,12 +1051,12 @@ int kzgpu_bsdf_query(kzgpu_ctx *ctx, int bsdf, int mode, const float wi[3], cons
     for (int k = 0; k < 3; ++k) { q.wi[k] = wi[k]; q.wo[k] = wo ? wo[k] : 0.f; }
     q.uv[0] = uv[0]; q.uv[1] = uv[1]; q.acc_rough = accumulated_roughness; q.s1 = sample1;
     q.s2[0] = sample2 ? sample2[0] : 0.f; q.s2[1] = sample2 ? sample2[1] : 0.f; q.mode = mode;
-    if ((rc = ensure_scratch(ctx, *d, 0, sizeof(q)))) return rc;
-    if ((rc = ensure_scratch(ctx, *d, 1, 32))) return rc;
-    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0], &q, sizeof(q), cudaMemcpyHostToDevice, d->stream));
-    k_bsdf_query<<<1, 32, 0, d->stream>>>(d->sc, reinterpret_cast<const KzBsdfQuery *>(d->scratch[0]), 1u, reinterpret_cast<float *>(d->scratch[1]));
+    KZ_CUDA(ctx, d->scratch[0].ensure(sizeof(q), SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[1].ensure(32, SCRATCH_MIN));
+    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0].p, &q, sizeof(q), cudaMemcpyHostToDevice, d->stream));
+    k_bsdf_query<<<1, 32, 0, d->stream>>>(d->sc, reinterpret_cast<const KzBsdfQuery *>(d->scratch[0].p), 1u, reinterpret_cast<float *>(d->scratch[1].p));
     ++d->launches;
-    KZ_CUDA(ctx, cudaMemcpyAsync(out, d->scratch[1], 32, cudaMemcpyDeviceToHost, d->stream));
+    KZ_CUDA(ctx, cudaMemcpyAsync(out, d->scratch[1].p, 32, cudaMemcpyDeviceToHost, d->stream));
     KZ_CUDA(ctx, cudaStreamSynchronize(d->stream));
     return KZ_OK;
 }
@@ -1073,11 +1070,11 @@ int kzgpu_image_lookup(kzgpu_ctx *ctx, int image, int level, const float *st, si
     if (level < 0) return fail(ctx, KZ_ERR_INVALID, "negative mip level");
     if (n == 0) return KZ_OK;
     if (!st || !rgb) return fail(ctx, KZ_ERR_INVALID, "null argument");
-    if ((rc = ensure_scratch(ctx, *d, 0, n * 8))) return rc;
-    if ((rc = ensure_scratch(ctx, *d, 1, n * 12))) return rc;
+    KZ_CUDA(ctx, d->scratch[0].ensure(n * 8, SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[1].ensure(n * 12, SCRATCH_MIN));
     KzScene sc = d->sc;
     int lookup_image = image;
-    std::vector<void *> temp;
+    DevMem pyr_mem, rec_mem;
     if (level > 0) {
         /* the renderer only reads level 0 (ImageTexture::eval passes zero derivatives, texture.cpp:52-57), so the pyramid is not
          * kept resident: it is built here, for this image, by 2x2 box filtering on the device */
@@ -1086,10 +1083,10 @@ int kzgpu_image_lookup(kzgpu_ctx *ctx, int image, int level, const float *st, si
         size_t total = (size_t)im.width * im.height;
         for (int w = im.width, h = im.height; w > 1 || h > 1;) { w = w > 1 ? w >> 1 : 1; h = h > 1 ? h >> 1 : 1; total += (size_t)w * h; ++pr.n_levels; }
         KzF4 *pyr = nullptr; KzImageRec *rec = nullptr;
-        if ((rc = dev_alloc(ctx, temp, total, &pyr)) || (rc = dev_alloc(ctx, temp, 1, &rec))) { free_all(temp); return rc; }
+        if ((rc = dev_alloc(ctx, pyr_mem, total, &pyr)) || (rc = dev_alloc(ctx, rec_mem, 1, &rec))) return rc;
         cudaError_t e = cudaMemcpyAsync(pyr, d->sc.texels + im.texel_offset, (size_t)im.width * im.height * sizeof(KzF4), cudaMemcpyDeviceToDevice, d->stream);
         if (e == cudaSuccess) e = cudaMemcpyAsync(rec, &pr, sizeof(pr), cudaMemcpyHostToDevice, d->stream);
-        if (e != cudaSuccess) { free_all(temp); KZ_CUDA(ctx, e); }
+        KZ_CUDA(ctx, e);
         size_t src = 0; int sw = im.width, sh = im.height;
         for (int l = 1; l <= pr.n_levels; ++l) {
             const int dw = sw > 1 ? sw >> 1 : 1, dh = sh > 1 ? sh >> 1 : 1;
@@ -1101,15 +1098,14 @@ int kzgpu_image_lookup(kzgpu_ctx *ctx, int image, int level, const float *st, si
         }
         sc.texels = pyr; sc.images = rec; lookup_image = 0;
     }
-    cudaError_t e = cudaMemcpyAsync(d->scratch[0], st, n * 8, cudaMemcpyHostToDevice, d->stream);
+    cudaError_t e = cudaMemcpyAsync(d->scratch[0].p, st, n * 8, cudaMemcpyHostToDevice, d->stream);
     if (e == cudaSuccess) {
-        k_image_lookup<<<(unsigned)((n + 127) / 128), 128, 0, d->stream>>>(sc, lookup_image, level, reinterpret_cast<const float *>(d->scratch[0]), (uint32_t)n,
-                                                                           reinterpret_cast<float *>(d->scratch[1]));
+        k_image_lookup<<<(unsigned)((n + 127) / 128), 128, 0, d->stream>>>(sc, lookup_image, level, reinterpret_cast<const float *>(d->scratch[0].p), (uint32_t)n,
+                                                                           reinterpret_cast<float *>(d->scratch[1].p));
         ++d->launches;
-        e = cudaMemcpyAsync(rgb, d->scratch[1], n * 12, cudaMemcpyDeviceToHost, d->stream);
+        e = cudaMemcpyAsync(rgb, d->scratch[1].p, n * 12, cudaMemcpyDeviceToHost, d->stream);
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(d->stream);
-    free_all(temp);
     KZ_CUDA(ctx, e);
     return KZ_OK;
 }
@@ -1122,13 +1118,13 @@ int kzgpu_intersection_dump(kzgpu_ctx *ctx, const kz_ray *rays, size_t n, float 
     if (n == 0) return KZ_OK;
     if (!rays || !out24) return fail(ctx, KZ_ERR_INVALID, "null argument");
     if (n > 0x7FFFFFFFull) return fail(ctx, KZ_ERR_INVALID, "batch larger than 2^31-1 rays");
-    if ((rc = ensure_scratch(ctx, *d, 0, n * sizeof(kz_ray)))) return rc;
-    if ((rc = ensure_scratch(ctx, *d, 1, n * 96))) return rc;
-    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0], rays, n * sizeof(kz_ray), cudaMemcpyHostToDevice, d->stream));
-    k_intersection_dump<<<(unsigned)((n + KZ_TRACE_THREADS - 1) / KZ_TRACE_THREADS), KZ_TRACE_THREADS, 0, d->stream>>>(d->sc, reinterpret_cast<const KzF4 *>(d->scratch[0]), (uint32_t)n,
-                                                                                                                    reinterpret_cast<float *>(d->scratch[1]));
+    KZ_CUDA(ctx, d->scratch[0].ensure(n * sizeof(kz_ray), SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[1].ensure(n * 96, SCRATCH_MIN));
+    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0].p, rays, n * sizeof(kz_ray), cudaMemcpyHostToDevice, d->stream));
+    k_intersection_dump<<<(unsigned)((n + KZ_TRACE_THREADS - 1) / KZ_TRACE_THREADS), KZ_TRACE_THREADS, 0, d->stream>>>(d->sc, reinterpret_cast<const KzF4 *>(d->scratch[0].p), (uint32_t)n,
+                                                                                                                    reinterpret_cast<float *>(d->scratch[1].p));
     ++d->launches;
-    KZ_CUDA(ctx, cudaMemcpyAsync(out24, d->scratch[1], n * 96, cudaMemcpyDeviceToHost, d->stream));
+    KZ_CUDA(ctx, cudaMemcpyAsync(out24, d->scratch[1].p, n * 96, cudaMemcpyDeviceToHost, d->stream));
     KZ_CUDA(ctx, cudaStreamSynchronize(d->stream));
     return KZ_OK;
 }
@@ -1141,15 +1137,15 @@ int kzgpu_light_sample_dump(kzgpu_ctx *ctx, const float *ref3, const float *u5, 
     if (n == 0) return KZ_OK;
     if (!ref3 || !u5 || !out16) return fail(ctx, KZ_ERR_INVALID, "null argument");
     if (n > 0x7FFFFFFFull) return fail(ctx, KZ_ERR_INVALID, "batch too large");
-    if ((rc = ensure_scratch(ctx, *d, 0, n * 12))) return rc;
-    if ((rc = ensure_scratch(ctx, *d, 1, n * 64))) return rc;
-    if ((rc = ensure_scratch(ctx, *d, 2, n * 20))) return rc;
-    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0], ref3, n * 12, cudaMemcpyHostToDevice, d->stream));
-    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[2], u5, n * 20, cudaMemcpyHostToDevice, d->stream));
-    k_light_sample_dump<<<(unsigned)((n + 127) / 128), 128, 0, d->stream>>>(d->sc, reinterpret_cast<const float *>(d->scratch[0]), reinterpret_cast<const float *>(d->scratch[2]),
-                                                                            (uint32_t)n, reinterpret_cast<float *>(d->scratch[1]));
+    KZ_CUDA(ctx, d->scratch[0].ensure(n * 12, SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[1].ensure(n * 64, SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[2].ensure(n * 20, SCRATCH_MIN));
+    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0].p, ref3, n * 12, cudaMemcpyHostToDevice, d->stream));
+    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[2].p, u5, n * 20, cudaMemcpyHostToDevice, d->stream));
+    k_light_sample_dump<<<(unsigned)((n + 127) / 128), 128, 0, d->stream>>>(d->sc, reinterpret_cast<const float *>(d->scratch[0].p), reinterpret_cast<const float *>(d->scratch[2].p),
+                                                                            (uint32_t)n, reinterpret_cast<float *>(d->scratch[1].p));
     ++d->launches;
-    KZ_CUDA(ctx, cudaMemcpyAsync(out16, d->scratch[1], n * 64, cudaMemcpyDeviceToHost, d->stream));
+    KZ_CUDA(ctx, cudaMemcpyAsync(out16, d->scratch[1].p, n * 64, cudaMemcpyDeviceToHost, d->stream));
     KZ_CUDA(ctx, cudaStreamSynchronize(d->stream));
     return KZ_OK;
 }
@@ -1181,16 +1177,15 @@ int kzgpu_render_device(kzgpu_ctx *ctx, int device, const kz_render_req *req, vo
     Device *d;
     if ((rc = select(ctx, device, &d))) return rc;
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    /* caller-owned frame (e.g. a torch tensor that an NCCL reduce follows) or the context's own */
-    KzF4 *own = d->frame;
+    /* caller-owned frame (e.g. a torch tensor that an NCCL reduce follows) for this call, or the context's own */
     if (d_frame_inout && *d_frame_inout) d->frame = reinterpret_cast<KzF4 *>(*d_frame_inout);
     if (req->clear_frame) {
         cudaError_t e = cudaMemsetAsync(d->frame, 0, d->frame_texels * sizeof(KzF4), s);
-        if (e != cudaSuccess) { d->frame = own; return fail(ctx, KZ_ERR_CUDA, std::string("cudaMemsetAsync(frame): ") + cudaGetErrorString(e)); }
+        if (e != cudaSuccess) { d->frame = d->frame_mem.as<KzF4>(); return fail(ctx, KZ_ERR_CUDA, std::string("cudaMemsetAsync(frame): ") + cudaGetErrorString(e)); }
     }
     rc = enqueue_render(ctx, ctx, *d, *req, s);
     if (d_frame_inout) *d_frame_inout = d->frame;
-    d->frame = own;
+    d->frame = d->frame_mem.as<KzF4>();
     return rc;
 }
 
@@ -1271,16 +1266,16 @@ int kzgpu_resolve(kzgpu_ctx *ctx, const float *frame_rgbw, float *rgb_linear, ui
     const KzScene &sc = d->sc;
     const int W = sc.camera.width, H = sc.camera.height;
     const size_t npx = (size_t)W * H;
-    if ((rc = ensure_scratch(ctx, *d, 0, d->frame_texels * sizeof(KzF4)))) return rc;
-    if ((rc = ensure_scratch(ctx, *d, 1, npx * 12))) return rc;
-    if ((rc = ensure_scratch(ctx, *d, 2, npx * 3))) return rc;
-    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0], frame_rgbw, d->frame_texels * sizeof(KzF4), cudaMemcpyHostToDevice, d->stream));
+    KZ_CUDA(ctx, d->scratch[0].ensure(d->frame_texels * sizeof(KzF4), SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[1].ensure(npx * 12, SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[2].ensure(npx * 3, SCRATCH_MIN));
+    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0].p, frame_rgbw, d->frame_texels * sizeof(KzF4), cudaMemcpyHostToDevice, d->stream));
     dim3 blk(32, 8), grd((unsigned)(W + 31) / 32, (unsigned)(H + 7) / 8);
-    k_resolve<<<grd, blk, 0, d->stream>>>(reinterpret_cast<const KzF4 *>(d->scratch[0]), W, H, sc.border, rgb_linear ? reinterpret_cast<float *>(d->scratch[1]) : nullptr,
-                                          srgb8 ? reinterpret_cast<uint8_t *>(d->scratch[2]) : nullptr);
+    k_resolve<<<grd, blk, 0, d->stream>>>(reinterpret_cast<const KzF4 *>(d->scratch[0].p), W, H, sc.border, rgb_linear ? reinterpret_cast<float *>(d->scratch[1].p) : nullptr,
+                                          srgb8 ? reinterpret_cast<uint8_t *>(d->scratch[2].p) : nullptr);
     ++d->launches;
-    if (rgb_linear) KZ_CUDA(ctx, cudaMemcpyAsync(rgb_linear, d->scratch[1], npx * 12, cudaMemcpyDeviceToHost, d->stream));
-    if (srgb8) KZ_CUDA(ctx, cudaMemcpyAsync(srgb8, d->scratch[2], npx * 3, cudaMemcpyDeviceToHost, d->stream));
+    if (rgb_linear) KZ_CUDA(ctx, cudaMemcpyAsync(rgb_linear, d->scratch[1].p, npx * 12, cudaMemcpyDeviceToHost, d->stream));
+    if (srgb8) KZ_CUDA(ctx, cudaMemcpyAsync(srgb8, d->scratch[2].p, npx * 3, cudaMemcpyDeviceToHost, d->stream));
     KZ_CUDA(ctx, cudaStreamSynchronize(d->stream));
     return KZ_OK;
 }

@@ -17,6 +17,7 @@
 #define KZ_LBVH_CUH
 #include "kz_scene.h"
 #include "kz_bvh_build.h"
+#include "kz_owner.h"
 #include <cub/device/device_radix_sort.cuh>
 #include <cuda_runtime.h>
 #include <string>
@@ -25,8 +26,7 @@
 namespace kzlbvh {
 
 struct Result {
-    const KzNode8 *nodes = nullptr;
-    const KzF4 *tris = nullptr;
+    DevMem nodes, tris;          /* KzNode8[n_nodes] (allocated for more), KzF4[3 * n_tris] */
     uint32_t n_nodes = 0, n_tris = 0;
     float max_abs = 0.f;
     uint64_t launches = 0;
@@ -409,9 +409,9 @@ __global__ void k_make_refs(const kzbvh::Tri *tris, uint32_t n, const uint32_t *
 
 #define KZ_LBVH_MAX_LEVELS 31     /* levels the collapse walks; the API accepts KZ_MAX_ACCEL_DEPTH = 30 of them (stack budget in kz_traverse.h) */
 
-/* Builds the accel of the `n_tris_in` device-resident triangles `d_tris` (scene order) on the current device; the node/triangle
- * arrays are appended to `owner` (freed by the caller), temporaries are released before returning. */
-inline int build(const kzbvh::Tri *d_tris, uint32_t n_tris_in, cudaStream_t s, std::vector<void *> &owner, Result &r, std::string &err) {
+/* Builds the accel of the `n_tris_in` device-resident triangles `d_tris` (scene order) on the current device; `r` owns the node and
+ * triangle arrays (also after a failure), temporaries are released before returning. */
+inline int build(const kzbvh::Tri *d_tris, uint32_t n_tris_in, cudaStream_t s, Result &r, std::string &err) {
     std::vector<void *> temp;
     uint32_t n = n_tris_in;                  /* references: == triangles unless pre-splitting adds some */
     r = Result();
@@ -477,11 +477,8 @@ inline int build(const kzbvh::Tri *d_tris, uint32_t n_tris_in, cudaStream_t s, s
      * of n nodes is loose but safe (a wide node owns >= 1 triangle or >= 2 wide children) */
     KzNode8 *d_nodes; KzF4 *d_out_tris; uint32_t *counters; WorkItem *w0, *w1;
     const size_t max_nodes = (size_t)n;
-    {
-        void *p = nullptr;
-        KZL_CUDA(cudaMalloc(&p, max_nodes * sizeof(KzNode8))); owner.push_back(p); d_nodes = (KzNode8 *)p;
-        KZL_CUDA(cudaMalloc(&p, (size_t)n * 3 * sizeof(KzF4))); owner.push_back(p); d_out_tris = (KzF4 *)p;
-    }
+    KZL_CUDA(r.nodes.alloc(max_nodes * sizeof(KzNode8))); d_nodes = r.nodes.as<KzNode8>();
+    KZL_CUDA(r.tris.alloc((size_t)n * 3 * sizeof(KzF4))); d_out_tris = r.tris.as<KzF4>();
     /* counters[0] = wide nodes (root taken), [1] = emitted triangles, [2 + l] = work items of level l */
     uint32_t cinit[4 + KZ_LBVH_MAX_LEVELS];
     memset(cinit, 0, sizeof(cinit));
@@ -513,7 +510,7 @@ inline int build(const kzbvh::Tri *d_tris, uint32_t n_tris_in, cudaStream_t s, s
     KZL_CUDA(cudaMemcpyAsync(hb, bounds, 32, cudaMemcpyDeviceToHost, s));
     KZL_CUDA(cudaStreamSynchronize(s));
     KZL_CUDA(cudaGetLastError());
-    r.nodes = d_nodes; r.tris = d_out_tris; r.n_nodes = fin[0]; r.n_tris = fin[1];
+    r.n_nodes = fin[0]; r.n_tris = fin[1];
     r.max_abs = ord2f(hb[6]);
     for (int l = 0; l < KZ_LBVH_MAX_LEVELS && fin[2 + l] != 0u; ++l) r.depth = l + 1;
     /* level l + 1 is allocated (node_counter) while level l runs, so the levels are consecutive ranges in launch order */
