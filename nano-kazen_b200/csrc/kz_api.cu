@@ -63,7 +63,7 @@ struct Device {
     DevMem frame_mem;                /* the context's own frame; frame may point at a caller's instead (kzgpu_render_device) */
     KzF4 *frame = nullptr;
     size_t frame_texels = 0;
-    /* primary-hit hints (KzExtendJob<true>::seed): (geomID, primID) per film pixel, allocated by the first render that uses them and
+    /* primary-hit hints (k_raygen runs the seed test, KzExtendJob<true>::seed installs it): (geomID, primID) per film pixel, allocated by the first render that uses them and
      * invalidated (all 0xFF) whenever the accel or the film may have changed -- a hint is only worth something for the same triangles */
     DevMem hint;
     bool hint_stale = true;
@@ -100,7 +100,7 @@ struct kzgpu_ctx {
     bool uploaded = false, built = false;
     uint32_t pool_cap = 1u << 24;     /* path slots per chunk and lane (160 B each = 2.5 GiB): every launch costs ~18 us of ramp + tail, so few big chunks win */
     int lanes = 3;                    /* concurrent chunks per device at most, 1..4 (KZGPU_LANES=1: strictly serial chunks); frames below 2^25 paths use two */
-    int primary_hint = 1;             /* seed primary rays with the triangle their pixel hit last (KzExtendJob<true>::seed; KZGPU_PRIMARY_HINT / "primary_hint"):
+    int primary_hint = 1;             /* seed primary rays with the triangle their pixel hit last (k_raygen, KzExtendJob<true>::seed; KZGPU_PRIMARY_HINT / "primary_hint"):
                                        * 0 = never, 1 = for scenes of at least KZ_HINT_MIN_TRIS triangles, 2 = always.  Measured on B200, Mpaths/s off -> on:
                                        * 10^8-triangle 4K headline 909 -> 975 (primary pass ~25 % shorter); WarmStudio.xml 1292 -> 1269, configs[2] 873 -> 866,
                                        * configs[3] 849 -> 838 (few triangles: the primaries are cheap, the extra loads and spills of the seed are not) */
@@ -390,7 +390,7 @@ int enqueue_chunk(const kzgpu_ctx *ctx, kzgpu_ctx *ectx, Device &d, Lane &L, con
     {
         Timed t(d, s, CAT_SHADE);
         k_chunk_reset<<<1, 32, 0, s>>>(L.ctl, ch.count, new_paths);
-        k_raygen<<<(ch.count + KZ_SHADE_THREADS - 1) / KZ_SHADE_THREADS, KZ_SHADE_THREADS, 0, s>>>(sc, L.st, L.q.ext[0], ch);
+        k_raygen<<<(ch.count + KZ_SHADE_THREADS - 1) / KZ_SHADE_THREADS, KZ_SHADE_THREADS, 0, s>>>(sc, L.st, hint, ch);
         d.launches += 2;
     }
     if (alt) {

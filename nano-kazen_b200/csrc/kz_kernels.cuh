@@ -126,7 +126,7 @@ __device__ __forceinline__ void kz_flush_counters(KzControl *ctl, const KzCounte
  * Job: per-lane policy object.
  *   void begin(uint32_t item, KzRayIn &r)                   load the ray of work item `item`
  *   void seed(const KzScene &sc, KzTrav &t)                 called right after the traversal of that ray was initialised: may preset
- *                                                           its best hit (kz_trav_seed); not called for follow-up rays
+ *                                                           its best hit (kz_trav_preset); not called for follow-up rays
  *   bool end(uint32_t item, const KzHit &h, KzRayIn &r)     consume the closest hit; return true and fill `r`
  *                                                           to continue the same item with a follow-up ray
  *   static constexpr bool kStopsEarly                       the job only asks WHETHER something opaque is hit (shadow rays)
@@ -266,7 +266,7 @@ __device__ __forceinline__ void kz_push_divergent(uint32_t *const *queues, uint3
     queues[which][base + (uint32_t)__popc(peers & ((1u << lane) - 1u))] = value;
 }
 
-/* Start of a chunk: raygen fills every slot, so the first extension queue is the identity over `count` slots (no atomics). */
+/* Start of a chunk: raygen fills every slot, so the first extension pass takes slots 0 .. count-1 in order (k_extend<true> reads no queue). */
 __global__ void k_chunk_reset(KzControl *ctl, uint32_t count, unsigned long long new_paths) {
     if (threadIdx.x == 0) {
         ctl->ext_shadow[0] = (unsigned long long)count; ctl->ext_shadow[1] = 0ull;
@@ -287,8 +287,13 @@ __global__ void k_bounce_reset(KzControl *ctl, int nxt) {
 /* Slot i of the chunk = global path index first+i; a warp is one 8x4 pixel tile of one sample index: coherent primary rays,
  * and the splats of a warp land on neighbouring frame texels instead of piling onto one pixel.  Consecutive warps are
  * consecutive sample indices of the SAME tile (KzChunk::spp_group of them), so the warps resident on an SM walk the same
- * part of the accel and shade neighbouring surface points. */
-__global__ void __launch_bounds__(KZ_SHADE_THREADS) k_raygen(KzScene sc, KzPathState st, uint32_t *q0, KzChunk ch) {
+ * part of the accel and shade neighbouring surface points.
+ * hint: per film pixel the (geomID, primID) its last primary ray hit, or nullptr (no hints).  With hints, raygen also runs the seed test
+ * of the ray it has just generated against its pixel's hint (kz_seed_hit) and leaves the result, and the pixel, in the path's hit record
+ * for k_extend<true>.  The test is a chain of dependent loads (hint, mesh, index record, vertices): here every lane of the warp runs it
+ * at once, in a short kernel whose many resident warps hide the latency; at the refill point of the traversal loop only the refilled
+ * lanes ran it while the whole warp waited. */
+__global__ void __launch_bounds__(KZ_SHADE_THREADS) k_raygen(KzScene sc, KzPathState st, const uint2 *hint, KzChunk ch) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= ch.count) return;
     /* path order: (block of spp_group sample indices, tile, sample index in the block, pixel of the tile) */
@@ -303,8 +308,16 @@ __global__ void __launch_bounds__(KZ_SHADE_THREADS) k_raygen(KzScene sc, KzPathS
     const uint32_t s_local = blk * ch.spp_group + (r >> 5), in_tile = r & 31u;
     const int x = ch.x0 + (int)((tile % ch.tiles_x) * 8u + (in_tile & 7u));
     const int y = ch.y0 + (int)((tile / ch.tiles_x) * 4u + (in_tile >> 3));
-    if (x < ch.x1 && y < ch.y1) kz_raygen_item(sc, st, i, x, y, (uint32_t)(ch.spp_begin + (int)s_local));
-    else {
+    KzHit seed; seed.t = seed.u = seed.v = 0.f; seed.prim = seed.geom = KZ_INVALID_ID;
+    uint32_t pix = 0xFFFFFFFFu;
+    if (x < ch.x1 && y < ch.y1) {
+        const KzRayRec ray = kz_raygen_item(sc, st, i, x, y, (uint32_t)(ch.spp_begin + (int)s_local));
+        if (hint != nullptr) {
+            const uint2 h = hint[(size_t)y * (uint32_t)sc.camera.width + (uint32_t)x];
+            kz_seed_hit(sc, ray.o.x, ray.o.y, ray.o.z, ray.d.x, ray.d.y, ray.d.z, ray.o.w, ray.d.w, h.x, h.y, seed);
+            pix = (uint32_t)x | ((uint32_t)y << 16);
+        }
+    } else {
         /* padding lane of a tile that sticks out of the rectangle: a NaN ray (k_extend<true> drops it without counting it)
          * and the marker k_accumulate skips */
         const float nan = kz_u2f(0x7FC00000u);
@@ -312,7 +325,11 @@ __global__ void __launch_bounds__(KZ_SHADE_THREADS) k_raygen(KzScene sc, KzPathS
         st.a[i].ray = ray;
         st.b[i].smp.pix = 0xFFFFFFFFu;
     }
-    q0[i] = i;      /* one warp-sized run of the queue = one tile of one sample index */
+    if (hint != nullptr) {
+        KzHitRec rec = mk_hit_rec(seed);
+        rec.pix = pix;
+        st.a[i].hit = rec;
+    }
 }
 
 /* ---- extend: Scene::rayIntersect for every queued path, then sort by material class ------- */
@@ -328,24 +345,25 @@ struct KzExtendJob {
     kz3 d;
     __device__ KzExtendJob(const KzScene &s, const KzPathState &p, KzControl *c, const KzQueues &qq, const uint32_t *qu, uint2 *h)
         : sc(s), st(p), ctl(c), q(qq), queue(qu), hint(h), n_seeded(0u) { cnt.paths = cnt.rays_ext = cnt.rays_shadow = cnt.vertices = cnt.rays_seeded = 0ull; }
-    /* hint slot of the path's pixel; ~0 for the padding lanes of k_raygen (pix = 0xFFFFFFFF lies outside every film) */
+    /* hint slot of the path's pixel (KzHitRec::pix, written by k_raygen); ~0 for its padding lanes (0xFFFFFFFF lies outside every film) */
     __device__ __forceinline__ size_t hint_index() const {
-        const uint32_t pix = st.b[slot].smp.pix, px = pix & 0xFFFFu, py = pix >> 16;
+        const uint32_t pix = st.a[slot].hit.pix, px = pix & 0xFFFFu, py = pix >> 16;
         if (px >= (uint32_t)sc.camera.width || py >= (uint32_t)sc.camera.height) return ~(size_t)0;
         return (size_t)py * (uint32_t)sc.camera.width + px;
     }
     /* One triangle covers several pixels and every pixel is sampled many times, so the triangle the pixel's last primary ray hit is
      * usually hit again: as the preset best hit it lets the node step cull with its t from the root on, instead of walking every
-     * box along the ray up to the hit.  The hit found is the same either way (kz_trav_seed). */
-    __device__ __forceinline__ void seed(const KzScene &s, KzTrav &t) {
+     * box along the ray up to the hit.  The hit found is the same either way (kz_seed_hit).  k_raygen ran the seed test; this loads its
+     * result (one load: the slot is the item) and installs it.  Loaded here rather than with the ray in begin(), it is not held across
+     * kz_trav_init: 52 instead of 72 bytes of spills. */
+    __device__ __forceinline__ void seed(const KzScene &, KzTrav &t) {
         if (!FIRST || hint == nullptr) return;
-        const size_t i = hint_index();
-        if (i == ~(size_t)0) return;
-        const uint2 h = hint[i];
-        n_seeded += kz_trav_seed(s, t, h.x, h.y) ? 1u : 0u;
+        const KzHitRec s = st.a[slot].hit;
+        KzHit h; h.t = s.t; h.u = s.u; h.v = s.v; h.prim = s.prim; h.geom = s.geom;
+        n_seeded += kz_trav_preset(t, h) ? 1u : 0u;
     }
     __device__ __forceinline__ void begin(uint32_t item, KzRayIn &r) {
-        slot = queue[item];
+        slot = FIRST ? item : queue[item];          /* the first pass takes the chunk's slots in order (k_chunk_reset) */
         const KzRayRec ray = st.a[slot].ray;
         const KzF4 ro = ray.o, rd = ray.d;
         r.ox = ro.x; r.oy = ro.y; r.oz = ro.z; r.tmin = ro.w; r.dx = rd.x; r.dy = rd.y; r.dz = rd.z; r.tmax = rd.w;

@@ -28,7 +28,10 @@
  * Not stored: bsdfWeight (only lives between the tail of one loop iteration and the head of the next, both inside one shade
  * pass) and the pixel sample position (recomputed from the addressable sampler when the path is splatted). */
 struct alignas(16) KzRayRec { KzF4 o, d; };                          /* o.xyz tmin | d.xyz tmax */
-struct alignas(16) KzHitRec { float t, u, v; uint32_t prim, geom, pad0, pad1, pad2; };
+/* Hit record.  Between k_raygen and k_extend<true>, with primary-hit hints on, it holds the seed of the primary ray (kz_seed_hit; an
+ * invalid hit if there is none) and `pix` carries the film pixel the hint goes back to (as KzSmpRec::pix; 0xFFFFFFFF on padding lanes).
+ * No other stage reads `pix`: it is 0 in every hit that extend stores. */
+struct alignas(16) KzHitRec { float t, u, v; uint32_t prim, geom, pix, pad1, pad2; };
 struct alignas(64) KzBlockA { KzRayRec ray; KzHitRec hit; };
 struct alignas(16) KzRadRec { KzF4 thr, L; };                        /* throughput rgb, eta | Li rgb, bsdfPdf (< 0: discrete) */
 struct alignas(16) KzSmpRec { uint64_t rng_state, rng_inc; uint32_t dim, pix /* px | py << 16 */, sidx; float acc_rough; };
@@ -42,7 +45,7 @@ struct KzPathState {
     KzBlockB *b;
     KzBlockC *c;
 };
-KZ_HD KzHitRec mk_hit_rec(const KzHit &h) { KzHitRec r; r.t = h.t; r.u = h.u; r.v = h.v; r.prim = h.prim; r.geom = h.geom; r.pad0 = r.pad1 = r.pad2 = 0u; return r; }
+KZ_HD KzHitRec mk_hit_rec(const KzHit &h) { KzHitRec r; r.t = h.t; r.u = h.u; r.v = h.v; r.prim = h.prim; r.geom = h.geom; r.pix = r.pad1 = r.pad2 = 0u; return r; }
 
 struct KzCounters {
     unsigned long long paths, rays_ext, rays_shadow, vertices, rays_seeded;     /* rays_seeded: primary rays that started from a hit hint */
@@ -109,7 +112,8 @@ KZ_HD void kz_sampler_load(KzSampler &sm, const KzSmpRec &r) {
 }
 
 /* ---- raygen -------------------------------------------------------------------------------- */
-KZ_HD void kz_raygen_item(const KzScene &sc, const KzPathState &st, uint32_t slot, int px, int py, uint32_t sample_index) {
+/* Writes the path's camera ray and its throughput / sampler state; returns the ray. */
+KZ_HD KzRayRec kz_raygen_item(const KzScene &sc, const KzPathState &st, uint32_t slot, int px, int py, uint32_t sample_index) {
     KzSampler sm;
     kz_sampler_start(sc, sm, px, py, sample_index);
     kz2 pix = kz_next_pixel2d(sc, sm);
@@ -121,6 +125,7 @@ KZ_HD void kz_raygen_item(const KzScene &sc, const KzPathState &st, uint32_t slo
     st.a[slot].ray = ray;
     KzBlockB B; B.rad.thr = mkf4(1.f, 1.f, 1.f, 1.f); B.rad.L = mkf4(0.f, 0.f, 0.f, 0.f); B.smp = kz_sampler_save(sm, 0.f);
     st.b[slot] = B;
+    return ray;
 }
 
 KZ_HD int kz_classify(const KzScene &sc, uint32_t geom) {

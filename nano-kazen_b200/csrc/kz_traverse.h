@@ -177,6 +177,12 @@ struct KzTrav {
 };
 struct KzLocalStack { uint32_t x[KZ_LOCAL_STACK], y[KZ_LOCAL_STACK]; };
 
+/* False if a traversal of this ray is an immediate miss: an empty accel, or a NaN component (see kz_trav_init). */
+KZ_HD bool kz_trav_starts(const KzScene &sc, float ox, float oy, float oz, float dx, float dy, float dz, float tmin, float tmax) {
+    const bool has_nan = isnan(ox) || isnan(oy) || isnan(oz) || isnan(dx) || isnan(dy) || isnan(dz) || isnan(tmin) || isnan(tmax);
+    return sc.n_nodes != 0 && !has_nan;
+}
+
 KZ_HD void kz_trav_init(const KzScene &sc, KzTrav &t, float ox, float oy, float oz, float dx, float dy, float dz, float tmin, float tmax) {
     t.ox = ox; t.oy = oy; t.oz = oz; t.dx = dx; t.dy = dy; t.dz = dz; t.tmin = tmin;
     t.best.t = tmax; t.best.u = 0.f; t.best.v = 0.f; t.best.prim = KZ_INVALID_ID; t.best.geom = KZ_INVALID_ID;
@@ -192,8 +198,7 @@ KZ_HD void kz_trav_init(const KzScene &sc, KzTrav &t, float ox, float oy, float 
     /* A ray with a NaN component can never be accepted by the triangle test (every comparison fails), but fminf/fmaxf drop
      * NaNs, so the slab test would let it walk the whole tree.  Such rays do occur -- the reference's cosine-hemisphere warp
      * yields sqrt(-eps) for a sample that is exactly 0 (warp.cpp:85-115) -- so they are turned into an immediate miss. */
-    const bool has_nan = isnan(ox) || isnan(oy) || isnan(oz) || isnan(dx) || isnan(dy) || isnan(dz) || isnan(tmin) || isnan(tmax);
-    t.ng_x = 0u; t.ng_y = (sc.n_nodes && !has_nan) ? 0x80000000u : 0u;      /* root; an empty scene starts with nothing to do */
+    t.ng_x = 0u; t.ng_y = kz_trav_starts(sc, ox, oy, oz, dx, dy, dz, tmin, tmax) ? 0x80000000u : 0u;      /* root, or nothing to do */
     t.tg_x = 0u; t.tg_y = 0u; t.tg_m = 0u;
     t.sp = 0;
 }
@@ -344,10 +349,13 @@ KZ_HD bool kz_trav_tri(const KzScene &sc, KzTrav &t) {
     return false;
 }
 
-/* Presets the best hit of a freshly initialised traversal with triangle `prim` of mesh `geom` (a hint, e.g. what this ray's pixel
- * hit last time) if the ray hits it; returns true if it did.  An index out of range, or KZ_INVALID_ID, leaves the traversal as it was.
+/* The seed test: true if the ray (o, d) hits triangle `prim` of mesh `geom` (a hint, e.g. what this ray's pixel hit last time) inside
+ * [tmin, tmax]; fills `h` with that hit.  An index out of range, or KZ_INVALID_ID, is no hit, and so is every ray whose traversal would be
+ * an immediate miss (kz_trav_starts: NaN ray, empty accel).  k_raygen runs it on the primary ray it has just generated and leaves the
+ * result in the path's hit record for k_extend<true> to install (kz_trav_preset); kz_trav_seed runs it on a traversal's own ray.
  *
- * The closest hit the traversal returns does not change, so a wrong or stale hint costs time, never correctness:
+ * Installed as the best hit of a fresh traversal (t.best.t == tmax), a seed does not change the closest hit the traversal returns, so a
+ * wrong or stale hint costs time, never correctness:
  *   - kz_trav_tri keeps the minimum of (t, geomID, primID) over the triangles it accepts, and kz_pluecker accepts t <= tfar
  *     inclusively, so the true closest triangle -- whose t is <= the seed's -- still becomes the best hit when it is tested, and a
  *     tie at equal t still goes to the smaller (geomID, primID);
@@ -356,18 +364,31 @@ KZ_HD bool kz_trav_tri(const KzScene &sc, KzTrav &t) {
  *   - if the seed is the closest triangle itself, its t, u, v must be the bits the traversal computes for it.  They are: the vertices
  *     are read from the shading records (KzVertex px|py|pz through the index record), which are the very floats, in the very order,
  *     that the accel's 48-byte triangle record was gathered from (k_gather_tris, KzHostScene::flatten; both builders copy them
- *     unchanged), and the test is the same kz_pluecker with the same tnear (t.tmin) and tfar (the ray's tmax). */
-KZ_HD bool kz_trav_seed(const KzScene &sc, KzTrav &t, uint32_t geom, uint32_t prim) {
-    if (geom >= sc.n_meshes || t.ng_y == 0u) return false;          /* kz_trav_init made it an immediate miss (NaN ray, empty accel) */
+ *     unchanged), and the test is the same kz_pluecker with the same tnear (the ray's tmin) and tfar (the ray's tmax).  k_raygen tests
+ *     the very ray bits it stores, and k_extend<true> traverses the bits it loads back. */
+KZ_HD bool kz_seed_hit(const KzScene &sc, float ox, float oy, float oz, float dx, float dy, float dz, float tmin, float tmax,
+                       uint32_t geom, uint32_t prim, KzHit &h) {
+    if (geom >= sc.n_meshes || !kz_trav_starts(sc, ox, oy, oz, dx, dy, dz, tmin, tmax)) return false;
     const KzMeshRec &m = sc.meshes[geom];
     if (prim >= m.n_triangles) return false;
     const KzU4 ix = kz_load_u4(sc.indices + (m.index_offset + prim));
     const KzVertex *vb = sc.vertices + m.vertex_offset;
     const KzU4 a = kz_load_u4(vb + ix.x), b = kz_load_u4(vb + ix.y), c = kz_load_u4(vb + ix.z);      /* px, py, pz, (u: unused) */
-    float tt, u, v;
-    if (!kz_pluecker(t.ox, t.oy, t.oz, t.dx, t.dy, t.dz, t.tmin, t.best.t, a, b, c, tt, u, v)) return false;
-    t.best.t = tt; t.best.u = u; t.best.v = v; t.best.geom = geom; t.best.prim = prim;
+    if (!kz_pluecker(ox, oy, oz, dx, dy, dz, tmin, tmax, a, b, c, h.t, h.u, h.v)) return false;
+    h.geom = geom; h.prim = prim;
     return true;
+}
+/* Presets the best hit of a freshly initialised traversal with a seed hit (kz_seed_hit on the same ray); returns true if it did.  An
+ * invalid hit, or a traversal that kz_trav_init made an immediate miss, leaves the traversal as it was. */
+KZ_HD bool kz_trav_preset(KzTrav &t, const KzHit &h) {
+    if (h.geom == KZ_INVALID_ID || t.ng_y == 0u) return false;
+    t.best = h;
+    return true;
+}
+/* Seeds a freshly initialised traversal with a hint (kz_seed_hit on its ray, then kz_trav_preset); returns true if the ray hit it. */
+KZ_HD bool kz_trav_seed(const KzScene &sc, KzTrav &t, uint32_t geom, uint32_t prim) {
+    KzHit h;
+    return kz_seed_hit(sc, t.ox, t.oy, t.oz, t.dx, t.dy, t.dz, t.tmin, t.best.t, geom, prim, h) && kz_trav_preset(t, h);
 }
 
 /* The plain per-ray loop.  `stk` gives the shared-memory short stack on the device; on the host
