@@ -246,6 +246,12 @@ typedef struct kz_stats {
 
 #define KZ_BUILD_HOST_SAH 0    /* binned SAH on the host, collapsed to 8-wide, uploaded */
 #define KZ_BUILD_LBVH     1    /* on-GPU Morton LBVH, collapsed to 8-wide               */
+/* On-GPU LBVH whose subtrees never mix meshes: every slot of every node holds triangles of exactly one mesh, or whole meshes only (so no
+ * leaf slot holds two meshes).  The references are sorted by mesh first (meshes ranked by the Morton code of their box centres), then by
+ * Morton code, and not pre-split.  A fresh build traces as fast as KZ_BUILD_LBVH or up to ~10 % slower where meshes overlap, but when meshes move rigidly
+ * (kzgpu_mesh_transform) each mesh's subtrees move with it, so kzgpu_accel_refit keeps their boxes tight and only the few nodes above the
+ * meshes grow.  Build with it when whole meshes move from frame to frame and refit; DESIGN.md section 7 has measurements. */
+#define KZ_BUILD_LBVH_MESHES 2
 
 typedef struct kzgpu_ctx kzgpu_ctx;
 
@@ -267,6 +273,17 @@ int  kzgpu_accel_build(kzgpu_ctx *ctx, int builder);
  * Entry points that need the accel return KZ_ERR_STATE until kzgpu_accel_refit or kzgpu_accel_build has run.
  * The primary-hit hints are kept: any hint yields the same hits, and those of the last frame are the best guess. */
 int  kzgpu_mesh_update(kzgpu_ctx *ctx, int mesh, const float *positions, const float *normals);
+
+/* Sets mesh `mesh`'s positions to matrix * p and, if it has normals, its normals to normalize(inverse^T * n), where p and n are the
+ * mesh's rest pose: the arrays of the upload or of the last kzgpu_mesh_update of this mesh (so transforming twice does not compose).
+ * matrix and inverse are row-major 4x4, as kz_camera_desc's; inverse may be NULL for a mesh without normals.  The arithmetic is the
+ * C++ host's `toWorld` (Transform::point divides by w; normals are normalised as the OBJ loader does), rounded the same way, so a mesh
+ * placed here equals the same OBJ loaded with that transform, bit for bit.  It runs on every device; the rest pose is kept in HBM for
+ * meshes that have been transformed (12 bytes per vertex, 24 with normals) until the next kzgpu_scene_upload.  An emitter's area CDF and
+ * the bounds of the invisible emitters are recomputed.  A NULL matrix, a NULL inverse for a mesh with normals, a non-finite entry or a
+ * mesh index out of range is KZ_ERR_INVALID; an invalid call changes nothing.  As after kzgpu_mesh_update, entry points that need the
+ * accel return KZ_ERR_STATE until kzgpu_accel_refit or kzgpu_accel_build has run. */
+int  kzgpu_mesh_transform(kzgpu_ctx *ctx, int mesh, const float matrix[16], const float inverse[16]);
 
 /* Refits the built accel to the current vertex positions on every device of the context.
  * The tree is the same; the boxes, triangle records and traversal slack are recomputed, so trace and render return

@@ -13,6 +13,7 @@
 #include "kz_owner.h"
 #include <cuda_runtime.h>
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <memory>
@@ -72,6 +73,8 @@ struct Device {
      * uint, a failed level check) and whether this accel's level layout was checked on this device */
     DevMem refit_boxes, refit_flags;
     bool levels_checked = false;
+    /* kzgpu_mesh_transform: per mesh, its rest pose (positions, then normals if it has any, packed xyz) once it has been transformed */
+    std::vector<DevMem> rest;
     /* scratch for host-pointer entry points */
     DevMem scratch[3];
     /* launch geometry */
@@ -217,6 +220,8 @@ int grid_for(size_t n, int threads, int sm_count) {
 int upload_tables(kzgpu_ctx *ctx, Device &d) {
     const KzHostScene &h = *ctx->hs;
     d.tables.clear();
+    d.rest.clear();
+    d.rest.resize(h.meshes.size());
     d.frame_mem.reset();
     d.sc = h.sc;     /* flatten() without geometry leaves the accel fields of h.sc empty, as drop_all() left those of d.sc */
     auto next = [&d]() -> DevMem & { d.tables.emplace_back(); return d.tables.back(); };
@@ -519,6 +524,52 @@ int enqueue_render(const kzgpu_ctx *ctx, kzgpu_ctx *ectx, Device &d, const kz_re
     return KZ_OK;
 }
 
+uint32_t mesh_vertices(const KzHostScene &h, int mesh) {
+    const KzMeshRec &r = h.meshes[(size_t)mesh];
+    return (uint32_t)(((size_t)mesh + 1 < h.meshes.size() ? (uint64_t)h.meshes[(size_t)mesh + 1].vertex_offset : h.total_vertices) - r.vertex_offset);
+}
+
+/* An emitter's area CDF, normalisation and bounds for new vertex positions (kzgpu_mesh_update, kzgpu_mesh_transform): computed on the host
+ * by KzHostScene::emitter_tables from `positions` (a host array) and the mesh's index records (read back from device 0) before anything
+ * of the scene changes, then installed by emitter_apply and copied to every device by emitter_upload. */
+struct EmitterTables {
+    std::vector<float> cdf, bounds;
+    float inv_area = 0.f;
+    size_t light_k = 0;
+};
+int emitter_tables(kzgpu_ctx *ctx, int mesh, const float *positions, EmitterTables &t) {
+    const KzHostScene &h = *ctx->hs;
+    const KzMeshRec &r = h.meshes[(size_t)mesh];
+    Device &d0 = ctx->devs[0];
+    std::vector<KzU4> rec(r.n_triangles);
+    KZ_CUDA(ctx, cudaMemcpyAsync(rec.data(), d0.sc.indices + r.index_offset, (size_t)r.n_triangles * sizeof(KzU4), cudaMemcpyDeviceToHost, d0.stream));
+    KZ_CUDA(ctx, cudaStreamSynchronize(d0.stream));
+    std::vector<uint32_t> idx((size_t)r.n_triangles * 3);
+    for (size_t f = 0; f < rec.size(); ++f) { idx[3 * f] = rec[f].x; idx[3 * f + 1] = rec[f].y; idx[3 * f + 2] = rec[f].z; }
+    t.cdf.resize((size_t)r.n_triangles + 1);
+    t.bounds.resize(6);
+    KzHostScene::emitter_tables(positions, idx.data(), r.n_triangles, t.cdf.data(), t.inv_area, t.bounds.data());
+    t.light_k = 0;
+    while (h.light_meshes[t.light_k] != mesh) ++t.light_k;
+    return KZ_OK;
+}
+void emitter_apply(kzgpu_ctx *ctx, int mesh, const EmitterTables &t) {
+    KzHostScene &h = *ctx->hs;
+    KzMeshRec &r = h.meshes[(size_t)mesh];
+    std::copy(t.cdf.begin(), t.cdf.end(), h.light_cdf.begin() + r.cdf_offset);
+    r.inv_area = t.inv_area;
+    std::copy(t.bounds.begin(), t.bounds.end(), h.light_bounds.begin() + 6 * t.light_k);
+    h.invisible_light_bounds();
+}
+/* enqueues the copies on d.stream (current device); the caller synchronises */
+int emitter_upload(kzgpu_ctx *ctx, Device &d) {
+    const KzHostScene &h = *ctx->hs;
+    KZ_CUDA(ctx, cudaMemcpyAsync(const_cast<KzMeshRec *>(d.sc.meshes), h.meshes.data(), h.meshes.size() * sizeof(KzMeshRec), cudaMemcpyHostToDevice, d.stream));
+    KZ_CUDA(ctx, cudaMemcpyAsync(const_cast<float *>(d.sc.light_cdf), h.light_cdf.data(), h.light_cdf.size() * sizeof(float), cudaMemcpyHostToDevice, d.stream));
+    for (int a = 0; a < 3; ++a) { d.sc.inv_light_lo[a] = h.sc.inv_light_lo[a]; d.sc.inv_light_hi[a] = h.sc.inv_light_hi[a]; }
+    return KZ_OK;
+}
+
 int check_ready(kzgpu_ctx *ctx, bool need_accel) {
     if (!ctx) return fail(nullptr, KZ_ERR_INVALID, "null context");
     if (!ctx->uploaded) return fail(ctx, KZ_ERR_STATE, "no scene uploaded");
@@ -668,7 +719,7 @@ int kzgpu_scene_upload(kzgpu_ctx *ctx, const kz_scene_desc *scene) {
 int kzgpu_accel_build(kzgpu_ctx *ctx, int builder) {
     int rc = check_ready(ctx, false);
     if (rc) return rc;
-    if (builder != KZ_BUILD_HOST_SAH && builder != KZ_BUILD_LBVH) return fail(ctx, KZ_ERR_INVALID, "unknown builder");
+    if (builder != KZ_BUILD_HOST_SAH && builder != KZ_BUILD_LBVH && builder != KZ_BUILD_LBVH_MESHES) return fail(ctx, KZ_ERR_INVALID, "unknown builder");
     const auto t0 = std::chrono::steady_clock::now();
     Device &d0 = ctx->devs[0];
     KZ_CUDA(ctx, cudaSetDevice(d0.id));
@@ -706,7 +757,7 @@ int kzgpu_accel_build(kzgpu_ctx *ctx, int builder) {
         KZ_CUDA(ctx, cudaSetDevice(d0.id));
         kzlbvh::Result r;
         std::string err;
-        rc = kzlbvh::build(d_tris, n_tris, d0.stream, r, err);
+        rc = kzlbvh::build(d_tris, n_tris, d0.stream, r, err, builder == KZ_BUILD_LBVH_MESHES ? (uint32_t)ctx->hs->meshes.size() : 0u);
         tris_mem.reset();
         /* hand the pool's memory back: the path pools and the caller's own allocations need it, the next build allocates afresh */
         { cudaMemPool_t pool; if (cudaDeviceGetDefaultMemPool(&pool, d0.id) == cudaSuccess) { cudaStreamSynchronize(d0.stream); cudaMemPoolTrimTo(pool, 0); } }
@@ -739,14 +790,12 @@ int kzgpu_mesh_update(kzgpu_ctx *ctx, int mesh, const float *positions, const fl
     if (!positions) return fail(ctx, KZ_ERR_INVALID, "null positions");
     KzMeshRec &r = h.meshes[(size_t)mesh];
     if (normals && !(r.flags & KZ_MESH_HAS_NORMALS)) return fail(ctx, KZ_ERR_INVALID, "normals given for a mesh uploaded without normals");
-    const uint32_t nv = (uint32_t)(((size_t)mesh + 1 < h.meshes.size() ? (uint64_t)h.meshes[(size_t)mesh + 1].vertex_offset : h.total_vertices) - r.vertex_offset);
+    const uint32_t nv = mesh_vertices(h, mesh);
     Device &d0 = ctx->devs[0];
     KZ_CUDA(ctx, cudaSetDevice(d0.id));
-    /* an emitter's area CDF, normalisation and bounds are recomputed on the host from its new positions (read back if they are a
-     * device array, as kzgpu_scene_upload does) and its index records (read back from HBM); nothing is written before this succeeded */
-    std::vector<float> cdf, bounds(6);
-    float inv_area = 0.f;
-    size_t light_k = 0;
+    /* an emitter's tables come from its new positions (read back if they are a device array, as kzgpu_scene_upload does); nothing is
+     * written before this succeeded */
+    EmitterTables et;
     if (r.flags & KZ_MESH_IS_LIGHT) {
         std::vector<float> pos;
         const float *hp = positions;
@@ -755,14 +804,8 @@ int kzgpu_mesh_update(kzgpu_ctx *ctx, int mesh, const float *positions, const fl
             KZ_CUDA(ctx, cudaMemcpy(pos.data(), positions, (size_t)nv * 12, cudaMemcpyDeviceToHost));
             hp = pos.data();
         }
-        std::vector<KzU4> rec(r.n_triangles);
-        KZ_CUDA(ctx, cudaMemcpyAsync(rec.data(), d0.sc.indices + r.index_offset, (size_t)r.n_triangles * sizeof(KzU4), cudaMemcpyDeviceToHost, d0.stream));
-        KZ_CUDA(ctx, cudaStreamSynchronize(d0.stream));
-        std::vector<uint32_t> idx((size_t)r.n_triangles * 3);
-        for (size_t f = 0; f < rec.size(); ++f) { idx[3 * f] = rec[f].x; idx[3 * f + 1] = rec[f].y; idx[3 * f + 2] = rec[f].z; }
-        cdf.resize((size_t)r.n_triangles + 1);
-        KzHostScene::emitter_tables(hp, idx.data(), r.n_triangles, cdf.data(), inv_area, bounds.data());
-        while (h.light_meshes[light_k] != mesh) ++light_k;
+        int rc = emitter_tables(ctx, mesh, hp, et);
+        if (rc) return rc;
     }
     /* from here on the scene changes: the accel no longer matches it until a refit or a build */
     ctx->built = false;
@@ -787,21 +830,89 @@ int kzgpu_mesh_update(kzgpu_ctx *ctx, int mesh, const float *positions, const fl
         if (e == cudaSuccess) e = cudaStreamSynchronize(d0.stream);
         if (e != cudaSuccess) return fail(ctx, KZ_ERR_CUDA, std::string("mesh update: ") + cudaGetErrorString(e));
     }
-    if (r.flags & KZ_MESH_IS_LIGHT) {
-        std::copy(cdf.begin(), cdf.end(), h.light_cdf.begin() + r.cdf_offset);
-        r.inv_area = inv_area;
-        std::copy(bounds.begin(), bounds.end(), h.light_bounds.begin() + 6 * light_k);
-        h.invisible_light_bounds();
-    }
+    if (r.flags & KZ_MESH_IS_LIGHT) emitter_apply(ctx, mesh, et);
     for (Device &d : ctx->devs) {
         KZ_CUDA(ctx, cudaSetDevice(d.id));
         if (&d != &d0 && nv)
             KZ_CUDA(ctx, cudaMemcpyPeerAsync(const_cast<KzVertex *>(d.sc.vertices) + r.vertex_offset, d.id, d0.sc.vertices + r.vertex_offset, d0.id, (size_t)nv * sizeof(KzVertex), d.stream));
-        if (r.flags & KZ_MESH_IS_LIGHT) {
-            KZ_CUDA(ctx, cudaMemcpyAsync(const_cast<KzMeshRec *>(d.sc.meshes), h.meshes.data(), h.meshes.size() * sizeof(KzMeshRec), cudaMemcpyHostToDevice, d.stream));
-            KZ_CUDA(ctx, cudaMemcpyAsync(const_cast<float *>(d.sc.light_cdf), h.light_cdf.data(), h.light_cdf.size() * sizeof(float), cudaMemcpyHostToDevice, d.stream));
-            for (int a = 0; a < 3; ++a) { d.sc.inv_light_lo[a] = h.sc.inv_light_lo[a]; d.sc.inv_light_hi[a] = h.sc.inv_light_hi[a]; }
+        /* a transformed mesh's rest pose becomes the new arrays: a later kzgpu_mesh_transform places these */
+        if (DevMem &rest = d.rest[(size_t)mesh]; rest.p && nv) {
+            k_copy_rest<<<grid_for(nv, 256, d.sm_count), 256, 0, d.stream>>>(d.sc.vertices + r.vertex_offset, nv, rest.as<float>(), normals ? rest.as<float>() + 3 * (size_t)nv : nullptr);
+            ++d.launches;
+            KZ_CUDA(ctx, cudaGetLastError());
         }
+        if (r.flags & KZ_MESH_IS_LIGHT) { int rc = emitter_upload(ctx, d); if (rc) return rc; }
+        KZ_CUDA(ctx, cudaStreamSynchronize(d.stream));
+    }
+    KZ_CUDA(ctx, cudaSetDevice(d0.id));
+    return KZ_OK;
+}
+
+int kzgpu_mesh_transform(kzgpu_ctx *ctx, int mesh, const float matrix[16], const float inverse[16]) {
+    if (!ctx) return fail(nullptr, KZ_ERR_INVALID, "null context");
+    if (!ctx->uploaded) return fail(ctx, KZ_ERR_STATE, "no scene uploaded");
+    KzHostScene &h = *ctx->hs;
+    if (mesh < 0 || mesh >= (int)h.meshes.size()) return fail(ctx, KZ_ERR_INVALID, "mesh index out of range");
+    if (!matrix) return fail(ctx, KZ_ERR_INVALID, "null matrix");
+    const KzMeshRec &r = h.meshes[(size_t)mesh];
+    const bool has_normals = (r.flags & KZ_MESH_HAS_NORMALS) != 0;
+    if (has_normals && !inverse) return fail(ctx, KZ_ERR_INVALID, "null inverse for a mesh with normals");
+    KzXform x;
+    for (int i = 0; i < 16; ++i) {
+        x.m[i] = matrix[i];
+        x.inv[i] = inverse ? inverse[i] : 0.f;
+        if (!std::isfinite(x.m[i]) || !std::isfinite(x.inv[i])) return fail(ctx, KZ_ERR_INVALID, "non-finite matrix entry");
+    }
+    const uint32_t nv = mesh_vertices(h, mesh);
+    const size_t rest_floats = (size_t)nv * (has_normals ? 6 : 3);
+    Device &d0 = ctx->devs[0];
+    /* an emitter's tables come from its placed positions, computed on the host by the kernel's own per-vertex body from the rest pose of
+     * device 0 (its vertex records if it has not been transformed before) */
+    EmitterTables et;
+    if (r.flags & KZ_MESH_IS_LIGHT) {
+        KZ_CUDA(ctx, cudaSetDevice(d0.id));
+        std::vector<float> rest((size_t)nv * 3), pos((size_t)nv * 3);
+        if (d0.rest[(size_t)mesh].p) {
+            KZ_CUDA(ctx, cudaMemcpy(rest.data(), d0.rest[(size_t)mesh].p, (size_t)nv * 12, cudaMemcpyDeviceToHost));
+        } else {
+            std::vector<KzVertex> v(nv);
+            KZ_CUDA(ctx, cudaMemcpy(v.data(), d0.sc.vertices + r.vertex_offset, (size_t)nv * sizeof(KzVertex), cudaMemcpyDeviceToHost));
+            for (size_t i = 0; i < nv; ++i) { rest[3 * i] = v[i].px; rest[3 * i + 1] = v[i].py; rest[3 * i + 2] = v[i].pz; }
+        }
+        for (size_t i = 0; i < nv; ++i) kz_transform_point(x.m, rest.data() + 3 * i, pos.data() + 3 * i);
+        int rc = emitter_tables(ctx, mesh, pos.data(), et);
+        if (rc) return rc;
+    }
+    /* the first transform of a mesh copies its rest pose out of the vertex records, on every device (allocated before anything is
+     * written: a failure leaves copies of the current pose behind, which is what a rest pose is until the first transform) */
+    for (Device &d : ctx->devs) {
+        DevMem &rest = d.rest[(size_t)mesh];
+        if (rest.p) continue;
+        KZ_CUDA(ctx, cudaSetDevice(d.id));
+        KZ_CUDA(ctx, rest.alloc(rest_floats * sizeof(float)));
+        if (nv) {
+            k_copy_rest<<<grid_for(nv, 256, d.sm_count), 256, 0, d.stream>>>(d.sc.vertices + r.vertex_offset, nv, rest.as<float>(), has_normals ? rest.as<float>() + 3 * (size_t)nv : nullptr);
+            ++d.launches;
+            KZ_CUDA(ctx, cudaGetLastError());
+        }
+    }
+    /* from here on the scene changes: the accel no longer matches it until a refit or a build */
+    ctx->built = false;
+    if (r.flags & KZ_MESH_IS_LIGHT) emitter_apply(ctx, mesh, et);
+    /* every device places its own rest copy: the arithmetic is per vertex and exact, so all of them end up with the same bytes */
+    for (Device &d : ctx->devs) {
+        KZ_CUDA(ctx, cudaSetDevice(d.id));
+        if (nv) {
+            const float *rest = d.rest[(size_t)mesh].as<float>();
+            k_transform_vertices<<<grid_for(nv, 256, d.sm_count), 256, 0, d.stream>>>(rest, has_normals ? rest + 3 * (size_t)nv : nullptr, nv, x,
+                                                                                     const_cast<KzVertex *>(d.sc.vertices) + r.vertex_offset);
+            ++d.launches;
+            KZ_CUDA(ctx, cudaGetLastError());
+        }
+        if (r.flags & KZ_MESH_IS_LIGHT) { int rc = emitter_upload(ctx, d); if (rc) return rc; }
+    }
+    for (Device &d : ctx->devs) {
+        KZ_CUDA(ctx, cudaSetDevice(d.id));
         KZ_CUDA(ctx, cudaStreamSynchronize(d.stream));
     }
     KZ_CUDA(ctx, cudaSetDevice(d0.id));

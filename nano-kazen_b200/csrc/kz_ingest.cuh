@@ -2,6 +2,8 @@
  *
  *   k_ingest_vertices   Mesh::m_V / m_N / m_UV (mesh.h:175-178: packed xyz / uv arrays) -> 32-byte KzVertex records
  *   k_update_vertices   kzgpu_mesh_update: new positions (and normals) into existing KzVertex records, the other fields kept
+ *   k_transform_vertices kzgpu_mesh_transform: a mesh's rest pose placed by a matrix (kz_transform.h) into its KzVertex records, u / v kept
+ *   k_copy_rest         positions (and normals) of KzVertex records -> a mesh's rest pose (packed xyz arrays)
  *   k_ingest_indices    Mesh::m_F -> 16-byte index records, validated against the vertex count
  *   k_ingest_texels     decoded rgb image -> float4 texels (level 0)
  *   k_gather_tris       (mesh table, vertex records, index records) -> the accel builders' triangle list in scene
@@ -16,6 +18,7 @@
 #define KZ_INGEST_CUH
 #include "kz_scene.h"
 #include "kz_bvh_build.h"
+#include "kz_transform.h"
 
 __global__ void k_ingest_vertices(const float *pos, const float *nrm, const float *uv, uint32_t n, KzVertex *out) {
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
@@ -35,6 +38,29 @@ __global__ void k_update_vertices(const float *pos, const float *nrm, uint32_t n
         const float4 a = o[0];
         o[0] = make_float4(pos[3 * (size_t)i], pos[3 * (size_t)i + 1], pos[3 * (size_t)i + 2], a.w);
         if (nrm) { const float4 b = o[1]; o[1] = make_float4(nrm[3 * (size_t)i], nrm[3 * (size_t)i + 1], nrm[3 * (size_t)i + 2], b.w); }
+    }
+}
+
+/* rest_nrm == nullptr: the records' normals are kept (a mesh without normals) */
+__global__ void k_transform_vertices(const float *rest_pos, const float *rest_nrm, uint32_t n, KzXform x, KzVertex *out) {
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        float4 *o = reinterpret_cast<float4 *>(out + i);
+        float r[3];
+        kz_transform_point(x.m, rest_pos + 3 * (size_t)i, r);
+        o[0] = make_float4(r[0], r[1], r[2], o[0].w);
+        if (rest_nrm) {
+            kz_transform_normal(x.inv, rest_nrm + 3 * (size_t)i, r);
+            o[1] = make_float4(r[0], r[1], r[2], o[1].w);
+        }
+    }
+}
+
+/* nrm == nullptr: positions only */
+__global__ void k_copy_rest(const KzVertex *v, uint32_t n, float *pos, float *nrm) {
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const KzVertex r = v[i];
+        pos[3 * (size_t)i] = r.px; pos[3 * (size_t)i + 1] = r.py; pos[3 * (size_t)i + 2] = r.pz;
+        if (nrm) { nrm[3 * (size_t)i] = r.nx; nrm[3 * (size_t)i + 1] = r.ny; nrm[3 * (size_t)i + 2] = r.nz; }
     }
 }
 

@@ -3,12 +3,19 @@
  *   k_scene_bounds   centroid bounds + max |coordinate|           (block reduce + ordered-int atomics)
  *   k_morton         63-bit Morton key of every triangle centroid
  *   cub radix sort   (key, triangle) pairs  -- library utility, the only non-hand-written step
+ *   k_mesh_bounds    (KZ_BUILD_LBVH_MESHES) centroid bounds of every mesh; the meshes are ranked by the Morton code of their box
+ *   k_rank_keys      centres, and a second, stable cub sort by that rank puts every mesh's references in one run, in Morton order
+ *   k_permute        inside it; kz_delta then compares (rank, Morton code), so every mesh, and every run of neighbouring meshes, is
+ *                    a subtree of the radix tree
  *   k_karras         binary radix tree over the sorted keys (Karras 2012), one thread per internal node
  *   k_fit            bottom-up AABB fit, second-arriver-continues
  *   k_collapse       level-synchronous collapse into the 80-byte 8-wide compressed nodes of
  *                    kz_scene.h: subtrees of <= 3 triangles become leaf slots, the child with the
  *                    largest area is opened until 8 slots are used, slots are octant-ordered,
  *                    child boxes are quantised outwards in double precision (conservative).
+ *
+ * With KZ_BUILD_LBVH_MESHES no subtree mixes meshes unless it holds them whole, so a rigid motion of a mesh moves its subtrees with it and
+ * a refit keeps them tight (DESIGN.md section 3, "Rigid motion").
  *
  * Tree quality does not affect results: culling is conservative and ties on t are broken by
  * (geomID, primID) in the traversal, so the host-SAH and the LBVH accel return identical hits.
@@ -20,7 +27,9 @@
 #include "kz_owner.h"
 #include <cub/device/device_radix_sort.cuh>
 #include <cuda_runtime.h>
+#include <algorithm>
 #include <string>
+#include <utility>
 #include <vector>
 
 namespace kzlbvh {
@@ -42,6 +51,7 @@ struct BuildState {
     uint32_t n;                  /* references */
     const uint32_t *order;       /* sorted position -> triangle */
     const unsigned long long *keys;
+    const uint32_t *rank;        /* KZ_BUILD_LBVH_MESHES: rank of the mesh of each sorted reference, the key's leading part (else nullptr) */
     int32_t *left, *right;       /* >= 0 internal node, < 0: ~leaf (sorted position) */
     int32_t *parent;             /* [0, n-1): internal nodes, [n-1, 2n-1): leaves */
     uint32_t *first, *last;      /* sorted range covered by an internal node */
@@ -84,7 +94,7 @@ __global__ void k_scene_bounds(const kzbvh::Tri *tris, uint32_t n, uint32_t *bou
     }
 }
 
-__device__ __forceinline__ unsigned long long expand21(unsigned long long v) {
+__host__ __device__ __forceinline__ unsigned long long expand21(unsigned long long v) {
     v &= 0x1FFFFFull;
     v = (v | (v << 32)) & 0x1F00000000FFFFull;
     v = (v | (v << 16)) & 0x1F0000FF0000FFull;
@@ -120,11 +130,19 @@ __global__ void k_morton(const kzbvh::Tri *tris, const float4 *rlo, const float4
     keys[i] = code; vals[i] = i;
 }
 
-__device__ __forceinline__ int kz_delta(const unsigned long long *keys, int n, int i, int j) {
+/* common prefix length of the keys of sorted references i and j (ties broken by position); with ranks the key is (rank, Morton code):
+ * two ranks that differ share fewer than 32 bits, two equal ones 32 plus the Morton prefix */
+__device__ __forceinline__ int kz_delta(const unsigned long long *keys, const uint32_t *rank, int n, int i, int j) {
     if (j < 0 || j >= n) return -1;
+    int off = 0;
+    if (rank) {
+        const uint32_t ra = rank[i], rb = rank[j];
+        if (ra != rb) return __clz(ra ^ rb);
+        off = 32;
+    }
     const unsigned long long a = keys[i], b = keys[j];
-    if (a == b) return 64 + __clz(i ^ j);
-    return __clzll((long long)(a ^ b));
+    if (a == b) return off + 64 + __clz(i ^ j);
+    return off + __clzll((long long)(a ^ b));
 }
 
 __global__ void k_karras(BuildState b) {
@@ -132,19 +150,20 @@ __global__ void k_karras(BuildState b) {
     const int i = (int)(blockIdx.x * blockDim.x + threadIdx.x);
     if (i >= n - 1) return;
     const unsigned long long *keys = b.keys;
-    const int d = (kz_delta(keys, n, i, i + 1) - kz_delta(keys, n, i, i - 1)) >= 0 ? 1 : -1;
-    const int dmin = kz_delta(keys, n, i, i - d);
+    const uint32_t *rank = b.rank;
+    const int d = (kz_delta(keys, rank, n, i, i + 1) - kz_delta(keys, rank, n, i, i - 1)) >= 0 ? 1 : -1;
+    const int dmin = kz_delta(keys, rank, n, i, i - d);
     int lmax = 2;
-    while (kz_delta(keys, n, i, i + lmax * d) > dmin) lmax <<= 1;
+    while (kz_delta(keys, rank, n, i, i + lmax * d) > dmin) lmax <<= 1;
     int l = 0;
     for (int t = lmax >> 1; t >= 1; t >>= 1)
-        if (kz_delta(keys, n, i, i + (l + t) * d) > dmin) l += t;
+        if (kz_delta(keys, rank, n, i, i + (l + t) * d) > dmin) l += t;
     const int j = i + l * d;
-    const int dnode = kz_delta(keys, n, i, j);
+    const int dnode = kz_delta(keys, rank, n, i, j);
     int s = 0;
     for (int div = 2;; div <<= 1) {
         const int t = (l + div - 1) / div;
-        if (kz_delta(keys, n, i, i + (s + t) * d) > dnode) s += t;
+        if (kz_delta(keys, rank, n, i, i + (s + t) * d) > dnode) s += t;
         if (t <= 1) break;
     }
     const int gamma = i + s * d + (d < 0 ? -1 : 0);
@@ -216,6 +235,10 @@ struct CollapseState {
 };
 
 __device__ __forceinline__ uint32_t sub_count(const BuildState &b, int c) { return c < 0 ? 1u : b.last[c] - b.first[c] + 1u; }
+/* whether radix-tree node c becomes a leaf slot: a single reference, or a subtree of at most KZ_LBVH_MAXLEAF references of one mesh */
+__device__ __forceinline__ bool is_leaf(const BuildState &b, int c) {
+    return c < 0 || (sub_count(b, c) <= KZ_LBVH_MAXLEAF && (!b.rank || b.rank[b.first[c]] == b.rank[b.last[c]]));
+}
 __device__ __forceinline__ float box_area(const Box6 &x) {
     const float dx = x.hi[0] - x.lo[0], dy = x.hi[1] - x.lo[1], dz = x.hi[2] - x.lo[2];
     return 2.f * (dx * dy + dy * dz + dz * dx);
@@ -230,7 +253,7 @@ __global__ void __launch_bounds__(64) k_collapse(CollapseState cs) {
     const WorkItem it = cs.in[wi];
     int ch[8]; Box6 bx[8]; int nch = 0;
     const int root = it.bnode;
-    if (root < 0 || sub_count(b, root) <= KZ_LBVH_MAXLEAF) { ch[0] = root; bx[0] = child_box(b, root); nch = 1; }
+    if (is_leaf(b, root)) { ch[0] = root; bx[0] = child_box(b, root); nch = 1; }
     else {
         ch[0] = b.left[root]; ch[1] = b.right[root];
         bx[0] = child_box(b, ch[0]); bx[1] = child_box(b, ch[1]); nch = 2;
@@ -238,7 +261,7 @@ __global__ void __launch_bounds__(64) k_collapse(CollapseState cs) {
     while (nch < 8) {
         int best = -1; float bestA = -1.f;
         for (int i = 0; i < nch; ++i) {
-            if (ch[i] < 0 || sub_count(b, ch[i]) <= KZ_LBVH_MAXLEAF) continue;
+            if (is_leaf(b, ch[i])) continue;
             const float a = box_area(bx[i]);
             if (a > bestA) { bestA = a; best = i; }
         }
@@ -287,8 +310,7 @@ __global__ void __launch_bounds__(64) k_collapse(CollapseState cs) {
     for (int s = 0; s < 8; ++s) {
         if (childAt[s] < 0) continue;
         const int c = ch[childAt[s]];
-        const uint32_t cnt = sub_count(b, c);
-        if (c >= 0 && cnt > KZ_LBVH_MAXLEAF) ++n_internal; else n_tris += cnt;
+        if (!is_leaf(b, c)) ++n_internal; else n_tris += sub_count(b, c);
     }
     const uint32_t child_base = n_internal ? atomicAdd(cs.node_counter, n_internal) : 0u;
     const uint32_t tri_base = n_tris ? atomicAdd(cs.tri_counter, n_tris) : 0u;
@@ -313,7 +335,7 @@ __global__ void __launch_bounds__(64) k_collapse(CollapseState cs) {
             qhi[a][s] = (uint8_t)fmin(255.0, fmax(0.0, hi));
         }
         const uint32_t cnt = sub_count(b, c);
-        if (c >= 0 && cnt > KZ_LBVH_MAXLEAF) {
+        if (!is_leaf(b, c)) {
             imask |= (uint8_t)(1u << s);
             WorkItem w; w.bnode = c; w.wnode = child_base + rel;
             cs.out[out_base + rel] = w;
@@ -336,6 +358,76 @@ __global__ void __launch_bounds__(64) k_collapse(CollapseState cs) {
     nd.imask = imask;
     cs.nodes[it.wnode] = nd;
     }
+}
+
+/* mb[6 g .. 6 g + 5] = min / max centroid of mesh g's triangles (ordered uints).  The triangles are in scene order, so a warp almost always
+ * sees one mesh: it reduces and lets one lane do the atomics; a warp that straddles meshes does them lane by lane. */
+__global__ void k_mesh_bounds(const kzbvh::Tri *tris, uint32_t n, uint32_t *mb) {
+    for (uint32_t base = blockIdx.x * blockDim.x; base < n; base += gridDim.x * blockDim.x) {
+        const uint32_t i = base + threadIdx.x;
+        const bool ok = i < n;
+        const unsigned valid = __ballot_sync(0xFFFFFFFFu, ok);
+        if (!valid) continue;
+        uint32_t g = 0xFFFFFFFFu;
+        float lo[3] = {3.4e38f, 3.4e38f, 3.4e38f}, hi[3] = {-3.4e38f, -3.4e38f, -3.4e38f};
+        if (ok) {
+            const kzbvh::Tri t = tris[i];
+            g = t.geom;
+            for (int a = 0; a < 3; ++a) {
+                const float c = 0.5f * (fminf(t.p[0][a], fminf(t.p[1][a], t.p[2][a])) + fmaxf(t.p[0][a], fmaxf(t.p[1][a], t.p[2][a])));
+                lo[a] = c; hi[a] = c;
+            }
+        }
+        const uint32_t g0 = __shfl_sync(0xFFFFFFFFu, g, __ffs(valid) - 1);
+        if (__all_sync(0xFFFFFFFFu, !ok || g == g0)) {
+            for (int o = 16; o > 0; o >>= 1)
+                for (int a = 0; a < 3; ++a) {
+                    lo[a] = fminf(lo[a], __shfl_down_sync(0xFFFFFFFFu, lo[a], o));
+                    hi[a] = fmaxf(hi[a], __shfl_down_sync(0xFFFFFFFFu, hi[a], o));
+                }
+            if ((threadIdx.x & 31) != 0) continue;
+            g = g0;
+        } else if (!ok) continue;
+        for (int a = 0; a < 3; ++a) { atomicMin(mb + 6 * (size_t)g + a, f2ord(lo[a])); atomicMax(mb + 6 * (size_t)g + 3 + a, f2ord(hi[a])); }
+    }
+}
+
+/* rk[j] = rank of the mesh of sorted reference j, idx[j] = j */
+__global__ void k_rank_keys(const kzbvh::Tri *tris, const uint32_t *order, const uint32_t *mesh_rank, uint32_t n, uint32_t *rk, uint32_t *idx) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    rk[j] = mesh_rank[tris[order[j]].geom];
+    idx[j] = j;
+}
+
+/* the Morton-sorted keys and triangles in the order of the rank sort */
+__global__ void k_permute(const uint32_t *perm, const unsigned long long *keys, const uint32_t *order, uint32_t n, unsigned long long *keys_out, uint32_t *order_out) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const uint32_t p = perm[j];
+    keys_out[j] = keys[p]; order_out[j] = order[p];
+}
+
+/* Ranks of the meshes (host side, once per build): the meshes ordered by the Morton code of their centroid boxes' centres in the scene's
+ * centroid bounds (the frame of k_morton), ties and empty meshes by index.  `mb` as k_mesh_bounds leaves it, `bounds` as k_scene_bounds. */
+inline std::vector<uint32_t> mesh_ranks(const std::vector<uint32_t> &mb, const uint32_t *bounds) {
+    const size_t nm = mb.size() / 6;
+    std::vector<std::pair<unsigned long long, uint32_t>> code(nm);
+    for (size_t g = 0; g < nm; ++g) {
+        unsigned long long c = 0ull;
+        if (ord2f(mb[6 * g]) <= ord2f(mb[6 * g + 3]))
+            for (int a = 0; a < 3; ++a) {
+                const float lo = ord2f(bounds[a]), ext = ord2f(bounds[3 + a]) - lo;
+                const float centre = 0.5f * (ord2f(mb[6 * g + a]) + ord2f(mb[6 * g + 3 + a]));
+                const float u = ext > 0.f ? std::min(std::max((centre - lo) / ext, 0.f), 1.f) : 0.f;
+                c |= expand21(std::min<unsigned long long>((unsigned long long)(u * 2097152.0f), 2097151ull)) << (2 - a);
+            }
+        code[g] = {c, (uint32_t)g};
+    }
+    std::sort(code.begin(), code.end());
+    std::vector<uint32_t> rank(nm);
+    for (size_t k = 0; k < nm; ++k) rank[code[k].second] = (uint32_t)k;
+    return rank;
 }
 
 /* Reference pre-splitting (as in the host SAH builder, kz_bvh_build.h): a triangle whose box is expected to hold other primitives,
@@ -410,8 +502,9 @@ __global__ void k_make_refs(const kzbvh::Tri *tris, uint32_t n, const uint32_t *
 #define KZ_LBVH_MAX_LEVELS 31     /* levels the collapse walks; the API accepts KZ_MAX_ACCEL_DEPTH = 30 of them (stack budget in kz_traverse.h) */
 
 /* Builds the accel of the `n_tris_in` device-resident triangles `d_tris` (scene order) on the current device; `r` owns the node and
- * triangle arrays (also after a failure), temporaries are released before returning. */
-inline int build(const kzbvh::Tri *d_tris, uint32_t n_tris_in, cudaStream_t s, Result &r, std::string &err) {
+ * triangle arrays (also after a failure), temporaries are released before returning.  n_meshes > 0: KZ_BUILD_LBVH_MESHES over that many
+ * meshes (geomIDs below it), without pre-splitting -- every slot's subtree holds one mesh or whole meshes; 0: KZ_BUILD_LBVH. */
+inline int build(const kzbvh::Tri *d_tris, uint32_t n_tris_in, cudaStream_t s, Result &r, std::string &err, uint32_t n_meshes = 0) {
     std::vector<void *> temp;
     uint32_t n = n_tris_in;                  /* references: == triangles unless pre-splitting adds some */
     r = Result();
@@ -428,7 +521,7 @@ inline int build(const kzbvh::Tri *d_tris, uint32_t n_tris_in, cudaStream_t s, R
     float4 *rlo = nullptr, *rhi = nullptr;
     {
         const char *e = getenv("KZ_LBVH_PRESPLIT");
-        const bool presplit = e ? atoi(e) != 0 : KZ_LBVH_PRESPLIT_DEFAULT != 0;
+        const bool presplit = n_meshes == 0 && (e ? atoi(e) != 0 : KZ_LBVH_PRESPLIT_DEFAULT != 0);
         if (presplit && n_tris_in >= 64u && n_tris_in < 0x3FFFFFFFu) {
             const char *ne = getenv("KZ_SAH_PRESPLIT_NEED");
             const float need = ne ? (float)atof(ne) : 0.25f;
@@ -460,7 +553,36 @@ inline int build(const kzbvh::Tri *d_tris, uint32_t n_tris_in, cudaStream_t s, R
     r.launches += 8;
 
     BuildState b;
-    b.tris = d_tris; b.rlo = rlo; b.rhi = rhi; b.n = n; b.order = dv.Current(); b.keys = dk.Current();
+    b.tris = d_tris; b.rlo = rlo; b.rhi = rhi; b.n = n; b.order = dv.Current(); b.keys = dk.Current(); b.rank = nullptr;
+    if (n_meshes > 0) {
+        /* mesh ranks, then a stable sort of the Morton-ordered references by the rank of their mesh */
+        uint32_t *mb, *mrank, *r0, *r1, *p0, *p1;
+        KZL_CUDA(talloc((size_t)n_meshes * 24, (void **)&mb)); KZL_CUDA(talloc((size_t)n_meshes * 4, (void **)&mrank));
+        std::vector<uint32_t> hmb((size_t)n_meshes * 6);
+        for (size_t g = 0; g < n_meshes; ++g) for (int a = 0; a < 3; ++a) { hmb[6 * g + a] = 0xFFFFFFFFu; hmb[6 * g + 3 + a] = 0u; }
+        KZL_CUDA(cudaMemcpyAsync(mb, hmb.data(), hmb.size() * 4, cudaMemcpyHostToDevice, s));
+        k_mesh_bounds<<<std::min((n + 255u) / 256u, 148u * 8u), 256, 0, s>>>(d_tris, n, mb);
+        uint32_t hb[6];
+        KZL_CUDA(cudaMemcpyAsync(hmb.data(), mb, hmb.size() * 4, cudaMemcpyDeviceToHost, s));
+        KZL_CUDA(cudaMemcpyAsync(hb, bounds, sizeof(hb), cudaMemcpyDeviceToHost, s));
+        KZL_CUDA(cudaStreamSynchronize(s));
+        const std::vector<uint32_t> rank = mesh_ranks(hmb, hb);
+        KZL_CUDA(cudaMemcpyAsync(mrank, rank.data(), rank.size() * 4, cudaMemcpyHostToDevice, s));
+        KZL_CUDA(talloc((size_t)n * 4, (void **)&r0)); KZL_CUDA(talloc((size_t)n * 4, (void **)&r1));
+        KZL_CUDA(talloc((size_t)n * 4, (void **)&p0)); KZL_CUDA(talloc((size_t)n * 4, (void **)&p1));
+        k_rank_keys<<<blocks, 256, 0, s>>>(d_tris, dv.Current(), mrank, n, r0, p0);
+        int bits = 1;
+        while (bits < 32 && (n_meshes - 1u) >> bits) ++bits;
+        cub::DoubleBuffer<uint32_t> dr(r0, r1), dp(p0, p1);
+        size_t rank_bytes = 0;
+        KZL_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, rank_bytes, dr, dp, (int)n, 0, bits, s));
+        void *rank_tmp;
+        KZL_CUDA(talloc(rank_bytes, &rank_tmp));
+        KZL_CUDA(cub::DeviceRadixSort::SortPairs(rank_tmp, rank_bytes, dr, dp, (int)n, 0, bits, s));
+        k_permute<<<blocks, 256, 0, s>>>(dp.Current(), dk.Current(), dv.Current(), n, dk.Alternate(), dv.Alternate());
+        r.launches += 11;
+        b.order = dv.Alternate(); b.keys = dk.Alternate(); b.rank = dr.Current();
+    }
     const size_t ni = n > 1 ? n - 1 : 1;
     KZL_CUDA(talloc(ni * 4, (void **)&b.left)); KZL_CUDA(talloc(ni * 4, (void **)&b.right));
     KZL_CUDA(talloc((size_t)(2 * (size_t)n) * 4, (void **)&b.parent));

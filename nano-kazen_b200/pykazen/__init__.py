@@ -23,7 +23,7 @@ CONDUCTORS = {"Au": ((0.1431189557, 0.3749570432, 1.4424785571), (3.9831604247, 
               "Cr": ((4.3696828663, 2.9167024892, 1.6547005413), (5.2064337956, 4.2313645277, 3.7549467933))}
 CAM_PERSPECTIVE, CAM_THINLENS = range(2)
 SAMPLER_INDEPENDENT, SAMPLER_STRATIFIED, SAMPLER_CORRELATED, SAMPLER_PMJ02BN = range(4)
-BUILD_HOST_SAH, BUILD_LBVH = 0, 1
+BUILD_HOST_SAH, BUILD_LBVH, BUILD_LBVH_MESHES = 0, 1, 2
 
 RAY_DTYPE = np.dtype([("o", "<f4", 3), ("tmin", "<f4"), ("d", "<f4", 3), ("tmax", "<f4")])
 HIT_DTYPE = np.dtype([("t", "<f4"), ("u", "<f4"), ("v", "<f4"), ("prim_id", "<u4"), ("geom_id", "<u4")])
@@ -577,6 +577,17 @@ class Gpu(_Backend):
             return a.ctypes.data_as(C.c_void_p)
         keep = []
         self._call("mesh_update", self.h, C.c_int(mesh), ptr(positions), ptr(normals))
+
+    def mesh_transform(self, mesh, matrix, inverse=None):
+        """places mesh `mesh`'s rest pose (its uploaded or last mesh_update arrays) by the 4x4 `matrix` (row-major array-like, as the
+        C++ host's toWorld); normals go through `inverse`'s transpose.  inverse=None on a mesh with normals: np.linalg.inv of the matrix
+        in float64, rounded to float32 (kazen's Transform inverts in double and rounds once too).  Trace and render need refit() (or a
+        rebuild) afterwards."""
+        M = np.ascontiguousarray(matrix, np.float32).reshape(4, 4)
+        if inverse is None and 0 <= mesh < self._desc.n_meshes and self._desc.meshes[mesh].normals:
+            inverse = np.linalg.inv(M.astype(np.float64))
+        inv = None if inverse is None else np.ascontiguousarray(inverse, np.float32).reshape(4, 4)
+        self._call("mesh_transform", self.h, C.c_int(mesh), M.ctypes.data_as(c_float_p), None if inv is None else inv.ctypes.data_as(c_float_p))
 
     def refit(self):
         """refits the accel to the current vertex positions on every device (same tree, new boxes)"""
