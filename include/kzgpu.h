@@ -193,6 +193,13 @@ typedef struct kz_integrator_desc {
     int32_t regularization;
     float   accumulated_roughness;
     int32_t type;                  /* kz_integrator_type */
+    /* path_mis only ("envSampling", default 0 = the reference estimator): 1 also samples the background as a light.  Next-event
+     * estimation then picks the environment with probability 1 / (emitters + 1) and draws a direction from a luminance table of the
+     * background (built on the GPU at kzgpu_scene_upload), and a BSDF-sampled ray that escapes is weighted by the power heuristic
+     * against that density.  The estimate is unbiased either way; with an HDR sky whose light comes from a small bright region (a sun,
+     * a window) it converges much faster.  Nothing changes when the background is absent or black in every direction (no
+     * background, zero intensity, colorramp / blend chains, an all-black image), nor for the other integrators. */
+    int32_t env_sampling;
 } kz_integrator_desc;
 
 /* Reconstruction filter tabulated as ImageBlock does (block.cpp:13-21). */
@@ -358,6 +365,11 @@ int  kzgpu_intersection_dump(kzgpu_ctx *ctx, const kz_ray *rays, size_t n, float
  * barycentric 1, barycentric 2, unused) in the order Li draws them.  16 floats per query: mesh, p[3], n[3], wi[3], dist, pdf (solid
  * angle, without the light-pick probability), Le/pdf [3], 0. */
 int  kzgpu_light_sample_dump(kzgpu_ctx *ctx, const float *ref3, const float *u5, size_t n, float *out16);
+
+/* Environment sampling probe (path_mis with env_sampling): for each pair u2[i] = (row draw, column draw) of device `device`'s
+ * environment table, 8 floats: the sampled direction [3], its solid-angle density (the one the miss branch uses), the background's
+ * radiance in that direction [3], 0.  KZ_ERR_STATE when the uploaded scene does not count the environment as a light. */
+int  kzgpu_env_sample_dump(kzgpu_ctx *ctx, int device, const float *u2, size_t n, float *out8);
 
 /* Tuning knobs of the wavefront (defaults: up to 3 lanes -- frames below 2^25 paths use 2 --, 2^24 path slots per lane, runs of 64 sample
  * indices per pixel tile in path order; also read from KZGPU_LANES / KZGPU_POOL_LOG2 / KZGPU_SPP_GROUP at

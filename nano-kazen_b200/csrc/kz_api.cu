@@ -10,6 +10,7 @@
 #include "kz_lbvh.cuh"
 #include "kz_ingest.cuh"
 #include "kz_refit.cuh"
+#include "kz_env.cuh"
 #include "kz_owner.h"
 #include <cuda_runtime.h>
 #include <chrono>
@@ -79,6 +80,10 @@ struct Device {
     DevMem scratch[3];
     /* launch geometry */
     int grid_extend0 = 0, grid_extend = 0, grid_shadow = 0, grid_trace = 0, grid_occ = 0, grid_shade[KZ_NUM_CLASSES] = {0, 0, 0, 0, 0};
+    int grid_shade_env[KZ_NUM_CLASSES] = {0, 0, 0, 0, 0};     /* k_shade<CLS, true>: the environment is a light */
+    /* the environment as a light (env_setup): its table (in `tables`) and whether the render samples it */
+    KzEnvTable env{};
+    bool env_counted = false;
     /* timing */
     std::vector<EvPair> pending;
     std::vector<cudaEvent_t> free_events;
@@ -223,6 +228,8 @@ int upload_tables(kzgpu_ctx *ctx, Device &d) {
     d.rest.clear();
     d.rest.resize(h.meshes.size());
     d.frame_mem.reset();
+    d.env = KzEnvTable{};
+    d.env_counted = false;
     d.sc = h.sc;     /* flatten() without geometry leaves the accel fields of h.sc empty, as drop_all() left those of d.sc */
     auto next = [&d]() -> DevMem & { d.tables.emplace_back(); return d.tables.back(); };
     int rc;
@@ -384,6 +391,13 @@ bool hints_on(const kzgpu_ctx *ctx) {
     return ctx->primary_hint == 2 || (ctx->primary_hint == 1 && ctx->hs->total_triangles >= KZ_HINT_MIN_TRIS);
 }
 
+/* one path_mis shade pass of material class CLS; the environment-sampling instantiation when the scene counts the environment */
+template <int CLS> void launch_shade(Device &d, Lane &L, int nxt, int b, cudaStream_t s) {
+    if (d.env_counted) k_shade<CLS, true><<<d.grid_shade_env[CLS], KZ_SHADE_THREADS, 0, s>>>(d.sc, L.st, L.ctl, L.q, nxt, b, d.env);
+    else k_shade<CLS><<<d.grid_shade[CLS], KZ_SHADE_THREADS, 0, s>>>(d.sc, L.st, L.ctl, L.q, nxt, b, KzEnvTable{});
+    ++d.launches;
+}
+
 int enqueue_chunk(const kzgpu_ctx *ctx, kzgpu_ctx *ectx, Device &d, Lane &L, const KzChunk &ch, unsigned long long new_paths, cudaStream_t s) {
     const KzScene &sc = d.sc;
     const int max_depth = sc.integrator.max_depth;
@@ -413,7 +427,7 @@ int enqueue_chunk(const kzgpu_ctx *ctx, kzgpu_ctx *ectx, Device &d, Lane &L, con
             }
             {
                 Timed t(d, s, CAT_SHADE);
-                k_shade<KZ_CLASS_GENERIC><<<d.grid_shade[4], KZ_SHADE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, nxt, b);
+                k_shade<KZ_CLASS_GENERIC><<<d.grid_shade[4], KZ_SHADE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, nxt, b, KzEnvTable{});
                 ++d.launches;
             }
             if (sc.integrator.type == KZ_INTEGRATOR_AO || sc.integrator.type == KZ_INTEGRATOR_WHITTED) {
@@ -440,16 +454,15 @@ int enqueue_chunk(const kzgpu_ctx *ctx, kzgpu_ctx *ectx, Device &d, Lane &L, con
         }
         {
             Timed t(d, s, CAT_SHADE);
-            k_shade<KZ_CLASS_TERMINAL><<<d.grid_shade[0], KZ_SHADE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, nxt, b);
-            ++d.launches;
+            launch_shade<KZ_CLASS_TERMINAL>(d, L, nxt, b, s);
             if (b < max_depth) {
-                if (ctx->class_present[KZ_CLASS_DIFFUSE]) { k_shade<KZ_CLASS_DIFFUSE><<<d.grid_shade[1], KZ_SHADE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, nxt, b); ++d.launches; }
-                if (ctx->class_present[KZ_CLASS_KISS]) { k_shade<KZ_CLASS_KISS><<<d.grid_shade[2], KZ_SHADE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, nxt, b); ++d.launches; }
-                if (ctx->class_present[KZ_CLASS_NORMALMAP]) { k_shade<KZ_CLASS_NORMALMAP><<<d.grid_shade[3], KZ_SHADE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, nxt, b); ++d.launches; }
-                if (ctx->class_present[KZ_CLASS_GENERIC]) { k_shade<KZ_CLASS_GENERIC><<<d.grid_shade[4], KZ_SHADE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, nxt, b); ++d.launches; }
+                if (ctx->class_present[KZ_CLASS_DIFFUSE]) launch_shade<KZ_CLASS_DIFFUSE>(d, L, nxt, b, s);
+                if (ctx->class_present[KZ_CLASS_KISS]) launch_shade<KZ_CLASS_KISS>(d, L, nxt, b, s);
+                if (ctx->class_present[KZ_CLASS_NORMALMAP]) launch_shade<KZ_CLASS_NORMALMAP>(d, L, nxt, b, s);
+                if (ctx->class_present[KZ_CLASS_GENERIC]) launch_shade<KZ_CLASS_GENERIC>(d, L, nxt, b, s);
             }
         }
-        if (b < max_depth && sc.n_light_meshes > 0) {
+        if (b < max_depth && (sc.n_light_meshes > 0 || d.env_counted)) {
             Timed t(d, s, CAT_TRACE);
             k_shadow<<<d.grid_shadow, KZ_TRACE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, nxt);
             ++d.launches;
@@ -570,6 +583,50 @@ int emitter_upload(kzgpu_ctx *ctx, Device &d) {
     return KZ_OK;
 }
 
+/* The environment as a light (kz_env.h).  Only for path_mis with env_sampling set and a background that is not 0 in every direction:
+ * every device builds the luminance table from its own texels (sequential double sums: the same bytes on every device), and the
+ * environment counts as a light when the table's total is positive.  Otherwise the scene renders with the reference estimator. */
+int env_setup(kzgpu_ctx *ctx) {
+    const KzHostScene &h = *ctx->hs;
+    if (!h.env_sampling || h.sc.integrator.type != KZ_INTEGRATOR_PATH_MIS) return KZ_OK;
+    const KzEnvChain ch = kz_env_classify(h.sc);
+    if (ch.kind == KZ_ENV_ZERO) return KZ_OK;
+    int w = 0, hh = 0;
+    kz_env_dims(h.sc, ch, w, hh);
+    std::vector<double> sines((size_t)hh);
+    kz_env_row_sines(hh, sines.data());
+    const size_t cells = (size_t)w * (size_t)hh;
+    const unsigned cell_blocks = (unsigned)((cells + 255) / 256), row_blocks = (unsigned)((hh + 127) / 128);
+    for (Device &d : ctx->devs) {
+        KZ_CUDA(ctx, cudaSetDevice(d.id));
+        float *cdf = nullptr, *marginal = nullptr, *prob = nullptr;
+        int rc;
+        d.tables.emplace_back();
+        if ((rc = dev_alloc(ctx, d.tables.back(), cells + (size_t)hh, &cdf))) return rc;
+        d.tables.emplace_back();
+        if ((rc = dev_alloc(ctx, d.tables.back(), (size_t)hh + 1, &marginal))) return rc;
+        d.tables.emplace_back();
+        if ((rc = dev_alloc(ctx, d.tables.back(), cells, &prob))) return rc;
+        AsyncMem sin_mem, weight_mem, rows_mem, total_mem;
+        double *row_sin = nullptr, *weight = nullptr, *row_sum = nullptr, *total = nullptr;
+        if ((rc = temp_alloc(ctx, sin_mem, (size_t)hh, d.stream, &row_sin)) || (rc = temp_alloc(ctx, weight_mem, cells, d.stream, &weight)) ||
+            (rc = temp_alloc(ctx, rows_mem, (size_t)hh, d.stream, &row_sum)) || (rc = temp_alloc(ctx, total_mem, 1, d.stream, &total))) return rc;
+        KZ_CUDA(ctx, cudaMemcpyAsync(row_sin, sines.data(), (size_t)hh * sizeof(double), cudaMemcpyHostToDevice, d.stream));
+        k_env_weights<<<cell_blocks, 256, 0, d.stream>>>(d.sc, ch, row_sin, w, hh, weight);
+        k_env_rows<<<row_blocks, 128, 0, d.stream>>>(weight, w, hh, cdf, row_sum);
+        k_env_marginal<<<1, 32, 0, d.stream>>>(row_sum, hh, marginal, total);
+        k_env_probs<<<cell_blocks, 256, 0, d.stream>>>(weight, cells, total, prob);
+        d.launches += 4;
+        KZ_CUDA(ctx, cudaGetLastError());
+        double h_total = 0.0;
+        KZ_CUDA(ctx, cudaMemcpyAsync(&h_total, total, sizeof(double), cudaMemcpyDeviceToHost, d.stream));
+        KZ_CUDA(ctx, cudaStreamSynchronize(d.stream));
+        d.env = KzEnvTable{cdf, marginal, prob, w, hh};
+        d.env_counted = h_total > 0.0;
+    }
+    return KZ_OK;
+}
+
 int check_ready(kzgpu_ctx *ctx, bool need_accel) {
     if (!ctx) return fail(nullptr, KZ_ERR_INVALID, "null context");
     if (!ctx->uploaded) return fail(ctx, KZ_ERR_STATE, "no scene uploaded");
@@ -636,6 +693,11 @@ int kzgpu_create(const int *device_ids, int n_devices, kzgpu_ctx **out) {
         d.grid_shade[2] = persistent_grid(d, k_shade<KZ_CLASS_KISS>, KZ_SHADE_THREADS);
         d.grid_shade[3] = persistent_grid(d, k_shade<KZ_CLASS_NORMALMAP>, KZ_SHADE_THREADS);
         d.grid_shade[4] = persistent_grid(d, k_shade<KZ_CLASS_GENERIC>, KZ_SHADE_THREADS);
+        d.grid_shade_env[0] = persistent_grid(d, k_shade<KZ_CLASS_TERMINAL, true>, KZ_SHADE_THREADS);
+        d.grid_shade_env[1] = persistent_grid(d, k_shade<KZ_CLASS_DIFFUSE, true>, KZ_SHADE_THREADS);
+        d.grid_shade_env[2] = persistent_grid(d, k_shade<KZ_CLASS_KISS, true>, KZ_SHADE_THREADS);
+        d.grid_shade_env[3] = persistent_grid(d, k_shade<KZ_CLASS_NORMALMAP, true>, KZ_SHADE_THREADS);
+        d.grid_shade_env[4] = persistent_grid(d, k_shade<KZ_CLASS_GENERIC, true>, KZ_SHADE_THREADS);
     }
     /* a multi-device context replicates the scene and merges the frames through peer memory (NVLink / NVSwitch): every pair of its
      * devices must be able to map each other's HBM */
@@ -710,6 +772,7 @@ int kzgpu_scene_upload(kzgpu_ctx *ctx, const kz_scene_desc *scene) {
         else rc = replicate_geometry(ctx, d, ctx->devs[0]);
         if (rc) return rc;
     }
+    if (int rc = env_setup(ctx)) return rc;
     KZ_CUDA(ctx, cudaSetDevice(ctx->devs[0].id));
     ctx->uploaded = true;
     ctx->ms_upload = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -1257,6 +1320,25 @@ int kzgpu_light_sample_dump(kzgpu_ctx *ctx, const float *ref3, const float *u5, 
                                                                             (uint32_t)n, reinterpret_cast<float *>(d->scratch[1].p));
     ++d->launches;
     KZ_CUDA(ctx, cudaMemcpyAsync(out16, d->scratch[1].p, n * 64, cudaMemcpyDeviceToHost, d->stream));
+    KZ_CUDA(ctx, cudaStreamSynchronize(d->stream));
+    return KZ_OK;
+}
+
+int kzgpu_env_sample_dump(kzgpu_ctx *ctx, int device, const float *u2, size_t n, float *out8) {
+    int rc = check_ready(ctx, false);
+    if (rc) return rc;
+    Device *d;
+    if ((rc = select(ctx, device, &d))) return rc;
+    if (!d->env_counted) return fail(ctx, KZ_ERR_STATE, "the scene does not count the environment as a light (env_sampling off, not path_mis, or a background that is 0 everywhere)");
+    if (n == 0) return KZ_OK;
+    if (!u2 || !out8) return fail(ctx, KZ_ERR_INVALID, "null argument");
+    if (n > 0x7FFFFFFFull) return fail(ctx, KZ_ERR_INVALID, "batch too large");
+    KZ_CUDA(ctx, d->scratch[0].ensure(n * 8, SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[1].ensure(n * 32, SCRATCH_MIN));
+    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0].p, u2, n * 8, cudaMemcpyHostToDevice, d->stream));
+    k_env_sample_dump<<<(unsigned)((n + 127) / 128), 128, 0, d->stream>>>(d->sc, d->env, reinterpret_cast<const float *>(d->scratch[0].p), (uint32_t)n, reinterpret_cast<float *>(d->scratch[1].p));
+    ++d->launches;
+    KZ_CUDA(ctx, cudaMemcpyAsync(out8, d->scratch[1].p, n * 32, cudaMemcpyDeviceToHost, d->stream));
     KZ_CUDA(ctx, cudaStreamSynchronize(d->stream));
     return KZ_OK;
 }

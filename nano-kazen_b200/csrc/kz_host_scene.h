@@ -28,6 +28,7 @@ struct KzHostScene {
     std::vector<kzbvh::Tri> tris;       /* scene order, input of the accel build */
     KzScene sc;                         /* pointers into the vectors above once finalize() ran */
     uint64_t total_vertices = 0, total_triangles = 0;
+    bool env_sampling = false;          /* kz_integrator_desc::env_sampling (kz_api.cu builds the environment table, kz_env.h) */
     std::string error;
 
     /* geometry = true: vertex / index records and the triangle list are built here (tests/hostemu runs the device headers on
@@ -143,7 +144,10 @@ struct KzHostScene {
         sc.background = d->background;
         if (sc.background >= (int)d->n_textures) { error = "background texture out of range"; return false; }
         sc.camera = d->camera;
-        sc.integrator = d->integrator;
+        sc.integrator.max_depth = d->integrator.max_depth; sc.integrator.trace_bias = d->integrator.trace_bias;
+        sc.integrator.regularization = d->integrator.regularization; sc.integrator.accumulated_roughness = d->integrator.accumulated_roughness;
+        sc.integrator.type = d->integrator.type;
+        env_sampling = d->integrator.env_sampling != 0;
         if (sc.integrator.type < KZ_INTEGRATOR_PATH_MIS || sc.integrator.type > KZ_INTEGRATOR_PATH_MATS) { error = "unknown integrator type"; return false; }
         sc.filter = d->filter;
         sc.border = (int32_t)ceilf(d->filter.radius - 0.5f);

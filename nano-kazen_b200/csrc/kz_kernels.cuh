@@ -421,8 +421,12 @@ __global__ void __launch_bounds__(KZ_TRACE_THREADS, KZ_TRACE_MIN_BLOCKS) k_exten
 #ifndef KZ_SHADE_MIN_BLOCKS
 #define KZ_SHADE_MIN_BLOCKS 4
 #endif
-template <int CLS>
-__global__ void __launch_bounds__(KZ_SHADE_THREADS, (CLS == KZ_CLASS_DIFFUSE ? KZ_SHADE_MIN_BLOCKS_DIFFUSE : (CLS == KZ_CLASS_TERMINAL ? KZ_SHADE_MIN_BLOCKS_TERMINAL : KZ_SHADE_MIN_BLOCKS))) k_shade(KzScene sc, KzPathState st, KzControl *ctl, KzQueues q, int nxt, int bounce) {
+#ifndef KZ_SHADE_MIN_BLOCKS_ENV
+#define KZ_SHADE_MIN_BLOCKS_ENV 3           /* environment sampling: up to 168 registers, so that no class spills more than its flag-off kernel */
+#endif
+/* ENV: the environment is a light with table `env` (ignored when ENV is false), see kz_shade_item */
+template <int CLS, bool ENV = false>
+__global__ void __launch_bounds__(KZ_SHADE_THREADS, (ENV && CLS != KZ_CLASS_TERMINAL ? KZ_SHADE_MIN_BLOCKS_ENV : (CLS == KZ_CLASS_DIFFUSE ? KZ_SHADE_MIN_BLOCKS_DIFFUSE : (CLS == KZ_CLASS_TERMINAL ? KZ_SHADE_MIN_BLOCKS_TERMINAL : KZ_SHADE_MIN_BLOCKS)))) k_shade(KzScene sc, KzPathState st, KzControl *ctl, KzQueues q, int nxt, int bounce, KzEnvTable env) {
     const uint32_t n = ctl->n_class[CLS];
     const uint32_t *queue = q.cls[CLS];
     const uint32_t stride = gridDim.x * blockDim.x;
@@ -439,7 +443,7 @@ __global__ void __launch_bounds__(KZ_SHADE_THREADS, (CLS == KZ_CLASS_DIFFUSE ? K
         uint32_t slot = 0u, flags = 0u;
         if (idx < n) {
             slot = queue[idx];
-            flags = kz_shade_item<CLS>(sc, st, slot, bounce, cnt);
+            flags = kz_shade_item<CLS, ENV>(sc, st, slot, bounce, cnt, env);
         }
         if (CLS != KZ_CLASS_TERMINAL) {
             const bool pa = (flags & KZ_SHADE_CONTINUE) != 0u, pb = (flags & KZ_SHADE_SHADOW) != 0u;
@@ -467,7 +471,7 @@ __global__ void __launch_bounds__(KZ_SHADE_THREADS, (CLS == KZ_CLASS_DIFFUSE ? K
         uint32_t slot = 0u, flags = 0u;
         if (idx < n) {
             slot = queue[idx];
-            flags = kz_shade_item<CLS>(sc, st, slot, bounce, cnt);
+            flags = kz_shade_item<CLS, ENV>(sc, st, slot, bounce, cnt, env);
         }
         __syncwarp();
         if (CLS != KZ_CLASS_TERMINAL)

@@ -16,7 +16,7 @@
  */
 #ifndef KZ_PATH_H
 #define KZ_PATH_H
-#include "kz_shade.h"
+#include "kz_env.h"
 
 /* Path state: three 64-byte blocks per slot, grouped by which stage touches what, so that every access of a stage is a
  * whole 32-byte DRAM sector (slots are visited in queue order, i.e. scattered: the former one-array-per-field layout moved a
@@ -170,11 +170,9 @@ struct KzEmitterSample {
     kz3 p, n, wi;        /* sampled point, its (unnormalised) normal, direction ref -> p */
     float dist, pdf;     /* |p - ref|, solid-angle density (0: not usable); the pick probability 1/n_lights is NOT included */
 };
-KZ_HD KzEmitterSample kz_sample_emitter(const KzScene &sc, kz3 ref, float u_pick, float u_tri, float u_b1, float u_b2) {
+/* `index`: the picked emitter, into light_meshes */
+KZ_HD KzEmitterSample kz_sample_emitter_at(const KzScene &sc, uint32_t index, kz3 ref, float u_tri, float u_b1, float u_b2) {
     KzEmitterSample es;
-    const uint32_t nl = (uint32_t)sc.n_light_meshes;
-    uint32_t index = (uint32_t)floorf((float)nl * u_pick);
-    if (index > nl - 1) index = nl - 1;
     es.mesh = sc.light_meshes[index];
     const KzMeshRec lm = sc.meshes[es.mesh];
     es.light = lm.light;
@@ -199,13 +197,22 @@ KZ_HD KzEmitterSample kz_sample_emitter(const KzScene &sc, kz3 ref, float u_pick
     es.pdf = light_pdf(lm.inv_area, ref, es.p, es.n, es.wi);
     return es;
 }
+KZ_HD KzEmitterSample kz_sample_emitter(const KzScene &sc, kz3 ref, float u_pick, float u_tri, float u_b1, float u_b2) {
+    const uint32_t nl = (uint32_t)sc.n_light_meshes;
+    uint32_t index = (uint32_t)floorf((float)nl * u_pick);
+    if (index > nl - 1) index = nl - 1;
+    return kz_sample_emitter_at(sc, index, ref, u_tri, u_b1, u_b2);
+}
 
 /* ---- shade --------------------------------------------------------------------------------- */
 KZ_HD_NOINLINE uint32_t kz_shade_alt_item(const KzScene &sc, const KzPathState &st, uint32_t slot, int bounce, KzCounters &cnt);
 
-/* CLS = material class of the queue this item was sorted into (-1: unknown, resolve at run time) */
-template <int CLS = -1>
-KZ_HD uint32_t kz_shade_item(const KzScene &sc, const KzPathState &st, uint32_t slot, int bounce, KzCounters &cnt) {
+/* CLS = material class of the queue this item was sorted into (-1: unknown, resolve at run time).
+ * ENV = the environment is a light with table `env` (kz_env.h): next-event estimation picks it as light n_light_meshes with
+ * probability 1 / (n_light_meshes + 1), and a BSDF-sampled ray that escapes is weighted against its density.  ENV = false is the
+ * reference estimator and does not read `env`. */
+template <int CLS = -1, bool ENV = false>
+KZ_HD uint32_t kz_shade_item(const KzScene &sc, const KzPathState &st, uint32_t slot, int bounce, KzCounters &cnt, const KzEnvTable &env = KzEnvTable{}) {
     if ((CLS < 0 || CLS == KZ_CLASS_GENERIC) && sc.integrator.type != KZ_INTEGRATOR_PATH_MIS) return kz_shade_alt_item(sc, st, slot, bounce, cnt);
     const KzBlockA A = st.a[slot];
     const KzF4 ro = A.ray.o, rd = A.ray.d;
@@ -216,13 +223,14 @@ KZ_HD uint32_t kz_shade_item(const KzScene &sc, const KzPathState &st, uint32_t 
     kz3 throughput = mk3(thr4.x, thr4.y, thr4.z), L = mk3(L4.x, L4.y, L4.z);
     float eta = thr4.w, bsdfWeight = 1.f;       /* integrator.cpp:207: only changes when a sampled ray lands on a light (below) */
     const float prevBsdfPdf = L4.w;
-    const kz_integrator_desc I = sc.integrator;
+    const KzIntegrator I = sc.integrator;
 
     if (CLS <= KZ_CLASS_TERMINAL && h.geom == KZ_INVALID_ID) {     /* material-class queues never hold misses */
         /* bounce 0: camera rays never see the background (integrator.cpp:210-212);
          * later: Li += throughput * background(ray.d) (integrator.cpp:315-318) */
         if (bounce > 0) {
-            L += throughput * kz_background(sc, rayD);
+            if (ENV) L += throughput * kz_background(sc, rayD) * (prevBsdfPdf < 0.f ? 1.f : power_heuristic(prevBsdfPdf, kz_env_pdf(env, rayD)));
+            else L += throughput * kz_background(sc, rayD);
             st.b[slot].rad.L = mkf4(L.x, L.y, L.z, bsdfWeight);
         }
         return 0u;
@@ -269,7 +277,44 @@ KZ_HD uint32_t kz_shade_item(const KzScene &sc, const KzPathState &st, uint32_t 
 
     /* ---- light sampling, integrator.cpp:247-294 ---- */
     const float rnd = kz_next1d(sc, sm);
-    if (sc.n_light_meshes > 0) {
+    if (ENV) {
+        /* the reference's draws, whichever light is picked; the environment uses the second and third and leaves the fourth */
+        const uint32_t nl = (uint32_t)sc.n_light_meshes + 1u;
+        const float u_tri = kz_next1d(sc, sm);
+        const float u_b1 = kz_next1d(sc, sm);
+        const float u_b2 = kz_next1d(sc, sm);
+        uint32_t index = (uint32_t)floorf((float)nl * rnd);
+        if (index > nl - 1) index = nl - 1;
+        if (index == nl - 1) {
+            const kz3 lwi = kz_env_sample(env, u_tri, u_b1);
+            const float lpdf = kz_env_pdf(env, lwi);
+            if (lpdf > 0.f && !isnan(lpdf) && !isinf(lpdf)) {
+                const kz3 Ls = kz_background(sc, lwi) / lpdf * (float)nl;
+                kz3 f; float bsdfPdf;
+                bsdf_eval_pdf(bc, its, wiLocal, to_local(its.sh, lwi), &f, &bsdfPdf);
+                const kz3 contrib = throughput * Ls * f * power_heuristic(lpdf, bsdfPdf);
+                if (!iszero(contrib)) {
+                    KzShdRec shd; shd.d = mkf4(lwi.x, lwi.y, lwi.z, KZ_INF); shd.pending = mkf4(contrib.x, contrib.y, contrib.z, eps);
+                    st.c[slot].shd = shd;
+                    flags |= KZ_SHADE_SHADOW;
+                }
+            }
+        } else {
+            const KzEmitterSample es = kz_sample_emitter_at(sc, index, its.p, u_tri, u_b1, u_b2);
+            if (es.pdf > 0.f && !isnan(es.pdf) && !isinf(es.pdf)) {
+                const kz_light_desc l = sc.lights[es.light];
+                const kz3 Ls = mk3(l.radiance[0], l.radiance[1], l.radiance[2]) / es.pdf / (1.f / (float)nl);
+                kz3 f; float bsdfPdf;
+                bsdf_eval_pdf(bc, its, wiLocal, to_local(its.sh, es.wi), &f, &bsdfPdf);
+                const kz3 contrib = throughput * Ls * f * power_heuristic(es.pdf, bsdfPdf);
+                if (!iszero(contrib)) {
+                    KzShdRec shd; shd.d = mkf4(es.wi.x, es.wi.y, es.wi.z, es.dist - eps); shd.pending = mkf4(contrib.x, contrib.y, contrib.z, eps);
+                    st.c[slot].shd = shd;
+                    flags |= KZ_SHADE_SHADOW;
+                }
+            }
+        }
+    } else if (sc.n_light_meshes > 0) {
         const uint32_t nl = (uint32_t)sc.n_light_meshes;
         const float u_tri = kz_next1d(sc, sm);
         const float u_b1 = kz_next1d(sc, sm);

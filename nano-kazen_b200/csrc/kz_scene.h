@@ -64,6 +64,15 @@ struct KzImageRec {
     int32_t  n_levels;        /* mip pyramid levels resident after level 0 (level l follows l-1) */
 };
 
+/* kz_integrator_desc as the kernels read it (the same layout as before env_sampling): kzgpu_scene_upload resolves env_sampling into which k_shade instantiations run */
+struct KzIntegrator {
+    int32_t max_depth;
+    float   trace_bias;
+    int32_t regularization;
+    float   accumulated_roughness;
+    int32_t type;
+};
+
 struct KzScene {
     /* accel */
     const KzNode8 *nodes;
@@ -89,7 +98,7 @@ struct KzScene {
     int32_t                background;
     /* render setup */
     kz_camera_desc     camera;
-    kz_integrator_desc integrator;
+    KzIntegrator       integrator;
     kz_filter_desc     filter;
     int32_t            border;
     /* sampler */

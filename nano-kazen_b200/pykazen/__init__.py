@@ -72,7 +72,7 @@ class SamplerDesc(C.Structure):
 
 class IntegratorDesc(C.Structure):
     _fields_ = [("max_depth", C.c_int32), ("trace_bias", C.c_float), ("regularization", C.c_int32),
-                ("accumulated_roughness", C.c_float), ("type", C.c_int32)]
+                ("accumulated_roughness", C.c_float), ("type", C.c_int32), ("env_sampling", C.c_int32)]
 
 
 class FilterDesc(C.Structure):
@@ -326,9 +326,10 @@ class SceneBuilder:
         self.filter.radius = r
         self.filter.table[:] = tab.tolist()
 
-    def set_integrator(self, max_depth=5, trace_bias=1e-3, regularization=False, accumulated_roughness=0.5, kind="path_mis"):
+    def set_integrator(self, max_depth=5, trace_bias=1e-3, regularization=False, accumulated_roughness=0.5, kind="path_mis", env_sampling=False):
+        """env_sampling: path_mis also samples the background as a light (kz_integrator_desc::env_sampling in include/kzgpu.h)"""
         t = {"path_mis": 0, "normals": 1, "ao": 2, "whitted": 3, "path_mats": 4}[kind]
-        self.integrator = IntegratorDesc(min(512, max_depth), trace_bias, int(regularization), accumulated_roughness, t)
+        self.integrator = IntegratorDesc(min(512, max_depth), trace_bias, int(regularization), accumulated_roughness, t, int(env_sampling))
 
     def desc(self):
         d = SceneDesc()
@@ -558,6 +559,14 @@ class Gpu(_Backend):
         st = np.ascontiguousarray(st, np.float32).reshape(-1, 2)
         out = np.zeros((st.shape[0], 3), np.float32)
         self._call("image_lookup", self.h, C.c_int(image), C.c_int(level), st.ctypes.data_as(c_float_p), C.c_size_t(st.shape[0]), out.ctypes.data_as(c_float_p))
+        return out
+
+    def env_sample_dump(self, u2, device=0):
+        """environment light samples of device `device` for (row draw, column draw) pairs: (n, 8) float32 = direction[3], density,
+        radiance[3], 0 (include/kzgpu.h); raises unless the scene counts the environment as a light"""
+        u2 = np.ascontiguousarray(u2, np.float32).reshape(-1, 2)
+        out = np.zeros((u2.shape[0], 8), np.float32)
+        self._call("env_sample_dump", self.h, C.c_int(device), u2.ctypes.data_as(c_float_p), C.c_size_t(u2.shape[0]), out.ctypes.data_as(c_float_p))
         return out
 
     def configure(self, key, value):
