@@ -200,6 +200,16 @@ typedef struct kz_integrator_desc {
      * a window) it converges much faster.  Nothing changes when the background is absent or black in every direction (no
      * background, zero intensity, colorramp / blend chains, an all-black image), nor for the other integrators. */
     int32_t env_sampling;
+    /* path_mis only ("textureFiltering", default 0 = every texture lookup reads mip level 0, as the reference does): 1 filters image
+     * textures by their screen footprint.  Every image then gets its full mip pyramid resident in HBM (built on the GPU at
+     * kzgpu_scene_upload; about a third more texels), and a uv-mode lookup of a texture a BSDF reads (kazenstandard baseColor /
+     * roughness / metallic, a normal map, the lambertian / ggx albedo) is a trilinear lookup at the level of the footprint: bicubic at
+     * the two levels around it, lerped; level 0 exactly when the texture is magnified.  The footprint is pbrt-v4's camera estimate
+     * (uv derivatives at the hit from the camera alone, scaled by max(1/8, 1/sqrt(sample_count))), so far-away and grazing textures
+     * stop aliasing and converge at low sample counts.  It does not follow the path: after a bounce the lookup is as sharp as the
+     * camera would see that point.  Background lookups always read level 0.  Nothing changes when no such texture reads an image,
+     * nor for the other integrators. */
+    int32_t texture_filtering;
 } kz_integrator_desc;
 
 /* Reconstruction filter tabulated as ImageBlock does (block.cpp:13-21). */
@@ -333,8 +343,8 @@ int  kzgpu_camera_rays(kzgpu_ctx *ctx, const float *samples4, size_t n, kz_ray *
 int  kzgpu_bsdf_query(kzgpu_ctx *ctx, int bsdf, int mode, const float wi[3], const float wo[3], const float uv[2],
                       float accumulated_roughness, float sample1, const float sample2[2], float out[8]);
 
-/* Texture probe: periodic bicubic lookup of image `image` at mip `level` (0 = finest; the pyramid is built on the GPU at
- * upload and stays resident in HBM) for n (s,t) pairs -> n rgb triples.  ImageTexture::eval's texture() call with zero
+/* Texture probe: periodic bicubic lookup of image `image` at mip `level` (0 = finest; the pyramid is built on the GPU by 2x2 box
+ * filtering: the resident one when the scene filters its textures, otherwise a temporary one for this call) for n (s,t) pairs -> n rgb triples.  ImageTexture::eval's texture() call with zero
  * derivatives (texture.cpp:46-64) is level 0 with s = u*scale, t = (1-v)*scale. */
 int  kzgpu_image_lookup(kzgpu_ctx *ctx, int image, int level, const float *st, size_t n, float *rgb);
 
@@ -370,6 +380,16 @@ int  kzgpu_light_sample_dump(kzgpu_ctx *ctx, const float *ref3, const float *u5,
  * environment table, 8 floats: the sampled direction [3], its solid-angle density (the one the miss branch uses), the background's
  * radiance in that direction [3], 0.  KZ_ERR_STATE when the uploaded scene does not count the environment as a light. */
 int  kzgpu_env_sample_dump(kzgpu_ctx *ctx, int device, const float *u2, size_t n, float *out8);
+
+/* Texture footprint probe (texture_filtering): traces each ray on device `device` and writes 8 floats at its closest hit: mesh (as
+ * float, -1 = miss), uv[2] (as the shader sees it), du/dx, dv/dx, du/dy, dv/dy (the footprint the filtered shade kernels compute
+ * there, for the current camera and vertices), 0.  Runs whether or not the scene filters its textures. */
+int  kzgpu_texture_footprint_dump(kzgpu_ctx *ctx, int device, const kz_ray *rays, size_t n, float *out8);
+
+/* Filtered texture probe: the shade kernels' lookup of image `image` for n (s, t) pairs with st derivatives dst4[i] = (ds/dx, dt/dx,
+ * ds/dy, dt/dy) -> n rgb triples (before sRGB linearisation), on the first device.  KZ_ERR_STATE unless the uploaded scene filters
+ * its textures (the pyramids are resident only then). */
+int  kzgpu_image_lookup_filtered(kzgpu_ctx *ctx, int image, const float *st, const float *dst4, size_t n, float *rgb);
 
 /* Tuning knobs of the wavefront (defaults: up to 3 lanes -- frames below 2^25 paths use 2 --, 2^24 path slots per lane, runs of 64 sample
  * indices per pixel tile in path order; also read from KZGPU_LANES / KZGPU_POOL_LOG2 / KZGPU_SPP_GROUP at

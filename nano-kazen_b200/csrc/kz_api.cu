@@ -84,6 +84,11 @@ struct Device {
     /* the environment as a light (env_setup): its table (in `tables`) and whether the render samples it */
     KzEnvTable env{};
     bool env_counted = false;
+    /* texture filtering: whether the scene's textures are filtered (their pyramids are resident), k_shade<CLS, ENV, true>'s grids,
+     * and the camera constants of the footprint (kept current for the footprint probe whether or not the scene filters) */
+    bool tex_filtering = false;
+    int grid_shade_tex[2][KZ_NUM_CLASSES] = {{0, 0, 0, 0, 0}, {0, 0, 0, 0, 0}};
+    KzTexLod lod{};
     /* timing */
     std::vector<EvPair> pending;
     std::vector<cudaEvent_t> free_events;
@@ -230,6 +235,8 @@ int upload_tables(kzgpu_ctx *ctx, Device &d) {
     d.frame_mem.reset();
     d.env = KzEnvTable{};
     d.env_counted = false;
+    d.tex_filtering = h.pyramids;
+    d.lod = kz_tex_lod(h.sc.camera, h.sc.sample_count);
     d.sc = h.sc;     /* flatten() without geometry leaves the accel fields of h.sc empty, as drop_all() left those of d.sc */
     auto next = [&d]() -> DevMem & { d.tables.emplace_back(); return d.tables.back(); };
     int rc;
@@ -252,7 +259,20 @@ int upload_tables(kzgpu_ctx *ctx, Device &d) {
     return KZ_OK;
 }
 
-/* Mesh and image arrays -> HBM records on device `d` (kz_ingest.cuh).  Host arrays are copied into a staging buffer with one
+/* Enqueues levels 1 .. n_levels of the mip pyramid whose level 0 (w x h) is at texels + offset, each the 2x2 box filter of the one before,
+ * contiguous after it (kz_mip_level's layout) */
+void enqueue_mip_levels(Device &d, KzF4 *texels, size_t offset, int w, int h, int n_levels) {
+    for (int l = 1; l <= n_levels; ++l) {
+        const int dw = w > 1 ? w >> 1 : 1, dh = h > 1 ? h >> 1 : 1;
+        const size_t dst = offset + (size_t)w * h;
+        dim3 blk(32, 8), grd((unsigned)(dw + 31) / 32, (unsigned)(dh + 7) / 8);
+        k_mip_level<<<grd, blk, 0, d.stream>>>(texels, offset, w, h, dst, dw, dh);
+        ++d.launches;
+        offset = dst; w = dw; h = dh;
+    }
+}
+
+/* Mesh and image arrays -> HBM records on device `d` (kz_ingest.cuh); with texture filtering the images' pyramids too.  Host arrays are copied into a staging buffer with one
  * cudaMemcpyAsync each; arrays that already live on a device are read where they are. */
 int ingest_geometry(kzgpu_ctx *ctx, Device &d, const kz_scene_desc *scene) {
     const KzHostScene &h = *ctx->hs;
@@ -299,6 +319,8 @@ int ingest_geometry(kzgpu_ctx *ctx, Device &d, const kz_scene_desc *scene) {
         if (e != cudaSuccess) break;
         k_ingest_texels<<<grid_for(n, 256, d.sm_count), 256, 0, d.stream>>>(rgb, n, texels + h.images[i].texel_offset);
         ++d.launches;
+        const KzImageRec &r = h.images[i];
+        if (d.tex_filtering) enqueue_mip_levels(d, texels, r.texel_offset, r.width, r.height, r.n_levels);
     }
     uint32_t h_bad = 0;
     if (e == cudaSuccess) e = cudaMemcpyAsync(&h_bad, bad, 4, cudaMemcpyDeviceToHost, d.stream);
@@ -391,10 +413,19 @@ bool hints_on(const kzgpu_ctx *ctx) {
     return ctx->primary_hint == 2 || (ctx->primary_hint == 1 && ctx->hs->total_triangles >= KZ_HINT_MIN_TRIS);
 }
 
-/* one path_mis shade pass of material class CLS; the environment-sampling instantiation when the scene counts the environment */
+/* one path_mis shade pass of material class CLS; the environment-sampling instantiation when the scene counts the environment, the
+ * texture-filtering one when the scene filters its textures and the class can read an image (TERMINAL and DIFFUSE read no textures) */
 template <int CLS> void launch_shade(Device &d, Lane &L, int nxt, int b, cudaStream_t s) {
-    if (d.env_counted) k_shade<CLS, true><<<d.grid_shade_env[CLS], KZ_SHADE_THREADS, 0, s>>>(d.sc, L.st, L.ctl, L.q, nxt, b, d.env);
-    else k_shade<CLS><<<d.grid_shade[CLS], KZ_SHADE_THREADS, 0, s>>>(d.sc, L.st, L.ctl, L.q, nxt, b, KzEnvTable{});
+    if constexpr (CLS == KZ_CLASS_KISS || CLS == KZ_CLASS_NORMALMAP || CLS == KZ_CLASS_GENERIC) {
+        if (d.tex_filtering) {
+            if (d.env_counted) k_shade<CLS, true, true><<<d.grid_shade_tex[1][CLS], KZ_SHADE_THREADS, 0, s>>>(d.sc, L.st, L.ctl, L.q, nxt, b, d.env, d.lod);
+            else k_shade<CLS, false, true><<<d.grid_shade_tex[0][CLS], KZ_SHADE_THREADS, 0, s>>>(d.sc, L.st, L.ctl, L.q, nxt, b, KzEnvTable{}, d.lod);
+            ++d.launches;
+            return;
+        }
+    }
+    if (d.env_counted) k_shade<CLS, true><<<d.grid_shade_env[CLS], KZ_SHADE_THREADS, 0, s>>>(d.sc, L.st, L.ctl, L.q, nxt, b, d.env, KzTexLod{});
+    else k_shade<CLS><<<d.grid_shade[CLS], KZ_SHADE_THREADS, 0, s>>>(d.sc, L.st, L.ctl, L.q, nxt, b, KzEnvTable{}, KzTexLod{});
     ++d.launches;
 }
 
@@ -427,7 +458,7 @@ int enqueue_chunk(const kzgpu_ctx *ctx, kzgpu_ctx *ectx, Device &d, Lane &L, con
             }
             {
                 Timed t(d, s, CAT_SHADE);
-                k_shade<KZ_CLASS_GENERIC><<<d.grid_shade[4], KZ_SHADE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, nxt, b, KzEnvTable{});
+                k_shade<KZ_CLASS_GENERIC><<<d.grid_shade[4], KZ_SHADE_THREADS, 0, s>>>(sc, L.st, L.ctl, L.q, nxt, b, KzEnvTable{}, KzTexLod{});
                 ++d.launches;
             }
             if (sc.integrator.type == KZ_INTEGRATOR_AO || sc.integrator.type == KZ_INTEGRATOR_WHITTED) {
@@ -698,6 +729,12 @@ int kzgpu_create(const int *device_ids, int n_devices, kzgpu_ctx **out) {
         d.grid_shade_env[2] = persistent_grid(d, k_shade<KZ_CLASS_KISS, true>, KZ_SHADE_THREADS);
         d.grid_shade_env[3] = persistent_grid(d, k_shade<KZ_CLASS_NORMALMAP, true>, KZ_SHADE_THREADS);
         d.grid_shade_env[4] = persistent_grid(d, k_shade<KZ_CLASS_GENERIC, true>, KZ_SHADE_THREADS);
+        d.grid_shade_tex[0][2] = persistent_grid(d, k_shade<KZ_CLASS_KISS, false, true>, KZ_SHADE_THREADS);
+        d.grid_shade_tex[0][3] = persistent_grid(d, k_shade<KZ_CLASS_NORMALMAP, false, true>, KZ_SHADE_THREADS);
+        d.grid_shade_tex[0][4] = persistent_grid(d, k_shade<KZ_CLASS_GENERIC, false, true>, KZ_SHADE_THREADS);
+        d.grid_shade_tex[1][2] = persistent_grid(d, k_shade<KZ_CLASS_KISS, true, true>, KZ_SHADE_THREADS);
+        d.grid_shade_tex[1][3] = persistent_grid(d, k_shade<KZ_CLASS_NORMALMAP, true, true>, KZ_SHADE_THREADS);
+        d.grid_shade_tex[1][4] = persistent_grid(d, k_shade<KZ_CLASS_GENERIC, true, true>, KZ_SHADE_THREADS);
     }
     /* a multi-device context replicates the scene and merges the frames through peer memory (NVLink / NVSwitch): every pair of its
      * devices must be able to map each other's HBM */
@@ -754,6 +791,9 @@ int kzgpu_scene_upload(kzgpu_ctx *ctx, const kz_scene_desc *scene) {
         const bool unsupported = hs->error.find("outside the hot-path scope") != std::string::npos || hs->error.find("unsupported") != std::string::npos;
         return fail(ctx, unsupported ? KZ_ERR_UNSUPPORTED : KZ_ERR_INVALID, hs->error);
     }
+    /* texture filtering: room for every image's pyramid (ingest_geometry fills it on the GPU after level 0); a scene where filtering does
+     * not count keeps the reference's layout, allocations and launches */
+    if (hs->filter_counts() && !hs->mip_layout()) return fail(ctx, KZ_ERR_INVALID, hs->error);
     ctx->hs = std::move(hs);
     ctx->uploaded = false;
     drop_all(ctx);
@@ -1047,7 +1087,8 @@ int kzgpu_camera_update(kzgpu_ctx *ctx, const kz_camera_desc *camera) {
     if (camera->width != ctx->hs->sc.camera.width || camera->height != ctx->hs->sc.camera.height)
         return fail(ctx, KZ_ERR_INVALID, "camera size differs from the uploaded one (the frame and the primary-hit hints are sized by it)");
     ctx->hs->sc.camera = *camera;
-    for (Device &d : ctx->devs) d.sc.camera = *camera;
+    const KzTexLod lod = kz_tex_lod(*camera, ctx->hs->sc.sample_count);
+    for (Device &d : ctx->devs) { d.sc.camera = *camera; d.lod = lod; }
     return KZ_OK;
 }
 
@@ -1249,9 +1290,9 @@ int kzgpu_image_lookup(kzgpu_ctx *ctx, int image, int level, const float *st, si
     KzScene sc = d->sc;
     int lookup_image = image;
     DevMem pyr_mem, rec_mem;
-    if (level > 0) {
-        /* the renderer only reads level 0 (ImageTexture::eval passes zero derivatives, texture.cpp:52-57), so the pyramid is not
-         * kept resident: it is built here, for this image, by 2x2 box filtering on the device */
+    if (level > 0 && !ctx->hs->pyramids) {
+        /* without texture filtering the renderer only reads level 0 (ImageTexture::eval passes zero derivatives, texture.cpp:52-57),
+         * so no pyramid is resident: it is built here, for this image, by 2x2 box filtering on the device */
         const KzImageRec im = ctx->hs->images[(size_t)image];
         KzImageRec pr = im; pr.texel_offset = 0; pr.n_levels = 0;
         size_t total = (size_t)im.width * im.height;
@@ -1261,15 +1302,7 @@ int kzgpu_image_lookup(kzgpu_ctx *ctx, int image, int level, const float *st, si
         cudaError_t e = cudaMemcpyAsync(pyr, d->sc.texels + im.texel_offset, (size_t)im.width * im.height * sizeof(KzF4), cudaMemcpyDeviceToDevice, d->stream);
         if (e == cudaSuccess) e = cudaMemcpyAsync(rec, &pr, sizeof(pr), cudaMemcpyHostToDevice, d->stream);
         KZ_CUDA(ctx, e);
-        size_t src = 0; int sw = im.width, sh = im.height;
-        for (int l = 1; l <= pr.n_levels; ++l) {
-            const int dw = sw > 1 ? sw >> 1 : 1, dh = sh > 1 ? sh >> 1 : 1;
-            const size_t dst = src + (size_t)sw * sh;
-            dim3 blk(32, 8), grd((unsigned)(dw + 31) / 32, (unsigned)(dh + 7) / 8);
-            k_mip_level<<<grd, blk, 0, d->stream>>>(pyr, src, sw, sh, dst, dw, dh);
-            ++d->launches;
-            src = dst; sw = dw; sh = dh;
-        }
+        enqueue_mip_levels(*d, pyr, 0, im.width, im.height, pr.n_levels);
         sc.texels = pyr; sc.images = rec; lookup_image = 0;
     }
     cudaError_t e = cudaMemcpyAsync(d->scratch[0].p, st, n * 8, cudaMemcpyHostToDevice, d->stream);
@@ -1281,6 +1314,47 @@ int kzgpu_image_lookup(kzgpu_ctx *ctx, int image, int level, const float *st, si
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(d->stream);
     KZ_CUDA(ctx, e);
+    return KZ_OK;
+}
+
+int kzgpu_image_lookup_filtered(kzgpu_ctx *ctx, int image, const float *st, const float *dst4, size_t n, float *rgb) {
+    int rc = check_ready(ctx, false);
+    if (rc) return rc;
+    Device *d;
+    if ((rc = select(ctx, 0, &d))) return rc;
+    if (!ctx->hs->pyramids) return fail(ctx, KZ_ERR_STATE, "the scene does not filter its textures (texture_filtering off, not path_mis, or no BSDF texture reads an image)");
+    if (image < 0 || image >= (int)ctx->hs->images.size()) return fail(ctx, KZ_ERR_INVALID, "image index out of range");
+    if (n == 0) return KZ_OK;
+    if (!st || !dst4 || !rgb) return fail(ctx, KZ_ERR_INVALID, "null argument");
+    if (n > 0x7FFFFFFFull) return fail(ctx, KZ_ERR_INVALID, "batch too large");
+    KZ_CUDA(ctx, d->scratch[0].ensure(n * 24, SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[1].ensure(n * 12, SCRATCH_MIN));
+    float *in = reinterpret_cast<float *>(d->scratch[0].p);
+    KZ_CUDA(ctx, cudaMemcpyAsync(in, st, n * 8, cudaMemcpyHostToDevice, d->stream));
+    KZ_CUDA(ctx, cudaMemcpyAsync(in + 2 * n, dst4, n * 16, cudaMemcpyHostToDevice, d->stream));
+    k_image_lookup_filtered<<<(unsigned)((n + 127) / 128), 128, 0, d->stream>>>(d->sc, image, in, in + 2 * n, (uint32_t)n, reinterpret_cast<float *>(d->scratch[1].p));
+    ++d->launches;
+    KZ_CUDA(ctx, cudaMemcpyAsync(rgb, d->scratch[1].p, n * 12, cudaMemcpyDeviceToHost, d->stream));
+    KZ_CUDA(ctx, cudaStreamSynchronize(d->stream));
+    return KZ_OK;
+}
+
+int kzgpu_texture_footprint_dump(kzgpu_ctx *ctx, int device, const kz_ray *rays, size_t n, float *out8) {
+    int rc = check_ready(ctx, true);
+    if (rc) return rc;
+    Device *d;
+    if ((rc = select(ctx, device, &d))) return rc;
+    if (n == 0) return KZ_OK;
+    if (!rays || !out8) return fail(ctx, KZ_ERR_INVALID, "null argument");
+    if (n > 0x7FFFFFFFull) return fail(ctx, KZ_ERR_INVALID, "batch larger than 2^31-1 rays");
+    KZ_CUDA(ctx, d->scratch[0].ensure(n * sizeof(kz_ray), SCRATCH_MIN));
+    KZ_CUDA(ctx, d->scratch[1].ensure(n * 32, SCRATCH_MIN));
+    KZ_CUDA(ctx, cudaMemcpyAsync(d->scratch[0].p, rays, n * sizeof(kz_ray), cudaMemcpyHostToDevice, d->stream));
+    k_texture_footprint_dump<<<(unsigned)((n + KZ_TRACE_THREADS - 1) / KZ_TRACE_THREADS), KZ_TRACE_THREADS, 0, d->stream>>>(d->sc, d->lod, reinterpret_cast<const KzF4 *>(d->scratch[0].p),
+                                                                                                                          (uint32_t)n, reinterpret_cast<float *>(d->scratch[1].p));
+    ++d->launches;
+    KZ_CUDA(ctx, cudaMemcpyAsync(out8, d->scratch[1].p, n * 32, cudaMemcpyDeviceToHost, d->stream));
+    KZ_CUDA(ctx, cudaStreamSynchronize(d->stream));
     return KZ_OK;
 }
 

@@ -29,6 +29,8 @@ struct KzHostScene {
     KzScene sc;                         /* pointers into the vectors above once finalize() ran */
     uint64_t total_vertices = 0, total_triangles = 0;
     bool env_sampling = false;          /* kz_integrator_desc::env_sampling (kz_api.cu builds the environment table, kz_env.h) */
+    bool texture_filtering = false;     /* kz_integrator_desc::texture_filtering (filter_counts) */
+    bool pyramids = false;              /* every image's mip pyramid is laid out after its level 0 (mip_layout): the scene filters its textures */
     std::string error;
 
     /* geometry = true: vertex / index records and the triangle list are built here (tests/hostemu runs the device headers on
@@ -148,6 +150,7 @@ struct KzHostScene {
         sc.integrator.regularization = d->integrator.regularization; sc.integrator.accumulated_roughness = d->integrator.accumulated_roughness;
         sc.integrator.type = d->integrator.type;
         env_sampling = d->integrator.env_sampling != 0;
+        texture_filtering = d->integrator.texture_filtering != 0;
         if (sc.integrator.type < KZ_INTEGRATOR_PATH_MIS || sc.integrator.type > KZ_INTEGRATOR_PATH_MATS) { error = "unknown integrator type"; return false; }
         sc.filter = d->filter;
         sc.border = (int32_t)ceilf(d->filter.radius - 0.5f);
@@ -206,6 +209,56 @@ struct KzHostScene {
                 sc.inv_light_hi[a] = fmaxf(sc.inv_light_hi[a], light_bounds[6 * k + 3 + a]);
             }
         }
+    }
+
+    /* Texture filtering counts when it is asked for, the integrator is path_mis, and an IMAGE node is reachable in uv mode (within
+     * kz_tex_eval_tree's stack depth) from a texture slot that a shaded mesh's BSDF reads: kiss base_color / roughness / metallic, a
+     * normal map, the lambertian / ggx base_color.  Otherwise the scene renders exactly as without the flag. */
+    bool filter_counts() const {
+        if (!texture_filtering || sc.integrator.type != KZ_INTEGRATOR_PATH_MIS) return false;
+        auto reaches_image = [&](int root) {
+            int node[KZ_TEX_MAX_DEPTH_HOST], next[KZ_TEX_MAX_DEPTH_HOST], sp = 0;
+            node[0] = root; next[0] = 0;
+            for (;;) {
+                const kz_texture_desc &t = textures[(size_t)node[sp]];
+                if (t.type == KZ_TEX_IMAGE) return true;
+                const int nchild = t.type == KZ_TEX_BLEND ? 3 : ((t.type == KZ_TEX_BACKGROUND || t.type == KZ_TEX_COLORRAMP) ? 1 : 0);
+                if (next[sp] < nchild) {
+                    const int c = t.child[next[sp]++];
+                    if (c >= 0 && sp + 1 < KZ_TEX_MAX_DEPTH_HOST) { ++sp; node[sp] = c; next[sp] = 0; }
+                    continue;
+                }
+                if (sp == 0) return false;
+                --sp;
+            }
+        };
+        auto leaf_reads_image = [&](const kz_bsdf_desc &b) {
+            if (b.type == KZ_BSDF_KISS) return reaches_image(b.base_color) || reaches_image(b.roughness) || reaches_image(b.metallic);
+            if (b.type == KZ_BSDF_LAMBERTIAN || b.type == KZ_BSDF_GGX) return reaches_image(b.base_color);
+            return false;
+        };
+        for (const KzMeshRec &m : meshes) {
+            if (m.flags & KZ_MESH_IS_LIGHT) continue;
+            const kz_bsdf_desc &b = bsdfs[(size_t)m.bsdf];
+            if (b.type == KZ_BSDF_NORMALMAP ? (reaches_image(b.normal_map) || leaf_reads_image(bsdfs[(size_t)b.nested])) : leaf_reads_image(b)) return true;
+        }
+        return false;
+    }
+    /* Makes room for every image's full mip pyramid (level 0, then levels 1 .. n contiguous, as kz_mip_level reads them) and sets
+     * n_levels; the atlas of all levels must stay below 2^32 texels.  The levels are filled on the GPU (k_mip_level). */
+    bool mip_layout() {
+        size_t total = 0;
+        for (KzImageRec &r : images) {
+            r.texel_offset = (uint32_t)total;
+            r.n_levels = 0;
+            size_t n = (size_t)r.width * r.height;
+            for (int w = r.width, h = r.height; w > 1 || h > 1;) { w = w > 1 ? w >> 1 : 1; h = h > 1 ? h >> 1 : 1; n += (size_t)w * h; ++r.n_levels; }
+            if (total + n > 0xFFFFFFFFull) { error = "texture atlas with mip pyramids (texture filtering) larger than 2^32 texels"; return false; }
+            total += n;
+        }
+        total_texels = total;
+        pyramids = true;
+        return true;
     }
 
     size_t total_texels = 0;

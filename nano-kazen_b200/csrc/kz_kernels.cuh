@@ -424,9 +424,14 @@ __global__ void __launch_bounds__(KZ_TRACE_THREADS, KZ_TRACE_MIN_BLOCKS) k_exten
 #ifndef KZ_SHADE_MIN_BLOCKS_ENV
 #define KZ_SHADE_MIN_BLOCKS_ENV 3           /* environment sampling: up to 168 registers, so that no class spills more than its flag-off kernel */
 #endif
-/* ENV: the environment is a light with table `env` (ignored when ENV is false), see kz_shade_item */
-template <int CLS, bool ENV = false>
-__global__ void __launch_bounds__(KZ_SHADE_THREADS, (ENV && CLS != KZ_CLASS_TERMINAL ? KZ_SHADE_MIN_BLOCKS_ENV : (CLS == KZ_CLASS_DIFFUSE ? KZ_SHADE_MIN_BLOCKS_DIFFUSE : (CLS == KZ_CLASS_TERMINAL ? KZ_SHADE_MIN_BLOCKS_TERMINAL : KZ_SHADE_MIN_BLOCKS)))) k_shade(KzScene sc, KzPathState st, KzControl *ctl, KzQueues q, int nxt, int bounce, KzEnvTable env) {
+#ifndef KZ_SHADE_MIN_BLOCKS_NMAP_ENV_FILT
+#define KZ_SHADE_MIN_BLOCKS_NMAP_ENV_FILT 2 /* normal map with environment sampling and texture filtering: 40 bytes of spills at 168 registers, none in its flag-off kernel */
+#endif
+/* ENV: the environment is a light with table `env` (ignored when ENV is false); FILT: textures are filtered by the footprint the camera
+ * constants `lod` give (ignored when FILT is false; only KISS, NORMALMAP and GENERIC read image textures); see kz_shade_item */
+template <int CLS, bool ENV = false, bool FILT = false>
+__global__ void __launch_bounds__(KZ_SHADE_THREADS, (ENV && FILT && CLS == KZ_CLASS_NORMALMAP ? KZ_SHADE_MIN_BLOCKS_NMAP_ENV_FILT :
+    ((ENV || FILT) && CLS != KZ_CLASS_TERMINAL ? KZ_SHADE_MIN_BLOCKS_ENV : (CLS == KZ_CLASS_DIFFUSE ? KZ_SHADE_MIN_BLOCKS_DIFFUSE : (CLS == KZ_CLASS_TERMINAL ? KZ_SHADE_MIN_BLOCKS_TERMINAL : KZ_SHADE_MIN_BLOCKS))))) k_shade(KzScene sc, KzPathState st, KzControl *ctl, KzQueues q, int nxt, int bounce, KzEnvTable env, KzTexLod lod) {
     const uint32_t n = ctl->n_class[CLS];
     const uint32_t *queue = q.cls[CLS];
     const uint32_t stride = gridDim.x * blockDim.x;
@@ -443,7 +448,7 @@ __global__ void __launch_bounds__(KZ_SHADE_THREADS, (ENV && CLS != KZ_CLASS_TERM
         uint32_t slot = 0u, flags = 0u;
         if (idx < n) {
             slot = queue[idx];
-            flags = kz_shade_item<CLS, ENV>(sc, st, slot, bounce, cnt, env);
+            flags = kz_shade_item<CLS, ENV, FILT>(sc, st, slot, bounce, cnt, env, lod);
         }
         if (CLS != KZ_CLASS_TERMINAL) {
             const bool pa = (flags & KZ_SHADE_CONTINUE) != 0u, pb = (flags & KZ_SHADE_SHADOW) != 0u;
@@ -471,7 +476,7 @@ __global__ void __launch_bounds__(KZ_SHADE_THREADS, (ENV && CLS != KZ_CLASS_TERM
         uint32_t slot = 0u, flags = 0u;
         if (idx < n) {
             slot = queue[idx];
-            flags = kz_shade_item<CLS, ENV>(sc, st, slot, bounce, cnt, env);
+            flags = kz_shade_item<CLS, ENV, FILT>(sc, st, slot, bounce, cnt, env, lod);
         }
         __syncwarp();
         if (CLS != KZ_CLASS_TERMINAL)
@@ -739,6 +744,14 @@ __global__ void k_image_lookup(KzScene sc, int image, int level, const float *st
     const kz3 c = kz_image_bicubic(sc, image, st[2 * i], st[2 * i + 1], level);
     rgb[3 * i] = c.x; rgb[3 * i + 1] = c.y; rgb[3 * i + 2] = c.z;
 }
+/* kzgpu_image_lookup_filtered: the shade kernels' filtered lookup for given (s, t) and st derivatives (ds/dx, dt/dx, ds/dy, dt/dy) */
+__global__ void k_image_lookup_filtered(KzScene sc, int image, const float *st, const float *dst4, uint32_t n, float *rgb) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float *g = dst4 + 4 * (size_t)i;
+    const kz3 c = kz_image_filtered(sc, image, st[2 * i], st[2 * i + 1], kz_tex_lambda(sc.images[image], g[0], g[1], g[2], g[3]));
+    rgb[3 * i] = c.x; rgb[3 * i + 1] = c.y; rgb[3 * i + 2] = c.z;
+}
 
 /* ---- resolve: block.cpp:39-45 + common.cpp:352-366 + bitmap.cpp:46-54 --------------------- */
 __global__ void k_resolve(const KzF4 *frame, int width, int height, int border, float *rgb, uint8_t *srgb8) {
@@ -775,6 +788,24 @@ __global__ void __launch_bounds__(KZ_TRACE_THREADS) k_intersection_dump(KzScene 
     o[13] = its.sh.t.x; o[14] = its.sh.t.y; o[15] = its.sh.t.z;
     o[16] = its.sh.n.x; o[17] = its.sh.n.y; o[18] = its.sh.n.z;
     o[19] = its.dpdu.x; o[20] = its.dpdu.y; o[21] = its.dpdu.z;
+}
+
+/* kzgpu_texture_footprint_dump: the footprint the filtered shade kernels compute at each ray's closest hit */
+__global__ void __launch_bounds__(KZ_TRACE_THREADS) k_texture_footprint_dump(KzScene sc, KzTexLod lod, const KzF4 *rays, uint32_t n, float *out8) {
+    const KzStackRef stk = kz_trav_shared_init();
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const KzF4 ro = rays[2 * (size_t)i], rd = rays[2 * (size_t)i + 1];
+    const KzHit h = kz_trace(sc, stk, ro.x, ro.y, ro.z, rd.x, rd.y, rd.z, ro.w, rd.w, false);
+    float *o = out8 + 8 * (size_t)i;
+    for (int k = 0; k < 8; ++k) o[k] = 0.f;
+    o[0] = -1.f;
+    if (h.geom == KZ_INVALID_ID) return;
+    KzIts its; its.acc_rough = 0.f;
+    fill_intersection(sc, h, its, mk3(0.f));
+    const KzUvDiff duv = kz_its_footprint(sc, lod, h, its);
+    o[0] = (float)its.mesh; o[1] = its.uv.x; o[2] = its.uv.y;
+    o[3] = duv.dudx; o[4] = duv.dvdx; o[5] = duv.dudy; o[6] = duv.dvdy;
 }
 
 /* scene.h:45-56 + mesh.cpp:108-133 + light.cpp:16-51 */

@@ -17,6 +17,7 @@
 #ifndef KZ_PATH_H
 #define KZ_PATH_H
 #include "kz_env.h"
+#include "kz_texlod.h"
 
 /* Path state: three 64-byte blocks per slot, grouped by which stage touches what, so that every access of a stage is a
  * whole 32-byte DRAM sector (slots are visited in queue order, i.e. scattered: the former one-array-per-field layout moved a
@@ -210,9 +211,12 @@ KZ_HD_NOINLINE uint32_t kz_shade_alt_item(const KzScene &sc, const KzPathState &
 /* CLS = material class of the queue this item was sorted into (-1: unknown, resolve at run time).
  * ENV = the environment is a light with table `env` (kz_env.h): next-event estimation picks it as light n_light_meshes with
  * probability 1 / (n_light_meshes + 1), and a BSDF-sampled ray that escapes is weighted against its density.  ENV = false is the
- * reference estimator and does not read `env`. */
-template <int CLS = -1, bool ENV = false>
-KZ_HD uint32_t kz_shade_item(const KzScene &sc, const KzPathState &st, uint32_t slot, int bounce, KzCounters &cnt, const KzEnvTable &env = KzEnvTable{}) {
+ * reference estimator and does not read `env`.
+ * FILT = uv-mode image lookups of the vertex's textures are filtered by its footprint (kz_texlod.h), estimated from the camera constants
+ * `lod`; FILT = false reads level 0 as the reference does and does not read `lod`. */
+template <int CLS = -1, bool ENV = false, bool FILT = false>
+KZ_HD uint32_t kz_shade_item(const KzScene &sc, const KzPathState &st, uint32_t slot, int bounce, KzCounters &cnt, const KzEnvTable &env = KzEnvTable{},
+                             const KzTexLod &lod = KzTexLod{}) {
     if ((CLS < 0 || CLS == KZ_CLASS_GENERIC) && sc.integrator.type != KZ_INTEGRATOR_PATH_MIS) return kz_shade_alt_item(sc, st, slot, bounce, cnt);
     const KzBlockA A = st.a[slot];
     const KzF4 ro = A.ray.o, rd = A.ray.d;
@@ -271,7 +275,9 @@ KZ_HD uint32_t kz_shade_item(const KzScene &sc, const KzPathState &st, uint32_t 
     }
     cnt.vertices += 1;
     uint32_t flags = 0u;
-    const KzBsdfCtx bc = bsdf_ctx<CLS>(sc, its);
+    KzUvDiff duv{0.f, 0.f, 0.f, 0.f};
+    if (FILT) duv = kz_its_footprint(sc, lod, h, its);
+    const KzBsdfCtx<FILT> bc = bsdf_ctx<CLS, FILT>(sc, its, duv);
     const kz3 wiLocal = to_local(its.sh, -rayD);
     const float eps = I.trace_bias;
 

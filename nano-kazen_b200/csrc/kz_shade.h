@@ -51,9 +51,10 @@ KZ_HD void kz_bspline_weights(float f, float w[4]) {
     w[2] = 2.0f / 3.0f - 0.5f * one_f * one_f * (2.0f - one_f);
     w[3] = (f * f * f) / 6.0f;
 }
-/* Mip pyramid resident in HBM: level l (max(1,w>>l) x max(1,h>>l) float4 texels) follows level l-1; built on the GPU
- * at upload by 2x2 box filtering (k_mip_level).  kazen calls OIIO with zero derivatives (texture.cpp:52-57), which selects
- * the finest level, so the render path always passes level 0; coarser levels serve filtered lookups (kzgpu_image_lookup). */
+/* Mip pyramid: level l (max(1,w>>l) x max(1,h>>l) float4 texels) follows level l-1, built on the GPU by 2x2 box filtering
+ * (k_mip_level).  kazen calls OIIO with zero derivatives (texture.cpp:52-57), which selects the finest level, so the reference
+ * render path always passes level 0.  With texture filtering (kz_integrator_desc::texture_filtering) every image's pyramid is
+ * resident from the upload on and uv-mode lookups pick their level from the vertex's footprint (kz_image_filtered). */
 KZ_HD void kz_mip_level(const KzImageRec &im, int level, int &w, int &h, size_t &offset) {
     w = im.width; h = im.height; offset = im.texel_offset;
     if (level > im.n_levels) level = im.n_levels;
@@ -88,12 +89,36 @@ KZ_HD_NOINLINE kz3 kz_image_bicubic(const KzScene &sc, int image, float s, float
     return acc;
 }
 
+/* Footprint of a shading vertex in texture space: uv derivatives per pixel step in x and y (kz_texlod.h computes them). */
+struct KzUvDiff { float dudx, dvdx, dudy, dvdy; };
+
+/* pbrt-v4's trilinear level (MIPMap::Filter) of an isotropic lookup whose st derivatives are dst = (ds/dx, dt/dx, ds/dy, dt/dy):
+ * log2 of twice the longest footprint axis in texels (exact for square power-of-two images, the longer side's texels otherwise). */
+KZ_HD float kz_tex_lambda(const KzImageRec &im, float dsdx, float dtdx, float dsdy, float dtdy) {
+    const float w = (float)im.width, h = (float)im.height;
+    const float width = 2.0f * fmaxf(fmaxf(fabsf(dsdx) * w, fabsf(dtdx) * h), fmaxf(fabsf(dsdy) * w, fabsf(dtdy) * h));
+    return log2f(fmaxf(width, 1e-8f));
+}
+/* Trilinear lookup at level lambda: lambda <= 0 is the reference's level-0 lookup itself, lambda >= n_levels the top level, and in
+ * between the lerp of the bicubic lookups of the two levels around it (bicubic per level, so that a magnified texture is the reference). */
+KZ_HD kz3 kz_image_filtered(const KzScene &sc, int image, float s, float t, float lambda) {
+    if (!(lambda > 0.f)) return kz_image_bicubic(sc, image, s, t);
+    const int top = sc.images[image].n_levels;
+    if (lambda >= (float)top) return kz_image_bicubic(sc, image, s, t, top);
+    const int l = (int)floorf(lambda);
+    const float f = lambda - (float)l;
+    const kz3 a = kz_image_bicubic(sc, image, s, t, l), b = kz_image_bicubic(sc, image, s, t, l + 1);
+    return (1.f - f) * a + f * b;
+}
+
 /* Expression trees are tiny (depth <= 3 in every kazen scene).  They are evaluated post-order
  * with an explicit frame stack of bounded depth: no recursion (no device call stack growth) and
  * no template expansion (a blend has three children; inlining the tree is exponential).
- * dir_mode: Texture::eval(dir) (texture.cpp:66-81,121-126) instead of eval(uv). */
+ * dir_mode: Texture::eval(dir) (texture.cpp:66-81,121-126) instead of eval(uv).
+ * FILT: uv-mode image lookups are filtered by the footprint `duv` (kz_image_filtered); without it every lookup reads level 0. */
 #define KZ_TEX_MAX_DEPTH 4
-KZ_HD_NOINLINE kz3 kz_tex_eval_tree(const KzScene &sc, int root, kz2 uv_, kz3 d, bool dir_mode) {
+template <bool FILT>
+KZ_HD kz3 kz_tex_eval_body(const KzScene &sc, int root, kz2 uv_, kz3 d, bool dir_mode, const KzUvDiff &duv) {
     int node[KZ_TEX_MAX_DEPTH], next[KZ_TEX_MAX_DEPTH];
     kz3 val[KZ_TEX_MAX_DEPTH][3];
     int sp = 0;
@@ -125,7 +150,11 @@ KZ_HD_NOINLINE kz3 kz_tex_eval_tree(const KzScene &sc, int root, kz2 uv_, kz3 d,
                     if (isnan(tt)) tt = 0.0f;
                     r = kz_image_bicubic(sc, t.image, s, tt);
                 } else {
-                    r = kz_image_bicubic(sc, t.image, uv_.x * t.scale, (1.0f - uv_.y) * t.scale);
+                    if (FILT)      /* s = u * scale, t = (1 - v) * scale: ds = scale * du, dt = -scale * dv */
+                        r = kz_image_filtered(sc, t.image, uv_.x * t.scale, (1.0f - uv_.y) * t.scale,
+                                              kz_tex_lambda(sc.images[t.image], t.scale * duv.dudx, -t.scale * duv.dvdx, t.scale * duv.dudy, -t.scale * duv.dvdy));
+                    else
+                        r = kz_image_bicubic(sc, t.image, uv_.x * t.scale, (1.0f - uv_.y) * t.scale);
                     if (t.srgb) r = mk3(srgb_to_linear1(r.x), srgb_to_linear1(r.y), srgb_to_linear1(r.z));
                 }
                 break;
@@ -151,9 +180,17 @@ KZ_HD_NOINLINE kz3 kz_tex_eval_tree(const KzScene &sc, int root, kz2 uv_, kz3 d,
         next[sp] += 1;
     }
 }
-KZ_HD kz3 kz_tex_uv(const KzScene &sc, int node, kz2 uv) {
+KZ_HD_NOINLINE kz3 kz_tex_eval_tree(const KzScene &sc, int root, kz2 uv_, kz3 d, bool dir_mode) {
+    return kz_tex_eval_body<false>(sc, root, uv_, d, dir_mode, KzUvDiff{0.f, 0.f, 0.f, 0.f});
+}
+KZ_HD_NOINLINE kz3 kz_tex_eval_tree(const KzScene &sc, int root, kz2 uv_, KzUvDiff duv) {     /* uv mode, filtered */
+    return kz_tex_eval_body<true>(sc, root, uv_, mk3(0.f), false, duv);
+}
+template <bool FILT = false>
+KZ_HD kz3 kz_tex_uv(const KzScene &sc, int node, kz2 uv, const KzUvDiff &duv = KzUvDiff{0.f, 0.f, 0.f, 0.f}) {
     const kz_texture_desc *t = sc.textures + node;
     if (t->type == KZ_TEX_CONSTANT) return mk3(t->color[0], t->color[1], t->color[2]);     /* the common case */
+    if (FILT) return kz_tex_eval_tree(sc, node, uv, duv);
     return kz_tex_eval_tree(sc, node, uv, mk3(0.f), false);
 }
 KZ_HD kz3 kz_background(const KzScene &sc, kz3 d) {   /* scene.cpp:54-79 */
@@ -225,11 +262,12 @@ KZ_HD kz3 lerp_color(kz3 c1, kz3 c2, float t) { return (1.f - t) * c1 + t * c2; 
 
 /* Texture fetches of one kiss lookup, shared by eval/pdf/sample of the same vertex. */
 struct KzKissParams { kz3 base; float metallic, roughness_raw; };
-KZ_HD KzKissParams kiss_params(const KzScene &sc, const kz_bsdf_desc &m, kz2 uv) {
+template <bool FILT = false>
+KZ_HD KzKissParams kiss_params(const KzScene &sc, const kz_bsdf_desc &m, kz2 uv, const KzUvDiff &duv = KzUvDiff{0.f, 0.f, 0.f, 0.f}) {
     KzKissParams p;
-    p.base = kz_tex_uv(sc, m.base_color, uv);
-    p.metallic = kz_tex_uv(sc, m.metallic, uv).x;
-    p.roughness_raw = kz_tex_uv(sc, m.roughness, uv).x;
+    p.base = kz_tex_uv<FILT>(sc, m.base_color, uv, duv);
+    p.metallic = kz_tex_uv<FILT>(sc, m.metallic, uv, duv).x;
+    p.roughness_raw = kz_tex_uv<FILT>(sc, m.roughness, uv, duv).x;
     return p;
 }
 KZ_HD_NOINLINE kz3 kiss_eval(const kz_bsdf_desc &m, const KzKissParams &kp, const KzBRec &b) {   /* bsdf.cpp:1215-1267 */
@@ -353,15 +391,17 @@ KZ_HD kz3 fresnel_cond(float c, kz3 eta, kz3 k) {                               
 }
 KZ_HD float kd_max(const kz_bsdf_desc &m) { return fmaxf(m.albedo[0], fmaxf(m.albedo[1], m.albedo[2])); }
 
-KZ_HD_NOINLINE kz3 extra_eval(const KzScene &sc, const kz_bsdf_desc &m, const KzBRec &b) {
+/* FILT: the base_color texture of lambertian / ggx is filtered by the vertex's footprint `duv` (extra_eval / extra_sample with it) */
+template <bool FILT>
+KZ_HD kz3 extra_eval_body(const KzScene &sc, const kz_bsdf_desc &m, const KzBRec &b, const KzUvDiff &duv) {
     const kz3 wi = b.wi, wo = b.wo;
     switch (m.type) {
         case KZ_BSDF_LAMBERTIAN:                                                             /* bsdf.cpp:211-221 */
             if (b.measure != KZ_MEASURE_SOLID_ANGLE || wi.z <= 0 || wo.z <= 0) return mk3(0.f);
-            return kz_tex_uv(sc, m.base_color, b.uv) * KZ_INV_PI * wo.z;
+            return kz_tex_uv<FILT>(sc, m.base_color, b.uv, duv) * KZ_INV_PI * wo.z;
         case KZ_BSDF_GGX:                                                                    /* bsdf.cpp:640-647 */
             if (wi.z <= 0 || wo.z <= 0) return mk3(0.f);
-            return ggx_smith_brdf(wi, wo, kz_tex_uv(sc, m.base_color, b.uv), m.alpha, m.anisotropy) * wo.z;
+            return ggx_smith_brdf(wi, wo, kz_tex_uv<FILT>(sc, m.base_color, b.uv, duv), m.alpha, m.anisotropy) * wo.z;
         case KZ_BSDF_ROUGHCONDUCTOR: {                                                       /* bsdf.cpp:765-775 */
             if (wi.z <= 0 || wo.z <= 0) return mk3(0.f);
             const kz3 wh = normalized(wi + wo);
@@ -399,6 +439,12 @@ KZ_HD_NOINLINE kz3 extra_eval(const KzScene &sc, const kz_bsdf_desc &m, const Kz
         }
         default: return mk3(0.f);                                                            /* dielectric, mirror: discrete */
     }
+}
+KZ_HD_NOINLINE kz3 extra_eval(const KzScene &sc, const kz_bsdf_desc &m, const KzBRec &b) {
+    return extra_eval_body<false>(sc, m, b, KzUvDiff{0.f, 0.f, 0.f, 0.f});
+}
+KZ_HD_NOINLINE kz3 extra_eval(const KzScene &sc, const kz_bsdf_desc &m, const KzBRec &b, KzUvDiff duv) {
+    return extra_eval_body<true>(sc, m, b, duv);
 }
 KZ_HD_NOINLINE float extra_pdf(const kz_bsdf_desc &m, const KzBRec &b) {
     const kz3 wi = b.wi, wo = b.wo;
@@ -446,7 +492,8 @@ KZ_HD_NOINLINE float extra_pdf(const kz_bsdf_desc &m, const KzBRec &b) {
     }
 }
 /* returns the weight; *pdf_out = pdf(bRec) as the integrator queries it afterwards (integrator.cpp:314) */
-KZ_HD_NOINLINE kz3 extra_sample(const KzScene &sc, const kz_bsdf_desc &m, KzBRec &b, float sample1, kz2 sample2, float *pdf_out) {
+template <bool FILT>
+KZ_HD kz3 extra_sample_body(const KzScene &sc, const kz_bsdf_desc &m, KzBRec &b, float sample1, kz2 sample2, float *pdf_out, const KzUvDiff &duv) {
     *pdf_out = 0.f;
     kz3 w = mk3(0.f);
     switch (m.type) {
@@ -471,11 +518,11 @@ KZ_HD_NOINLINE kz3 extra_sample(const KzScene &sc, const kz_bsdf_desc &m, KzBRec
             b.measure = KZ_MEASURE_SOLID_ANGLE;
             b.wo = square_to_cosine_hemisphere(sample2);
             b.eta = 1.0f;
-            w = kz_tex_uv(sc, m.base_color, b.uv);
+            w = kz_tex_uv<FILT>(sc, m.base_color, b.uv, duv);
             break;
         case KZ_BSDF_GGX: {                                                                  /* bsdf.cpp:659-670 + ggx_brdf.h:175-203 (measure / eta keep their defaults) */
             if (b.wi.z <= 0) return mk3(0.f);
-            const kz3 albedo = kz_tex_uv(sc, m.base_color, b.uv);
+            const kz3 albedo = kz_tex_uv<FILT>(sc, m.base_color, b.uv, duv);
             const kz2 alpha = roughness_to_alpha(m.alpha, m.anisotropy);
             const kz3 H = sample_ggx_vndf(b.wi, alpha, sample2);
             b.wo = reflect3(b.wi, H);
@@ -535,10 +582,19 @@ KZ_HD_NOINLINE kz3 extra_sample(const KzScene &sc, const kz_bsdf_desc &m, KzBRec
     *pdf_out = extra_pdf(m, b);
     return w;
 }
+KZ_HD_NOINLINE kz3 extra_sample(const KzScene &sc, const kz_bsdf_desc &m, KzBRec &b, float sample1, kz2 sample2, float *pdf_out) {
+    return extra_sample_body<false>(sc, m, b, sample1, sample2, pdf_out, KzUvDiff{0.f, 0.f, 0.f, 0.f});
+}
+KZ_HD_NOINLINE kz3 extra_sample(const KzScene &sc, const kz_bsdf_desc &m, KzBRec &b, float sample1, kz2 sample2, float *pdf_out, KzUvDiff duv) {
+    return extra_sample_body<true>(sc, m, b, sample1, sample2, pdf_out, duv);
+}
 
 /* One shading vertex: the hit mesh's BSDF with its (single) optional normal-map wrapper resolved.
  * Supported nesting (everything kazen's scenes use): diffuse | kiss | normalmap(diffuse|kiss). */
-struct KzBsdfCtx {
+template <bool FILT> struct KzBsdfFoot {};
+template <> struct KzBsdfFoot<true> { KzUvDiff duv; };     /* the vertex's footprint, which filters every uv-mode image lookup of its textures */
+template <bool FILT = false>
+struct KzBsdfCtx : KzBsdfFoot<FILT> {                       /* FILT = false: no footprint (an empty base takes no room) */
     const KzScene *sc;
     const kz_bsdf_desc *outer;     /* mesh BSDF */
     const kz_bsdf_desc *leaf;      /* nested (== outer when not a normal map) */
@@ -549,19 +605,20 @@ struct KzBsdfCtx {
     KzFrame pert;                  /* perturbed frame (bsdf.cpp:366-374) */
 };
 /* CLS: material class the caller's queue was sorted into (KZ_CLASS_*), or -1 when unknown; a known
- * class turns the BSDF dispatch below into compile-time constants. */
-template <int CLS = -1>
-KZ_HD KzBsdfCtx bsdf_ctx(const KzScene &sc, const KzIts &its) {
-    KzBsdfCtx c;
+ * class turns the BSDF dispatch below into compile-time constants.  FILT: textures are filtered by the footprint `duv`. */
+template <int CLS = -1, bool FILT = false>
+KZ_HD KzBsdfCtx<FILT> bsdf_ctx(const KzScene &sc, const KzIts &its, const KzUvDiff &duv = KzUvDiff{0.f, 0.f, 0.f, 0.f}) {
+    KzBsdfCtx<FILT> c;
     c.sc = &sc;
+    if constexpr (FILT) c.duv = duv;
     c.outer = sc.bsdfs + sc.meshes[its.mesh].bsdf;
     c.is_nmap = CLS == KZ_CLASS_NORMALMAP ? true : (CLS >= 0 ? false : c.outer->type == KZ_BSDF_NORMALMAP);
     c.leaf = c.is_nmap ? sc.bsdfs + c.outer->nested : c.outer;
     c.leaf_type = CLS == KZ_CLASS_DIFFUSE ? KZ_BSDF_DIFFUSE : (CLS == KZ_CLASS_KISS ? KZ_BSDF_KISS : c.leaf->type);
-    if (c.leaf_type == KZ_BSDF_KISS) c.kp = kiss_params(sc, *c.leaf, its.uv);
+    if (c.leaf_type == KZ_BSDF_KISS) c.kp = kiss_params<FILT>(sc, *c.leaf, its.uv, duv);
     else { c.kp.base = mk3(0.f); c.kp.metallic = 0.f; c.kp.roughness_raw = 0.f; }
     if (c.is_nmap) {
-        kz3 rgb = kz_tex_uv(sc, c.outer->normal_map, its.uv);
+        kz3 rgb = kz_tex_uv<FILT>(sc, c.outer->normal_map, its.uv, duv);
         c.nm_n = mk3(2 * rgb.x - 1, 2 * rgb.y - 1, 2 * rgb.z - 1);
         kz3 n = normalized(c.nm_n);
         c.pert.n = normalized(to_world(its.sh, n));
@@ -573,21 +630,30 @@ KZ_HD KzBsdfCtx bsdf_ctx(const KzScene &sc, const KzIts &its) {
     }
     return c;
 }
-KZ_HD kz3 leaf_eval(const KzBsdfCtx &c, const KzBRec &b) {
+template <bool FILT>
+KZ_HD kz3 leaf_eval(const KzBsdfCtx<FILT> &c, const KzBRec &b) {
     if (c.leaf_type == KZ_BSDF_KISS) return kiss_eval(*c.leaf, c.kp, b);
-    if (c.leaf_type > KZ_BSDF_NORMALMAP) return extra_eval(*c.sc, *c.leaf, b);
+    if (c.leaf_type > KZ_BSDF_NORMALMAP) {
+        if constexpr (FILT) return extra_eval(*c.sc, *c.leaf, b, c.duv);
+        else return extra_eval(*c.sc, *c.leaf, b);
+    }
     if (b.measure != KZ_MEASURE_SOLID_ANGLE || b.wi.z <= 0 || b.wo.z <= 0) return mk3(0.0f);   /* bsdf.cpp:27-36 */
     return mk3(c.leaf->albedo[0], c.leaf->albedo[1], c.leaf->albedo[2]) * KZ_INV_PI * b.wo.z;
 }
-KZ_HD float leaf_pdf(const KzBsdfCtx &c, const KzBRec &b) {
+template <bool FILT>
+KZ_HD float leaf_pdf(const KzBsdfCtx<FILT> &c, const KzBRec &b) {
     if (c.leaf_type == KZ_BSDF_KISS) return kiss_pdf(*c.leaf, c.kp, b);
     if (c.leaf_type > KZ_BSDF_NORMALMAP) return extra_pdf(*c.leaf, b);
     if (b.measure != KZ_MEASURE_SOLID_ANGLE || b.wi.z <= 0 || b.wo.z <= 0) return 0.0f;        /* bsdf.cpp:39-55 */
     return KZ_INV_PI * b.wo.z;
 }
-KZ_HD kz3 leaf_sample(const KzBsdfCtx &c, KzBRec &b, float s1, kz2 s2, float *pdf_out) {
+template <bool FILT>
+KZ_HD kz3 leaf_sample(const KzBsdfCtx<FILT> &c, KzBRec &b, float s1, kz2 s2, float *pdf_out) {
     if (c.leaf_type == KZ_BSDF_KISS) return kiss_sample(*c.leaf, c.kp, b, s1, s2, pdf_out);
-    if (c.leaf_type > KZ_BSDF_NORMALMAP) return extra_sample(*c.sc, *c.leaf, b, s1, s2, pdf_out);
+    if (c.leaf_type > KZ_BSDF_NORMALMAP) {
+        if constexpr (FILT) return extra_sample(*c.sc, *c.leaf, b, s1, s2, pdf_out, c.duv);
+        else return extra_sample(*c.sc, *c.leaf, b, s1, s2, pdf_out);
+    }
     *pdf_out = 0.f;                                                                            /* bsdf.cpp:58-75 */
     if (b.wi.z <= 0) return mk3(0.0f);
     b.measure = KZ_MEASURE_SOLID_ANGLE;
@@ -598,7 +664,8 @@ KZ_HD kz3 leaf_sample(const KzBsdfCtx &c, KzBRec &b, float s1, kz2 s2, float *pd
 }
 
 /* eval + pdf of the mesh BSDF for (wi, wo) given in the ORIGINAL shading frame (NEE, integrator.cpp:283-290) */
-KZ_HD void bsdf_eval_pdf(const KzBsdfCtx &c, const KzIts &its, kz3 wi, kz3 wo, kz3 *f, float *pdf) {
+template <bool FILT>
+KZ_HD void bsdf_eval_pdf(const KzBsdfCtx<FILT> &c, const KzIts &its, kz3 wi, kz3 wo, kz3 *f, float *pdf) {
     KzBRec b; b.wi = wi; b.wo = wo; b.uv = its.uv; b.acc_rough = its.acc_rough; b.eta = 1.f; b.measure = KZ_MEASURE_SOLID_ANGLE;
     if (!c.is_nmap) { *f = leaf_eval(c, b); *pdf = leaf_pdf(c, b); return; }
     /* bsdf.cpp:290-336 */
@@ -613,7 +680,8 @@ KZ_HD void bsdf_eval_pdf(const KzBsdfCtx &c, const KzIts &its, kz3 wi, kz3 wo, k
 
 /* sample() of the mesh BSDF + the integrator's follow-up pdf(bRec) query (integrator.cpp:307-314).
  * wo is returned in the ORIGINAL shading frame. */
-KZ_HD kz3 bsdf_sample(const KzBsdfCtx &c, const KzIts &its, kz3 wi, float s1, kz2 s2, kz3 *wo, float *pdf, int *measure, float *eta) {
+template <bool FILT>
+KZ_HD kz3 bsdf_sample(const KzBsdfCtx<FILT> &c, const KzIts &its, kz3 wi, float s1, kz2 s2, kz3 *wo, float *pdf, int *measure, float *eta) {
     KzBRec b; b.wi = wi; b.wo = mk3(0.f); b.uv = its.uv; b.acc_rough = its.acc_rough; b.eta = 1.f; b.measure = KZ_MEASURE_UNKNOWN;
     if (!c.is_nmap || (wi.z > 0 && dot(c.nm_n, wi) <= 0)) {
         float p;
@@ -647,7 +715,8 @@ KZ_HD kz3 bsdf_sample(const KzBsdfCtx &c, const KzIts &its, kz3 wi, float s1, kz
     }
     return result;
 }
-KZ_HD float bsdf_regularize(const KzBsdfCtx &c) {   /* bsdf.h:125, bsdf.cpp:412,1397-1399 */
+template <bool FILT>
+KZ_HD float bsdf_regularize(const KzBsdfCtx<FILT> &c) {   /* bsdf.h:125, bsdf.cpp:412,1397-1399 */
     return c.leaf_type == KZ_BSDF_KISS ? c.kp.roughness_raw : 0.f;
 }
 

@@ -674,8 +674,9 @@ public:
         m_desc.accumulated_roughness = p.getFloat("accumulatedRoughness", 0.5f);
         m_desc.type = KZ_INTEGRATOR_PATH_MIS;
         m_desc.env_sampling = p.getBoolean("envSampling", false) ? 1 : 0;     /* the environment as a light (kz_env.h); off: the reference estimator */
+        m_desc.texture_filtering = p.getBoolean("textureFiltering", false) ? 1 : 0;     /* footprint-filtered image lookups (kz_texlod.h); off: mip level 0 */
     }
-    GpuPathMisIntegrator(const PropertyList &, int type) { m_desc = kz_integrator_desc{5, 0.001f, 0, 0.5f, type, 0}; }
+    GpuPathMisIntegrator(const PropertyList &, int type) { m_desc = kz_integrator_desc{5, 0.001f, 0, 0.5f, type, 0, 0}; }
     ~GpuPathMisIntegrator() override { if (m_ctx) kzgpu_destroy(m_ctx); }
     kz_integrator_desc describe() const override { return m_desc; }
 
@@ -715,8 +716,8 @@ public:
     kzgpu_ctx *context() const { return m_ctx; }
     std::string toString() const override {
         static const char *names[] = {"GpuPathMisIntegrator", "GpuNormalIntegrator", "GpuAmbientOcclusionIntegrator", "GpuWhittedIntegrator", "GpuPathMatsIntegrator"};
-        return fmt("%s[maxDepth=%d, traceBias=%g, regularization=%d, envSampling=%d]", names[m_desc.type], m_desc.max_depth, m_desc.trace_bias, m_desc.regularization,
-                   m_desc.env_sampling);
+        return fmt("%s[maxDepth=%d, traceBias=%g, regularization=%d, textureFiltering=%d, envSampling=%d]", names[m_desc.type], m_desc.max_depth, m_desc.trace_bias,
+                   m_desc.regularization, m_desc.texture_filtering, m_desc.env_sampling);
     }
 private:
     kz_integrator_desc m_desc; kzgpu_ctx *m_ctx = nullptr;

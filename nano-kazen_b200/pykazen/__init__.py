@@ -72,7 +72,7 @@ class SamplerDesc(C.Structure):
 
 class IntegratorDesc(C.Structure):
     _fields_ = [("max_depth", C.c_int32), ("trace_bias", C.c_float), ("regularization", C.c_int32),
-                ("accumulated_roughness", C.c_float), ("type", C.c_int32), ("env_sampling", C.c_int32)]
+                ("accumulated_roughness", C.c_float), ("type", C.c_int32), ("env_sampling", C.c_int32), ("texture_filtering", C.c_int32)]
 
 
 class FilterDesc(C.Structure):
@@ -326,10 +326,13 @@ class SceneBuilder:
         self.filter.radius = r
         self.filter.table[:] = tab.tolist()
 
-    def set_integrator(self, max_depth=5, trace_bias=1e-3, regularization=False, accumulated_roughness=0.5, kind="path_mis", env_sampling=False):
-        """env_sampling: path_mis also samples the background as a light (kz_integrator_desc::env_sampling in include/kzgpu.h)"""
+    def set_integrator(self, max_depth=5, trace_bias=1e-3, regularization=False, accumulated_roughness=0.5, kind="path_mis", env_sampling=False,
+                       texture_filtering=False):
+        """env_sampling: path_mis also samples the background as a light (kz_integrator_desc::env_sampling in include/kzgpu.h);
+        texture_filtering: path_mis filters image textures by their screen footprint (kz_integrator_desc::texture_filtering)"""
         t = {"path_mis": 0, "normals": 1, "ao": 2, "whitted": 3, "path_mats": 4}[kind]
-        self.integrator = IntegratorDesc(min(512, max_depth), trace_bias, int(regularization), accumulated_roughness, t, int(env_sampling))
+        self.integrator = IntegratorDesc(min(512, max_depth), trace_bias, int(regularization), accumulated_roughness, t, int(env_sampling),
+                                         int(texture_filtering))
 
     def desc(self):
         d = SceneDesc()
@@ -567,6 +570,25 @@ class Gpu(_Backend):
         u2 = np.ascontiguousarray(u2, np.float32).reshape(-1, 2)
         out = np.zeros((u2.shape[0], 8), np.float32)
         self._call("env_sample_dump", self.h, C.c_int(device), u2.ctypes.data_as(c_float_p), C.c_size_t(u2.shape[0]), out.ctypes.data_as(c_float_p))
+        return out
+
+    def image_lookup_filtered(self, image, st, dst):
+        """the shade kernels' filtered lookup of image `image` at (s, t) pairs with st derivatives dst = (ds/dx, dt/dx, ds/dy, dt/dy)
+        per pair: (n, 3) float32; raises unless the scene filters its textures"""
+        st = np.ascontiguousarray(st, np.float32).reshape(-1, 2)
+        dst = np.ascontiguousarray(dst, np.float32).reshape(-1, 4)
+        assert dst.shape[0] == st.shape[0]
+        out = np.zeros((st.shape[0], 3), np.float32)
+        self._call("image_lookup_filtered", self.h, C.c_int(image), st.ctypes.data_as(c_float_p), dst.ctypes.data_as(c_float_p), C.c_size_t(st.shape[0]),
+                   out.ctypes.data_as(c_float_p))
+        return out
+
+    def texture_footprint_dump(self, rays, device=0):
+        """the texture footprint at each ray's closest hit on device `device`: (n, 8) float32 = mesh (-1: miss), u, v, du/dx, dv/dx,
+        du/dy, dv/dy, 0 (include/kzgpu.h)"""
+        rays = np.ascontiguousarray(rays, RAY_DTYPE)
+        out = np.zeros((rays.shape[0], 8), np.float32)
+        self._call("texture_footprint_dump", self.h, C.c_int(device), rays.ctypes.data_as(C.c_void_p), C.c_size_t(rays.shape[0]), out.ctypes.data_as(c_float_p))
         return out
 
     def configure(self, key, value):
